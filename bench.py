@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py — voice-samples/sec of the render hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE config 3, per GPU): 65,536 voices, oscillator + resonant biquad (2nd-order
@@ -68,7 +68,13 @@ def parse():
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-seconds", type=float, default=30.0, help="target CPU time of the baseline sample")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last step computed as DIR/<name>.npy (float32, a fixed "
+                         "sample of voices, at most 64 MiB in all) so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def step_frames(steps, block):
@@ -300,6 +306,32 @@ def parity_of_timed_render(voices, final_state, last_block, frames, np):
             "voices_over_1e-4_unscaled": over, "oracle_seconds": dt}
 
 
+DUMP_SEED = 0
+DUMP_MAX_FRAMES = 4 << 20           # of one row: 16 MiB
+DUMP_ROW_BYTES = 40 << 20           # the sampled rows and their phases; the bus adds at most 16 MiB
+
+
+def dump_outputs(out_dir, block, frames, final_state, bus, np, torch):
+    """--dump-outputs: what a caller of the timed path holds after its last step, as float32 .npy files.
+      last_block.npy  [n, frames]  that step's output rows: every voice when they fit in the budget, else the
+                                   rows of n voices drawn with numpy's default_rng(DUMP_SEED), in voice order
+      phase.npy       [n]          the oscillator phase the same voices carry out of the step
+      bus.npy         [frames]     the step's part of the master bus (--master-bus only)
+    The bank is a pure function of the arguments (bankgen is counter-based), so runs with the same arguments
+    compare file for file."""
+    V = block.shape[0]
+    cols = min(frames, DUMP_MAX_FRAMES)
+    n = min(V, max(1, DUMP_ROW_BYTES // (4 * (cols + 1))))
+    idx = np.arange(V) if n == V else np.sort(np.random.default_rng(DUMP_SEED).choice(V, n, replace=False))
+    rows = block.index_select(0, torch.as_tensor(idx, device=block.device))[:, :cols]
+    out = {"last_block": rows.cpu().numpy(), "phase": final_state["phase"][idx]}
+    if bus is not None:
+        out["bus"] = bus[:cols].cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(a, dtype=np.float32))
+
+
 def _timed(torch, stream, bank, body):
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     torch.cuda.synchronize()
@@ -432,6 +464,7 @@ def extra_config4(s2, bankgen, torch, dist, stream, rank, world, dev_index, rank
 
 
 def main():
+    sys.dont_write_bytecode = True      # the tree may be read-only: nothing is written or cached there
     args = parse()
     capture_stdout()
     if args.impl == "reference":
@@ -509,6 +542,9 @@ def main():
     final_state = bank.get_state()
     assert np.all(final_state["frame_offset"] == total_frames)
     assert bool(torch.isfinite(ring[(len(frames) - 1) & 1][:, :frames[-1]]).all())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ring[(len(frames) - 1) & 1], frames[-1], final_state,
+                     master[total_frames - frames[-1]:] if want_master else None, np, torch)
 
     # ---- parity of the timed render against the CPU oracle (after the timed region) -------------
     parity = None

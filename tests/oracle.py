@@ -3,6 +3,7 @@ tests/, __graft_entry__.smoke() and bench.py's cpu_baseline / --impl reference l
 import ctypes as C
 import pathlib
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -67,18 +68,27 @@ _lib = None
 
 def use_native_build():
     """bench.py only: time the CPU baseline on a build tuned for THIS host (`make -C oracle native`: -O3
-    -march=native, same IEEE semantics).  Falls back to the portable library when it cannot be built.
-    Returns the flags description for the bench line."""
-    global _lib, SO
-    native = ROOT / "oracle" / "libs2oracle_native.so"
+    -march=native, same IEEE semantics).  Built fresh in a temporary directory, since the tree may be read-only
+    and a copy built on another host may use other instructions.  Falls back to the portable library when it
+    cannot be built.  Returns the flags description for the bench line."""
+    global _lib
     try:
-        native.unlink(missing_ok=True)          # a copy built on another host may use other instructions
-        subprocess.run(["make", "-C", str(native.parent), "native"], check=True, capture_output=True)
-        C.CDLL(str(native))
-        SO, _lib = native, None
+        with tempfile.TemporaryDirectory() as tmp:
+            native = pathlib.Path(tmp) / "libs2oracle_native.so"
+            subprocess.run(["make", "-C", str(ROOT / "oracle"), "native", f"NATIVE_SO={native}"],
+                           check=True, capture_output=True)
+            _lib = _load(native)                # stays mapped after the directory is removed
         return "-O3 -march=native -ffp-contract=off"
     except Exception:
         return "-O2 -march=x86-64-v3 -ffp-contract=off"
+
+
+def _load(path):
+    h = C.CDLL(str(path))
+    for name, (res, args) in _SIGS.items():
+        fn = getattr(h, name)
+        fn.restype, fn.argtypes = res, args
+    return h
 
 
 def lib():
@@ -86,11 +96,7 @@ def lib():
     if _lib is None:
         if not SO.exists():
             subprocess.run(["make", "-C", str(SO.parent)], check=True, capture_output=True)
-        h = C.CDLL(str(SO))
-        for name, (res, args) in _SIGS.items():
-            fn = getattr(h, name)
-            fn.restype, fn.argtypes = res, args
-        _lib = h
+        _lib = _load(SO)
     return _lib
 
 

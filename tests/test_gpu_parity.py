@@ -1070,6 +1070,33 @@ def test_render_cli(tmp_path):
     assert wav.read_bytes()[:4] == b"RIFF"
 
 
+def test_bench_times_the_steps_asked_and_dumps_the_last():
+    """bench.py --steps K times K steps, and --dump-outputs writes what the last of them rendered: the same bank
+    rendered here through the same pipelined path gives the same bits, and the oracle the same phases."""
+    import json, pathlib, subprocess, sys, tempfile
+    root = pathlib.Path(__file__).resolve().parent.parent
+    V, T, K = 4096, 1024, 3
+    with tempfile.TemporaryDirectory() as out:
+        res = subprocess.run([sys.executable, str(root / "bench.py"), "--voices", str(V), "--block", str(T),
+                              "--steps", str(K), "--warmup", "1", "--no-e2e", "--no-extra", "--no-cpu-baseline",
+                              "--no-parity", "--dump-outputs", out], capture_output=True, text=True, timeout=600)
+        assert res.returncode == 0, res.stderr
+        rows, phase = np.load(pathlib.Path(out) / "last_block.npy"), np.load(pathlib.Path(out) / "phase.npy")
+    line = json.loads(res.stdout.strip().splitlines()[-1])
+    assert line["steps"] == K and len(line["step_ms"]) == K and line["config"]["render_frames"] == K * T
+    assert rows.dtype == np.float32 and rows.shape == (V, T) and phase.shape == (V,)
+    v = bankgen.make_bank(V, 60 * SR, mod_to_lpf_choices=bankgen.MOD_TO_LPF_BIQUAD)
+    out = torch.empty((V, T), device="cuda", dtype=torch.float32)
+    with s2.VoiceBank(v, SR, 1) as bank:
+        bank.set_pipeline(4)
+        for _ in range(K):
+            bank.render(T, out, T, None)
+        bank.sync()
+    assert out.cpu().numpy().tobytes() == rows.tobytes()
+    _, _, rst = oracle_bank_render(v, 1, [T] * K)
+    assert rst["phase"].tobytes() == phase.tobytes()
+
+
 # ------------------------------------------------------------------------------ player hand-off
 
 def test_player_fill_is_the_reference_callback():

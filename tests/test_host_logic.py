@@ -267,6 +267,32 @@ def test_bench_reference_arm_runs_on_cpu():
     assert line["cpu_baseline"]["kind"] == "port" and line["e2e"]["h2d_bytes_per_step"] == 0
 
 
+def test_bench_dump_outputs_is_a_fixed_sample_within_64_mib(tmp_path):
+    """bench.py --dump-outputs: a 65,536-voice block is sampled to the same voices on every call and stays under
+    64 MiB; a narrow block is written whole; the rows, their phases and the bus are float32."""
+    import torch
+    import bench
+    for V, T, bus in ((65536, 4096, None), (300, 1000, torch.linspace(-1, 1, 1000))):
+        block = torch.arange(V, dtype=torch.float32)[:, None].expand(V, T)      # row v holds v
+        st = np.zeros(V, dtype=s2.VOICE_STATE)
+        st["phase"] = np.arange(V, dtype=np.float32)
+        dirs = [tmp_path / f"{V}_a", tmp_path / f"{V}_b"]
+        for d in dirs:
+            bench.dump_outputs(str(d), block, T, st, bus, np, torch)
+        files = sorted(p.name for p in dirs[0].iterdir())
+        assert files == (["bus.npy", "last_block.npy", "phase.npy"] if bus is not None else ["last_block.npy", "phase.npy"])
+        assert sum(p.stat().st_size for p in dirs[0].iterdir()) <= 64 << 20
+        rows, phase = np.load(dirs[0] / "last_block.npy"), np.load(dirs[0] / "phase.npy")
+        assert rows.dtype == phase.dtype == np.float32 and rows.shape == (phase.size, T)
+        assert np.array_equal(rows[:, 0], phase) and np.all(rows == rows[:, :1])      # each row beside its phase
+        assert np.all(np.diff(phase) > 0)
+        assert phase.size == min(V, bench.DUMP_ROW_BYTES // (4 * (T + 1)))
+        if bus is not None:
+            assert np.load(dirs[0] / "bus.npy").tobytes() == bus.numpy().tobytes()
+        for name in files:
+            assert (dirs[0] / name).read_bytes() == (dirs[1] / name).read_bytes()
+
+
 def test_math_kernels_round_once_on_cpu(tmp_path):
     """synth2_b200/csrc/s2_math.h (2^x, e^x, sin/cos used for filter coefficients) is host-and-device code:
     compiled for the CPU it must return the once-rounded binary64 result on dense sweeps (tools/check_math.cpp)."""
