@@ -64,6 +64,7 @@ namespace s2c {
 S2C_FN float vadd(float a, float b) { return S2C_ADD(a, b); }
 S2C_FN float vmul(float a, float b) { return S2C_MUL(a, b); }
 S2C_FN float vfma(float a, float b, float c) { return S2C_FMA(a, b, c); }
+S2C_FN float vmin(float a, float b) { return fminf(a, b); }
 template <class T> struct Splat;
 template <> struct Splat<float> { static S2C_FN float of(float x) { return x; } };
 template <class T> S2C_FN T splat(float x) { return Splat<T>::of(x); }
@@ -124,6 +125,7 @@ __device__ __forceinline__ float2 vfma(float2 a, float2 b, float2 c) { return ma
 template <> struct Splat<float2> { static __device__ __forceinline__ float2 of(float x) { return make_float2(x, x); } };
 __device__ __forceinline__ float2 vex2(float2 x) { return make_float2(vex2(x.x), vex2(x.y)); }
 __device__ __forceinline__ float2 vrcp(float2 x) { return make_float2(vrcp(x.x), vrcp(x.y)); }
+__device__ __forceinline__ float2 vmin(float2 a, float b) { return make_float2(fminf(a.x, b), fminf(a.y, b)); }
 #endif
 
 // prod + y with its own rounding, where prod may come from a packed multiply (see the hazard note)
@@ -160,10 +162,16 @@ template <class T>
 S2C_FN T div_in_range(T num, T den, T nden) { return div_in_range_from(num, nden, vrcp(den)); }
 
 // k = e^-theta in binary32 (one-pole, filters.rs:21): 2^-(theta log2 e), log2 e = L1 + L2, the product in two parts:
-// tn = RN(theta * -L1), r = theta * L1 + tn (exact), tl = r + theta * L2, k = 2^tn * (1 - tl ln 2)
+// tn = RN(theta * -L1), r = theta * L1 + tn (exact), tl = r + theta * L2, k = 2^tn * (1 - tl ln 2).
+// theta is first clamped to kThetaBig: a cutoff modulated past binary32 (2^(m amount) with m amount >= 128, or
+// 2 pi f beyond the largest float) gives theta = +inf, and then r = inf - inf is NaN where the reference's
+// exp(-inf) is 0.  Below the clamp nothing changes; from it up to ~2.3e38 the result was already 0 (2^tn
+// underflows), and above that theta * L1 overflows and the unclamped form gave NaN too.
+constexpr float kThetaBig = 128.0f;
 template <class T>
 S2C_FN T exp_neg_fast(T th) {
     const float L1 = 0x1.715476p+0f, L2 = 0x1.4ae0c0p-26f;
+    th = vmin(th, kThetaBig);
     const T tn = vmul(th, splat<T>(-L1));
     const T r = vfma(th, splat<T>(L1), tn);
     const T tl = vfma(th, splat<T>(L2), r);

@@ -3,7 +3,8 @@
 // 1. div_in_range against the IEEE quotient over the operand range of the second-order filters, with the reciprocal
 //    estimate off by up to +-2 ulp (the special-function unit's error is not modelled more finely than that): how
 //    often it is not the correctly rounded value, and by how much;
-// 2. exp_neg_fast against exp(-theta) in binary64;
+// 2. exp_neg_fast against exp(-theta) in binary64; at theta = +inf (an overflowing cutoff) it is 0, and its clamp
+//    against the unclamped form for every binary32 theta (every 61st in quick mode);
 // 3. windowed sin / cos against the once-rounded binary64 values: mismatch rates and worst absolute error;
 // 4. theta_of (division by the sample rate as reciprocal + residual step) against the IEEE quotient, for EVERY binary32
 //    numerator the path can produce, at the usual rates;
@@ -11,7 +12,8 @@
 // 6. a whole decay sweep of the resonant low-pass at its worst corner (100-200 Hz, damping 0.2): coefficients from
 //    windows vs the full per-frame evaluation (the reference's chain with binary64 transcendentals rounded once),
 //    and the filter outputs they produce.
-// Exits non-zero if 1 is off by more than an ulp or wrong in more than 1e-4 of the cases, if 2 exceeds 4 ulp, if 3 adds
+// Exits non-zero if 1 is off by more than an ulp or wrong in more than 1e-4 of the cases, if 2 exceeds 4 ulp, gives
+// anything but 0 at +inf or changes a bit of the unclamped form below the clamp, if 3 adds
 // more than 4e-9 to a correct rounding (or misses the rounded-once value in more than 2 % of slow-sweep frames), if 4
 // differs anywhere, if 5 differs in more than 1 % of arguments or by more than an ulp, or if 6 changes a coefficient
 // in more than 2 % of the frames.
@@ -79,6 +81,39 @@ int main(int argc, char** argv) {
         }
         printf("exp_neg_fast: worst error %.2f ulp over theta in [0.004, 40] (host exp2f standing in for ex2.approx)\n", worst);
         fail |= worst > 4.0;
+    }
+
+    // ---- 2b. exp_neg_fast at an overflowing cutoff: theta = +inf gives k = 0 (the reference's exp(-inf)), and the
+    //          clamp that does it changes no other result: below kThetaBig every binary32 theta keeps the bits of the
+    //          unclamped form; from kThetaBig up, the unclamped form gave 0, or NaN once theta * log2 e overflows
+    {
+        auto unclamped = [](float th) {
+            const float L1 = 0x1.715476p+0f, L2 = 0x1.4ae0c0p-26f;
+            const float tn = th * -L1;
+            const float r = fmaf(th, L1, tn);
+            const float tl = fmaf(th, L2, r);
+            const float e = vex2(tn);
+            return fmaf(e, tl * -0x1.62e430p-1f, e);
+        };
+        const float inf = INFINITY;
+        const float kinf = exp_neg_fast<float>(inf);
+        long n = 0, changed = 0, bad_big = 0;
+        const uint32_t step = quick ? 61u : 1u;
+        for (uint64_t u = 0; u <= 0xffffffffull; u += step) {
+            const float th = fbits((uint32_t)u);
+            if (th != th) continue;                                         // NaN: not an angle
+            const float got = exp_neg_fast<float>(th), old = unclamped(th);
+            n++;
+            if (th < kThetaBig) {
+                changed += bits(got) != bits(old);
+            } else {
+                const bool old_ok = bits(old) == 0u || (old != old && std::isinf(th * 0x1.715476p+0f));
+                bad_big += bits(got) != 0u || !old_ok;
+            }
+        }
+        printf("exp_neg_fast clamp: k(+inf) = %g; %ld thetas, %ld below %g changed, %ld from it up not (k = 0, was 0 "
+               "or NaN)\n", (double)kinf, n, changed, (double)kThetaBig, bad_big);
+        fail |= bits(kinf) != 0u || changed != 0 || bad_big != 0;
     }
 
     // ---- 3. windows.  "slack" = |result - exact| - ulp(result)/2: what the evaluation adds on top of a correct rounding.
