@@ -120,9 +120,14 @@ int s2_bank_set_releases(s2_bank* bank, const uint32_t* h_release);
  *   d_voice_out  device pointer or NULL; row v = d_voice_out + v*row_stride, `frames` floats;
  *                16-byte aligned base and row_stride % 4 == 0.  Inactive voices write zeros.
  *   d_bus_out    device pointer or NULL; `frames` floats, mono (audio_player.rs:23-24):
- *                bus[i] = sum over voices in index order (synth.rs:176-202).  For banks of up
- *                to 32 voices the order is exactly the reference's; above, per-warp partial
- *                sums (each in index order) are added in warp order.
+ *                bus[i] = sum over voices (synth.rs:176-202).  Banks of up to 32 voices add
+ *                in exactly the reference's order, in every mode: sequentially from 0.0 in
+ *                voice order.  Wider banks add per-warp partials, each a fixed tree over the
+ *                warp's 32 slots (slots are voices reordered at creation), then the partials
+ *                by a fixed reduction tree; time-split blocks above 32 voices add the rows by
+ *                a fixed tree.  Deterministic (the same state and frames give the same bits;
+ *                the default and pipelined paths also give the same bits as each other), but
+ *                in no particular voice order.
  * Asynchronous on the bank's stream.
  */
 int s2_bank_render(s2_bank* bank, size_t frames, float* d_voice_out, size_t row_stride,

@@ -364,11 +364,13 @@ int bank_render_time_split(s2_bank* b, size_t frames, float* d_voice_out, size_t
     CUDA_TRY(cudaEventRecord(b->ev_k2[p], b->stream));
     g_launches.fetch_add(2, std::memory_order_relaxed);
     if (d_bus_out) {
-        // one warp rendered one voice: the output rows (silent voices included, as zeros) are the partial sums,
-        // added by the same reduction kernel
+        // one warp rendered one voice: the output rows (silent voices included, as zeros) are the partial sums.
+        // Up to 32 voices they are added in voice order, as on the default path; wider banks take the reduction
+        // kernel's fixed tree.
         const uint32_t nv = (uint32_t)b->n_voices;
-        if (nv == 1) {
-            CUDA_TRY(cudaMemcpyAsync(d_bus_out, d_voice_out, frames * sizeof(float), cudaMemcpyDeviceToDevice, b->stream));
+        if (nv <= 32u) {
+            CUDA_TRY(s2::launch_ts_mix_rows(d_voice_out, nv, row_stride, (uint32_t)frames, d_bus_out, b->stream));
+            g_launches.fetch_add(1, std::memory_order_relaxed);
         } else {
             const size_t need = (size_t)s2::bus_segments(nv) * frames;
             if (need > b->partials_cap) {

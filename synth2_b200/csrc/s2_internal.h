@@ -77,6 +77,10 @@ cudaError_t launch_ts_phase(const RenderArgs& a, float* seg_phase, cudaStream_t 
 // moving: some voice's cutoff follows a ramping mod envelope in this block (per-frame coefficients)
 cudaError_t launch_ts_render(const RenderArgs& a, uint32_t filter_kind, bool moving, const float* seg_phase,
                              cudaStream_t stream);
+// bus[t] = sum of rows[r * row_stride + t] over r = 0, 1, ..., n_rows - 1, sequentially from +0.0 (the reference's
+// order; for banks of at most 32 voices)
+cudaError_t launch_ts_mix_rows(const float* rows, uint32_t n_rows, size_t row_stride, uint32_t frames, float* bus,
+                               cudaStream_t stream);
 // one kernel, fixed summation order; partial row w starts at partials + w * row_stride.  With `counters` (kBusCounters
 // zeroed words owned by the bank, launches on one stream at a time) and 4 * frames floats of scratch, wide banks
 // take the four-frames-per-lane form.

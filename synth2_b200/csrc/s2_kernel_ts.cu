@@ -314,7 +314,25 @@ __global__ void __launch_bounds__(32) ts_render_kernel(const RenderArgs a, const
     }
 }
 
+// The mix of a bank of at most one warp's voices, in the reference's order (synth.rs:176-202): one thread per frame
+// adds the rows in voice order to an accumulator that starts at +0.0, so a lone -0.0 sample comes out as +0.0.
+__global__ void __launch_bounds__(256) ts_mix_rows_kernel(const float* __restrict__ rows, uint32_t n_rows,
+                                                          size_t row_stride, uint32_t frames, float* __restrict__ bus) {
+    const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= frames) return;
+    float acc = 0.0f;
+    for (uint32_t r = 0; r < n_rows; r++) acc = __fadd_rn(acc, rows[(size_t)r * row_stride + t]);
+    bus[t] = acc;
+}
+
 }  // namespace
+
+cudaError_t launch_ts_mix_rows(const float* rows, uint32_t n_rows, size_t row_stride, uint32_t frames, float* bus,
+                               cudaStream_t stream) {
+    if (frames == 0) return cudaSuccess;
+    ts_mix_rows_kernel<<<(frames + 255u) / 256u, 256, 0, stream>>>(rows, n_rows, row_stride, frames, bus);
+    return cudaGetLastError();
+}
 
 cudaError_t launch_ts_phase(const RenderArgs& a, float* seg_phase, cudaStream_t stream) {
     if (a.n_voices == 0) return cudaSuccess;
