@@ -154,6 +154,10 @@ int s2_bank_render_bus_host_async(s2_bank* bank, size_t frames, float* d_voice_o
  *   - the caller must not reuse an output buffer the bank may still be writing (join first);
  *   - s2_bank_set_releases is pipelined too (each range applies the table before its next render);
  *     every other entry (set_voice, release_voice, get/set_state, trace) drains the pipeline first;
+ *   - edits take effect in call order, as in the default mode: set_voice, release_voice, a trace or a
+ *     pipeline change after s2_bank_set_releases applies the table first, so a later edit of a voice's
+ *     note-off is never overwritten by an earlier table;
+ *   - s2_bank_trace_phase returns after its render has finished;
  *   - s2_bank_render_bus_host_async makes the bank's own stream (given at creation) wait for the copy.
  * n_sub = 1 (default) keeps everything on the bank's stream.
  */

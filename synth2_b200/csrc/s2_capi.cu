@@ -212,6 +212,21 @@ int bank_drain(s2_bank* b) {
     return S2_OK;
 }
 
+// A note-off table staged for the next pipelined render (s2_bank_set_releases) is applied by that render's kernels.
+// An entry that writes the release row itself, renders outside the voice ranges or changes the ranges applies it
+// here first, on the bank's stream, so that edits take effect in call order.  Call after bank_drain.
+int apply_staged_table(s2_bank* b) {
+    if (b->n_sub <= 1 || b->table_pending < 0) return S2_OK;
+    CUDA_TRY(cudaStreamWaitEvent(b->stream, b->ev_stage[b->table_pending], 0));
+    CUDA_TRY(s2::launch_gather_u32(b->d_stage2[b->table_pending], b->d_params + (size_t)s2::P_ROW * b->vpad,
+                                   reinterpret_cast<uint32_t*>(b->d_params + (size_t)s2::P_RELEASE * b->vpad),
+                                   (uint32_t)b->n_voices, b->stream));
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    CUDA_TRY(cudaStreamSynchronize(b->stream));   // the staging buffer is free again before the next upload
+    b->table_pending = -1;
+    return S2_OK;
+}
+
 uint32_t sub_begin(const s2_bank* b, int k) {
     // contiguous slot ranges, multiples of 64 slots so that warps (32 or 64 slots) never straddle two
     const uint64_t groups = (b->n_voices + 63) / 64;
@@ -416,7 +431,11 @@ int bank_render_impl(s2_bank* b, size_t frames, float* d_voice_out, size_t row_s
     }
     b->ts_main_dirty = true;      // the general kernels below move the carried phase on the bank's stream
     if (b->n_sub > 1 && trace == s2::TRACE_NONE) return bank_render_pipelined(b, frames, d_voice_out, row_stride, d_bus_out);
-    if (b->n_sub > 1) { int rc = bank_drain(b); if (rc) return rc; }
+    if (b->n_sub > 1) {   // a trace: it renders the whole bank on the bank's stream
+        int rc = bank_drain(b);
+        if (rc == S2_OK) rc = apply_staged_table(b);
+        if (rc) return rc;
+    }
 
     const uint32_t n_warps = s2::render_warps((uint32_t)b->n_voices);
     float* partials = nullptr;
@@ -455,6 +474,8 @@ int bank_render_impl(s2_bank* b, size_t frames, float* d_voice_out, size_t row_s
     a.release_row = nullptr;
     CUDA_TRY(s2::launch_render(a, b->filter_kind, trace, b->stream));
     g_launches.fetch_add(1, std::memory_order_relaxed);
+    // the next pipelined render launches on the sub-streams, which do not wait for the bank's stream
+    if (b->n_sub > 1) CUDA_TRY(cudaStreamSynchronize(b->stream));
     if (d_bus_out && n_warps > 1) {
         CUDA_TRY(s2::launch_bus_reduce(partials, n_warps, frames, (uint32_t)frames, partials + (size_t)n_warps * frames,
                                        d_bus_out, b->stream, b->d_bus_counters, (size_t)s2::bus_segments(n_warps) * frames));
@@ -690,6 +711,7 @@ int s2_bank_set_voice(s2_bank* b, size_t index, const s2_voice_desc* voice) {
     if (rc) return rc;
     CUDA_TRY(cudaSetDevice(b->device));
     if ((rc = bank_drain(b)) != S2_OK) return rc;      // pipelined mode: per-voice edits are not pipelined
+    if ((rc = apply_staged_table(b)) != S2_OK) return rc;
     float hp[s2::P_COUNT], hs[s2::S_COUNT];
     const size_t slot = b->slot_of_voice[index];   // the voice keeps its slot (a changed kind makes that warp mixed)
     pack_voice(*voice, (uint32_t)index, hp, 1);
@@ -715,7 +737,7 @@ int s2_bank_release_voice(s2_bank* b, size_t index) {
     if (!b) return fail(S2_ERR_INVALID, "null bank");
     if (index >= b->n_voices) return fail(S2_ERR_INVALID, "voice index %zu out of range", index);
     CUDA_TRY(cudaSetDevice(b->device));
-    { int rc = bank_drain(b); if (rc) return rc; }
+    { int rc = bank_drain(b); if (rc == S2_OK) rc = apply_staged_table(b); if (rc) return rc; }
     const uint32_t rel = current_offset(b, index);   // release_frame_offset = current_frame_offset (synth.rs:75)
     CUDA_TRY(cudaMemcpyAsync(b->d_params + (size_t)s2::P_RELEASE * b->vpad + b->slot_of_voice[index], &rel,
                              sizeof rel, cudaMemcpyHostToDevice, b->stream));
@@ -853,16 +875,7 @@ int s2_bank_set_pipeline(s2_bank* b, int n_sub) {
     if (n_sub < 1 || n_sub > 8) return fail(S2_ERR_INVALID, "n_sub must be in [1, 8]");
     if (n_sub > 1 && b->ts_enabled) return fail(S2_ERR_INVALID, "time-split and pipelined voice ranges are exclusive");
     CUDA_TRY(cudaSetDevice(b->device));
-    { int rc = s2_bank_sync(b); if (rc) return rc; }
-    if (b->n_sub > 1 && b->table_pending >= 0) {
-        // a note-off table staged for the next pipelined render: apply it now, the ranges are about to change
-        CUDA_TRY(cudaStreamWaitEvent(b->stream, b->ev_stage[b->table_pending], 0));
-        CUDA_TRY(s2::launch_gather_u32(b->d_stage2[b->table_pending], b->d_params + (size_t)s2::P_ROW * b->vpad,
-                                       reinterpret_cast<uint32_t*>(b->d_params + (size_t)s2::P_RELEASE * b->vpad),
-                                       (uint32_t)b->n_voices, b->stream));
-        CUDA_TRY(cudaStreamSynchronize(b->stream));
-        b->table_pending = -1;
-    }
+    { int rc = s2_bank_sync(b); if (rc == S2_OK) rc = apply_staged_table(b); if (rc) return rc; }
     if (n_sub > 1) {
         for (int k = 0; k < n_sub; k++) {
             if (!b->sub[k]) CUDA_TRY(cudaStreamCreateWithFlags(&b->sub[k], cudaStreamNonBlocking));
