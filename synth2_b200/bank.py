@@ -18,6 +18,13 @@ def note_to_pitch(note: int) -> float:
     return float(lib().s2_note_to_pitch(int(note) & 0xFF))
 
 
+def _row_stride(buf, frames: int, given: int) -> int:
+    """The row stride in floats: `given` if set, else the buffer's own (a tensor's stride(0)), else `frames`."""
+    if given or buf is None:
+        return int(given)
+    return int(buf.stride(0)) if hasattr(buf, "stride") else int(frames)
+
+
 def default_voice(n: int = 1) -> np.ndarray:
     """`Synth::default_config()` (synth.rs:125-152) as n inactive voice descriptions."""
     one = np.zeros(1, dtype=VOICE_DESC)
@@ -72,30 +79,25 @@ class VoiceBank:
 
     # -- rendering (device buffers: anything with .data_ptr(), or a raw address)
     def render(self, frames: int, voice_out=None, row_stride: int = 0, bus_out=None):
-        if voice_out is not None and not row_stride:
-            row_stride = int(voice_out.stride(0)) if hasattr(voice_out, "stride") else int(frames)
-        check(lib().s2_bank_render(self._h, int(frames), ptr(voice_out), int(row_stride), ptr(bus_out)))
+        row_stride = _row_stride(voice_out, frames, row_stride)
+        check(lib().s2_bank_render(self._h, int(frames), ptr(voice_out), row_stride, ptr(bus_out)))
 
     def render_bus_host(self, frames: int, voice_out=None, row_stride: int = 0, out: np.ndarray = None):
         """Render and return the mono mix in host memory (the `Synth::sample` shape)."""
         if out is None:
             out = np.empty(int(frames), dtype=np.float32)
         assert out.dtype == np.float32 and out.flags.c_contiguous and out.size >= frames
-        if voice_out is not None and not row_stride:
-            row_stride = int(voice_out.stride(0)) if hasattr(voice_out, "stride") else int(frames)
-        check(lib().s2_bank_render_bus_host(self._h, int(frames), ptr(voice_out), int(row_stride), ptr(out)))
+        row_stride = _row_stride(voice_out, frames, row_stride)
+        check(lib().s2_bank_render_bus_host(self._h, int(frames), ptr(voice_out), row_stride, ptr(out)))
         return out
 
     def render_bus_host_async(self, frames: int, pinned_out, voice_out=None, row_stride: int = 0):
         """Streaming form: enqueue render + mix + D2H of the mix into pinned host memory, no sync."""
-        if voice_out is not None and not row_stride:
-            row_stride = int(voice_out.stride(0)) if hasattr(voice_out, "stride") else int(frames)
-        check(lib().s2_bank_render_bus_host_async(self._h, int(frames), ptr(voice_out), int(row_stride), ptr(pinned_out)))
+        row_stride = _row_stride(voice_out, frames, row_stride)
+        check(lib().s2_bank_render_bus_host_async(self._h, int(frames), ptr(voice_out), row_stride, ptr(pinned_out)))
 
     def trace_phase(self, frames: int, phase_out, row_stride: int = 0):
-        if not row_stride:
-            row_stride = int(phase_out.stride(0)) if hasattr(phase_out, "stride") else int(frames)
-        check(lib().s2_bank_trace_phase(self._h, int(frames), ptr(phase_out), int(row_stride)))
+        check(lib().s2_bank_trace_phase(self._h, int(frames), ptr(phase_out), _row_stride(phase_out, frames, row_stride)))
 
     def sync(self):
         check(lib().s2_bank_sync(self._h))

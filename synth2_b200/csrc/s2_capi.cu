@@ -21,32 +21,12 @@
 #include <vector>
 
 namespace {
-
 thread_local char g_err[512] = "";
 std::atomic<uint64_t> g_launches{0};
-
-int fail(int code, const char* fmt, ...) {
-    va_list ap;
-    va_start(ap, fmt);
-    vsnprintf(g_err, sizeof g_err, fmt, ap);
-    va_end(ap);
-    return code;
-}
-
-#define CUDA_TRY(expr)                                                                      \
-    do {                                                                                    \
-        cudaError_t e_ = (expr);                                                            \
-        if (e_ != cudaSuccess)                                                              \
-            return fail(S2_ERR_CUDA, "%s failed: %s (%s:%d)", #expr, cudaGetErrorString(e_), \
-                        __FILE__, __LINE__);                                                \
-    } while (0)
-
-bool finite_nonneg(float x) { return std::isfinite(x) && x >= 0.0f; }
-
 }  // namespace
 
 namespace s2 {
-// error reporting for the other host translation units of the library (s2_patch.cpp)
+// fills s2_last_error(); also the error reporting of the other host translation units of the library (s2_patch.cpp)
 int set_error(int code, const char* fmt, ...) {
     va_list ap;
     va_start(ap, fmt);
@@ -57,6 +37,18 @@ int set_error(int code, const char* fmt, ...) {
 }  // namespace s2
 
 namespace {
+
+constexpr auto fail = s2::set_error;
+
+#define CUDA_TRY(expr)                                                                      \
+    do {                                                                                    \
+        cudaError_t e_ = (expr);                                                            \
+        if (e_ != cudaSuccess)                                                              \
+            return fail(S2_ERR_CUDA, "%s failed: %s (%s:%d)", #expr, cudaGetErrorString(e_), \
+                        __FILE__, __LINE__);                                                \
+    } while (0)
+
+bool finite_nonneg(float x) { return std::isfinite(x) && x >= 0.0f; }
 
 int validate_voice(const s2_voice_desc& d, size_t index, uint32_t filter_kind = S2_FILTER_ONE_POLE) {
     // second-order filters: damping (band-pass: the quality factor) divides or scales the coefficients
@@ -129,14 +121,110 @@ struct VoiceBook {           // host mirror of what the device will hold, O(1) p
     uint32_t osc_kind;
 };
 
-}  // namespace
-
 // Partial-sum buffers of the pipelined mix.  The reduction of step i runs on the (high-priority) mix stream
 // while the sub-banks already render step i+1; with only two buffers step i+2 would have to wait for it,
 // and a reduction that is slow to get SM slots next to the render blocks then stalls the whole pipeline.
 constexpr int kMixBufs = 4;
 constexpr int kTsBufs = 4;                 // the phase pre-pass may run this many blocks ahead of the renders
 constexpr size_t kTsMaxVoices = 16384;     // beyond this a bank fills the machine with one voice per lane
+
+cudaError_t make_event(cudaEvent_t& e) { return e ? cudaSuccess : cudaEventCreateWithFlags(&e, cudaEventDisableTiming); }
+void destroy(cudaEvent_t e) { if (e) cudaEventDestroy(e); }
+void destroy(cudaStream_t s) { if (s) { cudaStreamSynchronize(s); cudaStreamDestroy(s); } }
+
+// Pipelined mode (s2_bank_set_pipeline): the bank is cut into n_sub contiguous slot ranges, each rendered on its
+// own internal stream.  Consecutive render calls then overlap across sub-banks (no device-wide barrier between
+// blocks), which keeps every SM sub-partition supplied with warps while the slower ones finish
+// (profiles/r1_notes.md: +14 % at 65,536 voices).
+struct Pipeline {
+    cudaStream_t sub[8] = {};
+    cudaStream_t mix = nullptr;           // bus reduction and copies of the pipelined mode
+    cudaStream_t upload = nullptr;        // note-off table uploads (independent of the mix stream)
+    cudaEvent_t ev_gather[8][2] = {};     // sub-bank k has applied the table staged in buffer q
+    cudaEvent_t ev_sub[8] = {};           // last work issued on sub-stream k
+    cudaEvent_t ev_mix[kMixBufs] = {};    // reduction of partial buffer p finished
+    cudaEvent_t ev_stage[2] = {};         // note-off table p has landed in its staging buffer
+    cudaEvent_t ev_tail = nullptr;        // last work issued on the mix stream
+    // Staging of the bulk note-off table, in voice order.  Buffer 0 also serves s2_bank_set_releases of a bank on
+    // one stream whose slots are permuted.
+    uint32_t* d_staging[2] = {};
+    float* d_partials[kMixBufs] = {};
+    size_t partials_cap = 0;              // floats, each of the kMixBufs buffers
+    uint64_t step = 0, table_step = 0;
+    int table_pending = -1;               // staging buffer index holding a table not yet applied, or -1
+
+    // What n_sub ranges need, created once and kept when the bank goes back to fewer ranges.
+    int create(int n_sub, size_t n_voices) {
+        for (int k = 0; k < n_sub; k++) {
+            if (!sub[k]) CUDA_TRY(cudaStreamCreateWithFlags(&sub[k], cudaStreamNonBlocking));
+            CUDA_TRY(make_event(ev_sub[k]));
+            CUDA_TRY(cudaEventRecord(ev_sub[k], sub[k]));
+        }
+        if (!mix) {
+            int prio_lo = 0, prio_hi = 0;
+            CUDA_TRY(cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi));
+            CUDA_TRY(cudaStreamCreateWithPriority(&mix, cudaStreamNonBlocking, prio_hi));
+        }
+        if (!upload) CUDA_TRY(cudaStreamCreateWithFlags(&upload, cudaStreamNonBlocking));
+        for (int k = 0; k < n_sub; k++)
+            for (int q = 0; q < 2; q++)
+                if (!ev_gather[k][q]) {
+                    CUDA_TRY(make_event(ev_gather[k][q]));
+                    CUDA_TRY(cudaEventRecord(ev_gather[k][q], sub[k]));
+                }
+        for (int i = 0; i < kMixBufs; i++) CUDA_TRY(make_event(ev_mix[i]));
+        for (int i = 0; i < 2; i++) {
+            CUDA_TRY(make_event(ev_stage[i]));
+            if (!d_staging[i]) CUDA_TRY(cudaMalloc(&d_staging[i], n_voices * sizeof(uint32_t)));
+        }
+        CUDA_TRY(make_event(ev_tail));
+        return S2_OK;
+    }
+
+    void release() {
+        for (int k = 0; k < 8; k++) {
+            destroy(sub[k]);
+            destroy(ev_sub[k]);
+            for (int q = 0; q < 2; q++) destroy(ev_gather[k][q]);
+        }
+        destroy(mix);
+        destroy(upload);
+        destroy(ev_tail);
+        for (int i = 0; i < 2; i++) { destroy(ev_stage[i]); cudaFree(d_staging[i]); }
+        for (int i = 0; i < kMixBufs; i++) { destroy(ev_mix[i]); cudaFree(d_partials[i]); }
+    }
+};
+
+// Time-split mode (s2_bank_set_time_split, s2_kernel_ts.cu): narrow one-pole banks render a block as 32 time
+// segments per voice.  The phase pre-pass runs on its own stream, ahead of the renders.
+struct TimeSplit {
+    bool enabled = false;
+    bool main_dirty = true;               // b->stream carries state writes the pre-pass stream has not seen
+    cudaStream_t stream = nullptr;        // the phase pre-pass
+    float* d_seg_phase[kTsBufs] = {};     // [n_voices][3][32] segment-start phases (and the two before) of block p
+    cudaEvent_t ev_k1[kTsBufs] = {}, ev_k2[kTsBufs] = {}, ev_main = nullptr;
+    uint64_t step = 0, blocks = 0;        // blocks: blocks rendered through the time-split kernels
+    std::vector<s2_voice_desc> descs;     // host copy of the voice descriptions (banks <= kTsMaxVoices only)
+
+    int create(size_t n_voices) {
+        if (!stream) CUDA_TRY(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
+        for (int i = 0; i < kTsBufs; i++) {
+            if (!d_seg_phase[i]) CUDA_TRY(cudaMalloc(&d_seg_phase[i], n_voices * 96 * sizeof(float)));
+            CUDA_TRY(make_event(ev_k1[i]));
+            CUDA_TRY(make_event(ev_k2[i]));
+        }
+        CUDA_TRY(make_event(ev_main));
+        return S2_OK;
+    }
+
+    void release() {
+        destroy(stream);
+        for (int i = 0; i < kTsBufs; i++) { destroy(ev_k1[i]); destroy(ev_k2[i]); cudaFree(d_seg_phase[i]); }
+        destroy(ev_main);
+    }
+};
+
+}  // namespace
 
 struct s2_bank {
     int device = 0;
@@ -161,34 +249,9 @@ struct s2_bank {
     std::vector<uint32_t> slot_of_voice, voice_of_slot;
     bool identity = true;
     uint32_t force_path = 0;      // test hook (S2_FORCE_PATH, see RenderArgs)
-    uint32_t* d_stage = nullptr;  // staging for the bulk note-off table when slots are permuted
-    // Pipelined mode (s2_bank_set_pipeline): the bank is cut into n_sub contiguous slot ranges, each
-    // rendered on its own internal stream.  Consecutive render calls then overlap across sub-banks (no
-    // device-wide barrier between blocks), which keeps every SM sub-partition supplied with warps while
-    // the slower ones finish (profiles/r1_notes.md: +14 % at 65,536 voices).
-    int n_sub = 1;
-    cudaStream_t sub[8] = {};
-    cudaStream_t mix = nullptr;           // bus reduction and copies of the pipelined mode
-    cudaStream_t upload = nullptr;        // note-off table uploads (independent of the mix stream)
-    cudaEvent_t ev_gather[8][2] = {};     // sub-bank k has applied the table staged in buffer q
-    cudaEvent_t ev_sub[8] = {};           // last work issued on sub-stream k
-    cudaEvent_t ev_mix[kMixBufs] = {};    // reduction of partial buffer p finished
-    cudaEvent_t ev_stage[2] = {};         // note-off table p has landed in its staging buffer
-    cudaEvent_t ev_tail = nullptr;        // last work issued on the mix stream
-    uint32_t* d_stage2[2] = {};
-    float* d_partials2[kMixBufs] = {};
-    size_t partials2_cap = 0;
-    uint64_t step = 0, table_step = 0;
-    int table_pending = -1;               // staging buffer index holding a table not yet applied, or -1
-    // Time-split mode (s2_bank_set_time_split, s2_kernel_ts.cu): narrow one-pole banks render a block as 32
-    // time segments per voice.  The phase pre-pass runs on its own stream, ahead of the renders.
-    bool ts_enabled = false;
-    bool ts_main_dirty = true;            // b->stream carries state writes the pre-pass stream has not seen
-    cudaStream_t ts = nullptr;
-    float* d_seg_phase[kTsBufs] = {};     // [n_voices][3][32] segment-start phases (and the two before) of block p
-    cudaEvent_t ev_k1[kTsBufs] = {}, ev_k2[kTsBufs] = {}, ev_main = nullptr;
-    uint64_t ts_step = 0, ts_blocks = 0;  // ts_blocks: blocks rendered through the time-split kernels
-    std::vector<s2_voice_desc> descs;     // host copy of the voice descriptions (banks <= kTsMaxVoices only)
+    int n_sub = 1;                // voice ranges of the pipelined mode; 1 = everything on the bank's stream
+    Pipeline pipe;
+    TimeSplit split;
     uint64_t total_frames = 0;
     uint64_t max_offset = 0;     // upper bound of any active voice's frame offset
     size_t n_sine = 0;
@@ -205,10 +268,26 @@ uint32_t current_offset(const s2_bank* b, size_t i) {
 
 // Waits (on the host) for everything the bank has issued on its internal streams.
 int bank_drain(s2_bank* b) {
-    for (int k = 0; k < b->n_sub && b->n_sub > 1; k++) CUDA_TRY(cudaStreamSynchronize(b->sub[k]));
-    if (b->mix) CUDA_TRY(cudaStreamSynchronize(b->mix));
-    if (b->upload) CUDA_TRY(cudaStreamSynchronize(b->upload));
-    if (b->ts) CUDA_TRY(cudaStreamSynchronize(b->ts));
+    for (int k = 0; k < b->n_sub && b->n_sub > 1; k++) CUDA_TRY(cudaStreamSynchronize(b->pipe.sub[k]));
+    if (b->pipe.mix) CUDA_TRY(cudaStreamSynchronize(b->pipe.mix));
+    if (b->pipe.upload) CUDA_TRY(cudaStreamSynchronize(b->pipe.upload));
+    if (b->split.stream) CUDA_TRY(cudaStreamSynchronize(b->split.stream));
+    return S2_OK;
+}
+
+// Grows the n device buffers bufs[0..n) to `need` floats each; they share the capacity `cap`.  The bank's internal
+// streams may still use the old buffers, so the bank (if any) is drained before they are freed.  A failed
+// allocation leaves that buffer null and cap 0.
+int grow(s2_bank* b, float** bufs, int n, size_t& cap, size_t need) {
+    if (need <= cap) return S2_OK;
+    if (b) { int rc = bank_drain(b); if (rc) return rc; }
+    for (int i = 0; i < n; i++) {
+        if (bufs[i]) CUDA_TRY(cudaFree(bufs[i]));
+        bufs[i] = nullptr;
+    }
+    cap = 0;
+    for (int i = 0; i < n; i++) CUDA_TRY(cudaMalloc(&bufs[i], need * sizeof(float)));
+    cap = need;
     return S2_OK;
 }
 
@@ -216,14 +295,62 @@ int bank_drain(s2_bank* b) {
 // An entry that writes the release row itself, renders outside the voice ranges or changes the ranges applies it
 // here first, on the bank's stream, so that edits take effect in call order.  Call after bank_drain.
 int apply_staged_table(s2_bank* b) {
-    if (b->n_sub <= 1 || b->table_pending < 0) return S2_OK;
-    CUDA_TRY(cudaStreamWaitEvent(b->stream, b->ev_stage[b->table_pending], 0));
-    CUDA_TRY(s2::launch_gather_u32(b->d_stage2[b->table_pending], b->d_params + (size_t)s2::P_ROW * b->vpad,
+    Pipeline& pl = b->pipe;
+    if (b->n_sub <= 1 || pl.table_pending < 0) return S2_OK;
+    CUDA_TRY(cudaStreamWaitEvent(b->stream, pl.ev_stage[pl.table_pending], 0));
+    CUDA_TRY(s2::launch_gather_u32(pl.d_staging[pl.table_pending], b->d_params + (size_t)s2::P_ROW * b->vpad,
                                    reinterpret_cast<uint32_t*>(b->d_params + (size_t)s2::P_RELEASE * b->vpad),
                                    (uint32_t)b->n_voices, b->stream));
     g_launches.fetch_add(1, std::memory_order_relaxed);
     CUDA_TRY(cudaStreamSynchronize(b->stream));   // the staging buffer is free again before the next upload
-    b->table_pending = -1;
+    pl.table_pending = -1;
+    return S2_OK;
+}
+
+// Before an entry that works on the bank's stream alone: every edit made so far is then on that stream, in call order.
+int settle_edits(s2_bank* b) {
+    int rc = bank_drain(b);
+    return rc ? rc : apply_staged_table(b);
+}
+
+// Every RenderArgs field from the bank, for the whole slot range, without bus partials or a staged table.
+s2::RenderArgs base_args(const s2_bank* b, size_t frames, float* d_voice_out, size_t row_stride) {
+    s2::RenderArgs a;
+    a.params = b->d_params;
+    a.state = b->d_state;
+    a.n_voices = (uint32_t)b->n_voices;
+    a.slot_begin = 0;
+    a.slot_end = (uint32_t)b->n_voices;
+    a.vpad = (uint32_t)b->vpad;
+    a.sample_rate = (float)b->sample_rate;
+    a.frames = (uint32_t)frames;
+    a.voice_out = d_voice_out;
+    a.row_stride = row_stride;
+    a.bus_partials = nullptr;
+    a.has_sine = b->n_sine ? 1u : 0u;
+    a.one = 1.0f;
+    a.force_path = b->force_path;
+    a.staged_release = nullptr;
+    a.release_row = nullptr;
+    return a;
+}
+
+// Floats of a partial-sum buffer: one row of `frames` per warp, then the scratch of the wide bus reduction.
+size_t partials_floats(uint32_t n_warps, size_t frames) {
+    return (size_t)n_warps * frames + s2::bus_scratch_floats(n_warps, (uint32_t)frames);
+}
+
+// The bus from the partial rows the render's warps wrote (partials_floats layout), on `st`.  A single warp's row is
+// the bus: the default path renders it straight there (partials == bus), the pipelined path copies it.
+int mix_partials(const s2_bank* b, float* partials, uint32_t n_warps, size_t frames, float* bus, cudaStream_t st) {
+    if (partials == bus) return S2_OK;
+    if (n_warps == 1) {
+        CUDA_TRY(cudaMemcpyAsync(bus, partials, frames * sizeof(float), cudaMemcpyDeviceToDevice, st));
+        return S2_OK;
+    }
+    CUDA_TRY(s2::launch_bus_reduce(partials, n_warps, frames, (uint32_t)frames, bus, st, b->d_bus_counters,
+                                   partials + (size_t)n_warps * frames));
+    g_launches.fetch_add(1, std::memory_order_relaxed);
     return S2_OK;
 }
 
@@ -236,73 +363,42 @@ uint32_t sub_begin(const s2_bank* b, int k) {
 }
 
 int bank_render_pipelined(s2_bank* b, size_t frames, float* d_voice_out, size_t row_stride, float* d_bus_out) {
+    Pipeline& pl = b->pipe;
     const uint32_t n_warps = s2::render_warps((uint32_t)b->n_voices);
-    const int p = (int)(b->step % (uint64_t)kMixBufs);
-    float* partials = nullptr;
+    const int p = (int)(pl.step % (uint64_t)kMixBufs);
+    s2::RenderArgs a = base_args(b, frames, d_voice_out, row_stride);
     if (d_bus_out) {
-        const size_t need = ((size_t)n_warps + s2::bus_segments(n_warps)) * frames;
-        if (need > b->partials2_cap) {
-            int rc = bank_drain(b);
-            if (rc) return rc;
-            for (int i = 0; i < kMixBufs; i++) {
-                if (b->d_partials2[i]) CUDA_TRY(cudaFree(b->d_partials2[i]));
-                b->d_partials2[i] = nullptr;
-            }
-            b->partials2_cap = 0;
-            for (int i = 0; i < kMixBufs; i++) CUDA_TRY(cudaMalloc(&b->d_partials2[i], need * sizeof(float)));
-            b->partials2_cap = need;
-        }
-        partials = b->d_partials2[p];
+        int rc = grow(b, pl.d_partials, kMixBufs, pl.partials_cap, partials_floats(n_warps, frames));
+        if (rc) return rc;
+        a.bus_partials = pl.d_partials[p];
     }
-    s2::RenderArgs a;
-    a.params = b->d_params;
-    a.state = b->d_state;
-    a.n_voices = (uint32_t)b->n_voices;
-    a.vpad = (uint32_t)b->vpad;
-    a.sample_rate = (float)b->sample_rate;
-    a.frames = (uint32_t)frames;
-    a.voice_out = d_voice_out;
-    a.row_stride = row_stride;
-    a.bus_partials = partials;
-    a.has_sine = b->n_sine ? 1u : 0u;
-    a.one = 1.0f;
-    a.force_path = b->force_path;
-    a.staged_release = nullptr;
-    a.release_row = nullptr;
     uint32_t* release_row = reinterpret_cast<uint32_t*>(b->d_params + (size_t)s2::P_RELEASE * b->vpad);
     for (int k = 0; k < b->n_sub; k++) {
         a.slot_begin = sub_begin(b, k);
         a.slot_end = sub_begin(b, k + 1);
         if (a.slot_begin >= a.slot_end) continue;
-        cudaStream_t sk = b->sub[k];
-        a.staged_release = nullptr;
-        a.release_row = nullptr;
-        if (b->table_pending >= 0) {
+        cudaStream_t sk = pl.sub[k];
+        if (pl.table_pending >= 0) {
             // the staged note-off table: this sub-bank's render applies it to its own slots first (kernel prologue),
             // ordered between its own renders
-            CUDA_TRY(cudaStreamWaitEvent(sk, b->ev_stage[b->table_pending], 0));
-            a.staged_release = b->d_stage2[b->table_pending];
+            CUDA_TRY(cudaStreamWaitEvent(sk, pl.ev_stage[pl.table_pending], 0));
+            a.staged_release = pl.d_staging[pl.table_pending];
             a.release_row = release_row;
         }
-        if (d_bus_out && b->step >= (uint64_t)kMixBufs) CUDA_TRY(cudaStreamWaitEvent(sk, b->ev_mix[p], 0));   // partials[p] are free again
+        if (d_bus_out && pl.step >= (uint64_t)kMixBufs) CUDA_TRY(cudaStreamWaitEvent(sk, pl.ev_mix[p], 0));   // partials[p] are free again
         CUDA_TRY(s2::launch_render(a, b->filter_kind, s2::TRACE_NONE, sk));
         g_launches.fetch_add(1, std::memory_order_relaxed);
-        if (b->table_pending >= 0) CUDA_TRY(cudaEventRecord(b->ev_gather[k][b->table_pending], sk));   // staging buffer read
-        CUDA_TRY(cudaEventRecord(b->ev_sub[k], sk));
+        if (pl.table_pending >= 0) CUDA_TRY(cudaEventRecord(pl.ev_gather[k][pl.table_pending], sk));   // staging buffer read
+        CUDA_TRY(cudaEventRecord(pl.ev_sub[k], sk));
     }
-    b->table_pending = -1;
+    pl.table_pending = -1;
     if (d_bus_out) {
-        for (int k = 0; k < b->n_sub; k++) CUDA_TRY(cudaStreamWaitEvent(b->mix, b->ev_sub[k], 0));
-        if (n_warps == 1) {
-            CUDA_TRY(cudaMemcpyAsync(d_bus_out, partials, frames * sizeof(float), cudaMemcpyDeviceToDevice, b->mix));
-        } else {
-            CUDA_TRY(s2::launch_bus_reduce(partials, n_warps, frames, (uint32_t)frames, partials + (size_t)n_warps * frames,
-                                           d_bus_out, b->mix, b->d_bus_counters, (size_t)s2::bus_segments(n_warps) * frames));
-            g_launches.fetch_add(1, std::memory_order_relaxed);
-        }
-        CUDA_TRY(cudaEventRecord(b->ev_mix[p], b->mix));
+        for (int k = 0; k < b->n_sub; k++) CUDA_TRY(cudaStreamWaitEvent(pl.mix, pl.ev_sub[k], 0));
+        int rc = mix_partials(b, a.bus_partials, n_warps, frames, d_bus_out, pl.mix);
+        if (rc) return rc;
+        CUDA_TRY(cudaEventRecord(pl.ev_mix[p], pl.mix));
     }
-    b->step++;
+    pl.step++;
     b->total_frames += frames;
     b->max_offset += frames;
     return S2_OK;
@@ -315,15 +411,14 @@ float host_ms_as_samples(float ms, float sr) { return sr * (ms / 1000.0f); }
 // block (no pitch modulation).  Returns 0 = no, 1 = yes and every cutoff rests too (mod envelope unused by the
 // cutoff, or in sustain / end until the block ends), 2 = yes but some cutoff follows a ramping mod envelope
 // (per-frame coefficients).  Conservative: anything unsure renders the general way.
-int ts_block_class(const s2_bank* b, size_t frames, const float* d_voice_out, const float* d_bus_out) {
-    if (!b->ts_enabled || !d_voice_out) return 0;                               // the mix is summed from the rows
-    (void)d_bus_out;
+int ts_block_class(const s2_bank* b, size_t frames, const float* d_voice_out) {
+    if (!b->split.enabled || !d_voice_out) return 0;                            // the mix is summed from the rows
     if (frames < 1024 || (frames & 1023u) != 0 || frames > (1u << 24)) return 0;   // 32 segments of whole chunks
     const float sr = (float)b->sample_rate;
     int cls = 1;
     for (size_t i = 0; i < b->n_voices; i++) {
         if (!b->book[i].active) continue;
-        const s2_voice_desc& d = b->descs[i];
+        const s2_voice_desc& d = b->split.descs[i];
         if (d.mod_env_to_osc_freq != 0.0f) return 0;
         const uint64_t n0 = current_offset(b, i);
         if (n0 + frames > (1ull << 24)) return 0;
@@ -347,59 +442,35 @@ int ts_block_class(const s2_bank* b, size_t frames, const float* d_voice_out, co
 
 int bank_render_time_split(s2_bank* b, size_t frames, float* d_voice_out, size_t row_stride, float* d_bus_out,
                            bool moving) {
-    const int p = (int)(b->ts_step % (uint64_t)kTsBufs);
-    s2::RenderArgs a;
-    a.params = b->d_params;
-    a.state = b->d_state;
-    a.n_voices = (uint32_t)b->n_voices;
-    a.slot_begin = 0;
-    a.slot_end = (uint32_t)b->n_voices;
-    a.vpad = (uint32_t)b->vpad;
-    a.sample_rate = (float)b->sample_rate;
-    a.frames = (uint32_t)frames;
-    a.voice_out = d_voice_out;
-    a.row_stride = row_stride;
-    a.bus_partials = nullptr;
-    a.has_sine = b->n_sine ? 1u : 0u;
-    a.one = 1.0f;
-    a.force_path = b->force_path;
-    a.staged_release = nullptr;
-    a.release_row = nullptr;
-    if (b->ts_main_dirty) {
+    TimeSplit& ts = b->split;
+    const int p = (int)(ts.step % (uint64_t)kTsBufs);
+    const s2::RenderArgs a = base_args(b, frames, d_voice_out, row_stride);
+    if (ts.main_dirty) {
         // the pre-pass reads the carried phase: order it after whatever the bank's stream wrote
-        CUDA_TRY(cudaEventRecord(b->ev_main, b->stream));
-        CUDA_TRY(cudaStreamWaitEvent(b->ts, b->ev_main, 0));
-        b->ts_main_dirty = false;
+        CUDA_TRY(cudaEventRecord(ts.ev_main, b->stream));
+        CUDA_TRY(cudaStreamWaitEvent(ts.stream, ts.ev_main, 0));
+        ts.main_dirty = false;
     }
-    if (b->ts_step >= (uint64_t)kTsBufs) CUDA_TRY(cudaStreamWaitEvent(b->ts, b->ev_k2[p], 0));   // seg_phase[p] is free again
-    CUDA_TRY(s2::launch_ts_phase(a, b->d_seg_phase[p], b->ts));
-    CUDA_TRY(cudaEventRecord(b->ev_k1[p], b->ts));
-    CUDA_TRY(cudaStreamWaitEvent(b->stream, b->ev_k1[p], 0));
-    CUDA_TRY(s2::launch_ts_render(a, b->filter_kind, moving, b->d_seg_phase[p], b->stream));
-    CUDA_TRY(cudaEventRecord(b->ev_k2[p], b->stream));
+    if (ts.step >= (uint64_t)kTsBufs) CUDA_TRY(cudaStreamWaitEvent(ts.stream, ts.ev_k2[p], 0));   // seg_phase[p] is free again
+    CUDA_TRY(s2::launch_ts_phase(a, ts.d_seg_phase[p], ts.stream));
+    CUDA_TRY(cudaEventRecord(ts.ev_k1[p], ts.stream));
+    CUDA_TRY(cudaStreamWaitEvent(b->stream, ts.ev_k1[p], 0));
+    CUDA_TRY(s2::launch_ts_render(a, b->filter_kind, moving, ts.d_seg_phase[p], b->stream));
+    CUDA_TRY(cudaEventRecord(ts.ev_k2[p], b->stream));
     g_launches.fetch_add(2, std::memory_order_relaxed);
     if (d_bus_out) {
         // one warp rendered one voice: the output rows (silent voices included, as zeros) are the partial sums.
         // Up to 32 voices they are added in voice order, as on the default path; wider banks take the reduction
-        // kernel's fixed tree.
+        // kernel's fixed tree (its one-frame-per-lane form, which needs no scratch).
         const uint32_t nv = (uint32_t)b->n_voices;
-        if (nv <= 32u) {
+        if (nv <= 32u)
             CUDA_TRY(s2::launch_ts_mix_rows(d_voice_out, nv, row_stride, (uint32_t)frames, d_bus_out, b->stream));
-            g_launches.fetch_add(1, std::memory_order_relaxed);
-        } else {
-            const size_t need = (size_t)s2::bus_segments(nv) * frames;
-            if (need > b->partials_cap) {
-                if (b->d_partials) CUDA_TRY(cudaFree(b->d_partials));
-                b->d_partials = nullptr; b->partials_cap = 0;
-                CUDA_TRY(cudaMalloc(&b->d_partials, need * sizeof(float)));
-                b->partials_cap = need;
-            }
-            CUDA_TRY(s2::launch_bus_reduce(d_voice_out, nv, row_stride, (uint32_t)frames, b->d_partials, d_bus_out, b->stream));
-            g_launches.fetch_add(1, std::memory_order_relaxed);
-        }
+        else
+            CUDA_TRY(s2::launch_bus_reduce(d_voice_out, nv, row_stride, (uint32_t)frames, d_bus_out, b->stream));
+        g_launches.fetch_add(1, std::memory_order_relaxed);
     }
-    b->ts_step++;
-    b->ts_blocks++;
+    ts.step++;
+    ts.blocks++;
     b->total_frames += frames;
     b->max_offset += frames;
     return S2_OK;
@@ -426,60 +497,34 @@ int bank_render_impl(s2_bank* b, size_t frames, float* d_voice_out, size_t row_s
     }
     CUDA_TRY(cudaSetDevice(b->device));
     if (trace == s2::TRACE_NONE) {
-        const int cls = ts_block_class(b, frames, d_voice_out, d_bus_out);
+        const int cls = ts_block_class(b, frames, d_voice_out);
         if (cls) return bank_render_time_split(b, frames, d_voice_out, row_stride, d_bus_out, cls == 2);
     }
-    b->ts_main_dirty = true;      // the general kernels below move the carried phase on the bank's stream
+    b->split.main_dirty = true;   // the general kernels below move the carried phase on the bank's stream
     if (b->n_sub > 1 && trace == s2::TRACE_NONE) return bank_render_pipelined(b, frames, d_voice_out, row_stride, d_bus_out);
     if (b->n_sub > 1) {   // a trace: it renders the whole bank on the bank's stream
-        int rc = bank_drain(b);
-        if (rc == S2_OK) rc = apply_staged_table(b);
+        int rc = settle_edits(b);
         if (rc) return rc;
     }
 
     const uint32_t n_warps = s2::render_warps((uint32_t)b->n_voices);
-    float* partials = nullptr;
+    s2::RenderArgs a = base_args(b, frames, d_voice_out, row_stride);
     if (d_bus_out) {
         if (n_warps == 1) {
-            partials = d_bus_out;   // a single warp sums its voices in index order: that IS the bus
+            a.bus_partials = d_bus_out;   // a single warp sums its voices in index order: that IS the bus
         } else {
-            // per-warp partials followed by the stage-1 segment sums of the bus reduction
-            const size_t need = ((size_t)n_warps + s2::bus_segments(n_warps)) * frames;
-            if (need > b->partials_cap) {
-                if (b->d_partials) CUDA_TRY(cudaFree(b->d_partials));
-                b->d_partials = nullptr; b->partials_cap = 0;
-                CUDA_TRY(cudaMalloc(&b->d_partials, need * sizeof(float)));
-                b->partials_cap = need;
-            }
-            partials = b->d_partials;
+            int rc = grow(b, &b->d_partials, 1, b->partials_cap, partials_floats(n_warps, frames));
+            if (rc) return rc;
+            a.bus_partials = b->d_partials;
         }
     }
-
-    s2::RenderArgs a;
-    a.params = b->d_params;
-    a.state = b->d_state;
-    a.n_voices = (uint32_t)b->n_voices;
-    a.slot_begin = 0;
-    a.slot_end = (uint32_t)b->n_voices;
-    a.vpad = (uint32_t)b->vpad;
-    a.sample_rate = (float)b->sample_rate;
-    a.frames = (uint32_t)frames;
-    a.voice_out = d_voice_out;
-    a.row_stride = row_stride;
-    a.bus_partials = partials;
-    a.has_sine = b->n_sine ? 1u : 0u;
-    a.one = 1.0f;
-    a.force_path = b->force_path;
-    a.staged_release = nullptr;
-    a.release_row = nullptr;
     CUDA_TRY(s2::launch_render(a, b->filter_kind, trace, b->stream));
     g_launches.fetch_add(1, std::memory_order_relaxed);
     // the next pipelined render launches on the sub-streams, which do not wait for the bank's stream
     if (b->n_sub > 1) CUDA_TRY(cudaStreamSynchronize(b->stream));
-    if (d_bus_out && n_warps > 1) {
-        CUDA_TRY(s2::launch_bus_reduce(partials, n_warps, frames, (uint32_t)frames, partials + (size_t)n_warps * frames,
-                                       d_bus_out, b->stream, b->d_bus_counters, (size_t)s2::bus_segments(n_warps) * frames));
-        g_launches.fetch_add(1, std::memory_order_relaxed);
+    if (d_bus_out) {
+        int rc = mix_partials(b, a.bus_partials, n_warps, frames, d_bus_out, b->stream);
+        if (rc) return rc;
     }
     b->total_frames += frames;
     b->max_offset += frames;
@@ -559,7 +604,7 @@ int s2_bank_create(int device, uint32_t sample_rate, uint32_t filter_kind, size_
     b->n_voices = n_voices;
     b->vpad = (n_voices + 63) & ~(size_t)63;
     b->book.resize(n_voices);
-    if (n_voices <= kTsMaxVoices) b->descs.assign(voices, voices + n_voices);
+    if (n_voices <= kTsMaxVoices) b->split.descs.assign(voices, voices + n_voices);
     if (const char* f = getenv("S2_FORCE_PATH")) b->force_path = (f[0] >= '1' && f[0] <= '3') ? (uint32_t)(f[0] - '0') : 0u;   // test hook
 
     b->voice_of_slot.resize(n_voices);
@@ -670,35 +715,13 @@ void s2_bank_destroy(s2_bank* b) {
     cudaSetDevice(b->device);
     bank_drain(b);
     cudaStreamSynchronize(b->stream);
+    b->pipe.release();
+    b->split.release();
     cudaFree(b->d_params);
     cudaFree(b->d_state);
     cudaFree(b->d_partials);
     cudaFree(b->d_bus_counters);
     cudaFree(b->d_bus);
-    cudaFree(b->d_stage);
-    for (int k = 0; k < 8; k++) {
-        if (b->sub[k]) { cudaStreamSynchronize(b->sub[k]); cudaStreamDestroy(b->sub[k]); }
-        if (b->ev_sub[k]) cudaEventDestroy(b->ev_sub[k]);
-    }
-    if (b->mix) { cudaStreamSynchronize(b->mix); cudaStreamDestroy(b->mix); }
-    if (b->upload) { cudaStreamSynchronize(b->upload); cudaStreamDestroy(b->upload); }
-    for (int k = 0; k < 8; k++) for (int q = 0; q < 2; q++) if (b->ev_gather[k][q]) cudaEventDestroy(b->ev_gather[k][q]);
-    for (int i = 0; i < 2; i++) {
-        if (b->ev_stage[i]) cudaEventDestroy(b->ev_stage[i]);
-        cudaFree(b->d_stage2[i]);
-    }
-    for (int i = 0; i < kMixBufs; i++) {
-        if (b->ev_mix[i]) cudaEventDestroy(b->ev_mix[i]);
-        cudaFree(b->d_partials2[i]);
-    }
-    if (b->ev_tail) cudaEventDestroy(b->ev_tail);
-    if (b->ts) { cudaStreamSynchronize(b->ts); cudaStreamDestroy(b->ts); }
-    for (int i = 0; i < kTsBufs; i++) {
-        if (b->ev_k1[i]) cudaEventDestroy(b->ev_k1[i]);
-        if (b->ev_k2[i]) cudaEventDestroy(b->ev_k2[i]);
-        cudaFree(b->d_seg_phase[i]);
-    }
-    if (b->ev_main) cudaEventDestroy(b->ev_main);
     delete b;
 }
 
@@ -710,8 +733,7 @@ int s2_bank_set_voice(s2_bank* b, size_t index, const s2_voice_desc* voice) {
     int rc = validate_voice(*voice, index, b->filter_kind);
     if (rc) return rc;
     CUDA_TRY(cudaSetDevice(b->device));
-    if ((rc = bank_drain(b)) != S2_OK) return rc;      // pipelined mode: per-voice edits are not pipelined
-    if ((rc = apply_staged_table(b)) != S2_OK) return rc;
+    if ((rc = settle_edits(b)) != S2_OK) return rc;    // pipelined mode: per-voice edits are not pipelined
     float hp[s2::P_COUNT], hs[s2::S_COUNT];
     const size_t slot = b->slot_of_voice[index];   // the voice keeps its slot (a changed kind makes that warp mixed)
     pack_voice(*voice, (uint32_t)index, hp, 1);
@@ -728,7 +750,7 @@ int s2_bank_set_voice(s2_bank* b, size_t index, const s2_voice_desc* voice) {
     if (b->book[index].osc_kind == S2_OSC_SINE) b->n_sine--;
     if (voice->osc_kind == S2_OSC_SINE) b->n_sine++;
     b->book[index] = {voice->frame_offset, b->total_frames, voice->active ? 1u : 0u, voice->osc_kind};
-    if (!b->descs.empty()) b->descs[index] = *voice;
+    if (!b->split.descs.empty()) b->split.descs[index] = *voice;
     if (voice->active && voice->frame_offset > b->max_offset) b->max_offset = voice->frame_offset;
     return S2_OK;
 }
@@ -737,35 +759,36 @@ int s2_bank_release_voice(s2_bank* b, size_t index) {
     if (!b) return fail(S2_ERR_INVALID, "null bank");
     if (index >= b->n_voices) return fail(S2_ERR_INVALID, "voice index %zu out of range", index);
     CUDA_TRY(cudaSetDevice(b->device));
-    { int rc = bank_drain(b); if (rc == S2_OK) rc = apply_staged_table(b); if (rc) return rc; }
+    { int rc = settle_edits(b); if (rc) return rc; }
     const uint32_t rel = current_offset(b, index);   // release_frame_offset = current_frame_offset (synth.rs:75)
     CUDA_TRY(cudaMemcpyAsync(b->d_params + (size_t)s2::P_RELEASE * b->vpad + b->slot_of_voice[index], &rel,
                              sizeof rel, cudaMemcpyHostToDevice, b->stream));
     CUDA_TRY(cudaStreamSynchronize(b->stream));
-    if (!b->descs.empty()) b->descs[index].release_offset = rel;
+    if (!b->split.descs.empty()) b->split.descs[index].release_offset = rel;
     return S2_OK;
 }
 
 int s2_bank_set_releases(s2_bank* b, const uint32_t* h_release) {
     if (!b || !h_release) return fail(S2_ERR_INVALID, "null argument");
     CUDA_TRY(cudaSetDevice(b->device));
-    for (size_t i = 0; i < b->descs.size(); i++) b->descs[i].release_offset = h_release[i];
+    for (size_t i = 0; i < b->split.descs.size(); i++) b->split.descs[i].release_offset = h_release[i];
+    Pipeline& pl = b->pipe;
     if (b->n_sub > 1) {
         // stage the table on the mix stream; every sub-bank applies it to its own slots right before its
         // next render (bank_render_pipelined), so no sub-bank waits for another
-        const int q = (int)(b->table_step & 1u);
-        if (b->table_pending >= 0) {
+        const int q = (int)(pl.table_step & 1u);
+        if (pl.table_pending >= 0) {
             // two tables without a render in between: the older one is simply superseded
-            b->table_pending = -1;
-            b->table_step--;
+            pl.table_pending = -1;
+            pl.table_step--;
             return s2_bank_set_releases(b, h_release);
         }
-        if (b->table_step >= 2)     // buffer q still feeds the gathers of the table staged two uploads ago
-            for (int k = 0; k < b->n_sub; k++) CUDA_TRY(cudaStreamWaitEvent(b->upload, b->ev_gather[k][q], 0));
-        CUDA_TRY(cudaMemcpyAsync(b->d_stage2[q], h_release, b->n_voices * sizeof(uint32_t), cudaMemcpyHostToDevice, b->upload));
-        CUDA_TRY(cudaEventRecord(b->ev_stage[q], b->upload));
-        b->table_pending = q;
-        b->table_step++;
+        if (pl.table_step >= 2)     // buffer q still feeds the gathers of the table staged two uploads ago
+            for (int k = 0; k < b->n_sub; k++) CUDA_TRY(cudaStreamWaitEvent(pl.upload, pl.ev_gather[k][q], 0));
+        CUDA_TRY(cudaMemcpyAsync(pl.d_staging[q], h_release, b->n_voices * sizeof(uint32_t), cudaMemcpyHostToDevice, pl.upload));
+        CUDA_TRY(cudaEventRecord(pl.ev_stage[q], pl.upload));
+        pl.table_pending = q;
+        pl.table_step++;
         return S2_OK;
     }
     uint32_t* row = reinterpret_cast<uint32_t*>(b->d_params + (size_t)s2::P_RELEASE * b->vpad);
@@ -773,9 +796,11 @@ int s2_bank_set_releases(s2_bank* b, const uint32_t* h_release) {
         CUDA_TRY(cudaMemcpyAsync(row, h_release, b->n_voices * sizeof(uint32_t), cudaMemcpyHostToDevice, b->stream));
         return S2_OK;
     }
-    if (!b->d_stage) CUDA_TRY(cudaMalloc(&b->d_stage, b->n_voices * sizeof(uint32_t)));
-    CUDA_TRY(cudaMemcpyAsync(b->d_stage, h_release, b->n_voices * sizeof(uint32_t), cudaMemcpyHostToDevice, b->stream));
-    CUDA_TRY(s2::launch_gather_u32(b->d_stage, b->d_params + (size_t)s2::P_ROW * b->vpad, row,
+    // Permuted slots on one stream: stage in voice order, gather into slot order.  Staging buffer 0 is free here:
+    // s2_bank_set_pipeline synchronises every stream when the ranges change, and no table is pending while n_sub == 1.
+    if (!pl.d_staging[0]) CUDA_TRY(cudaMalloc(&pl.d_staging[0], b->n_voices * sizeof(uint32_t)));
+    CUDA_TRY(cudaMemcpyAsync(pl.d_staging[0], h_release, b->n_voices * sizeof(uint32_t), cudaMemcpyHostToDevice, b->stream));
+    CUDA_TRY(s2::launch_gather_u32(pl.d_staging[0], b->d_params + (size_t)s2::P_ROW * b->vpad, row,
                                    (uint32_t)b->n_voices, b->stream));
     g_launches.fetch_add(1, std::memory_order_relaxed);
     return S2_OK;
@@ -802,19 +827,15 @@ int s2_bank_render_bus_host_async(s2_bank* b, size_t frames, float* d_voice_out,
     if (!b || !h_bus_out) return fail(S2_ERR_INVALID, "null argument");
     if (frames == 0) return S2_OK;
     CUDA_TRY(cudaSetDevice(b->device));
-    if (frames > b->bus_cap) {
-        if (b->d_bus) CUDA_TRY(cudaFree(b->d_bus));
-        b->d_bus = nullptr; b->bus_cap = 0;
-        CUDA_TRY(cudaMalloc(&b->d_bus, frames * sizeof(float)));
-        b->bus_cap = frames;
-    }
-    int rc = bank_render_impl(b, frames, d_voice_out, row_stride, b->d_bus, s2::TRACE_NONE);
+    int rc = grow(b, &b->d_bus, 1, b->bus_cap, frames);
+    if (rc) return rc;
+    rc = bank_render_impl(b, frames, d_voice_out, row_stride, b->d_bus, s2::TRACE_NONE);
     if (rc) return rc;
     if (b->n_sub > 1) {
         // pipelined: the mix lives on the bank's mix stream; the caller's stream only waits for the copy
-        CUDA_TRY(cudaMemcpyAsync(h_bus_out, b->d_bus, frames * sizeof(float), cudaMemcpyDeviceToHost, b->mix));
-        CUDA_TRY(cudaEventRecord(b->ev_tail, b->mix));
-        CUDA_TRY(cudaStreamWaitEvent(b->stream, b->ev_tail, 0));
+        CUDA_TRY(cudaMemcpyAsync(h_bus_out, b->d_bus, frames * sizeof(float), cudaMemcpyDeviceToHost, b->pipe.mix));
+        CUDA_TRY(cudaEventRecord(b->pipe.ev_tail, b->pipe.mix));
+        CUDA_TRY(cudaStreamWaitEvent(b->stream, b->pipe.ev_tail, 0));
         return S2_OK;
     }
     CUDA_TRY(cudaMemcpyAsync(h_bus_out, b->d_bus, frames * sizeof(float), cudaMemcpyDeviceToHost, b->stream));
@@ -873,39 +894,14 @@ int s2_bank_sync(s2_bank* b) {
 int s2_bank_set_pipeline(s2_bank* b, int n_sub) {
     if (!b) return fail(S2_ERR_INVALID, "null bank");
     if (n_sub < 1 || n_sub > 8) return fail(S2_ERR_INVALID, "n_sub must be in [1, 8]");
-    if (n_sub > 1 && b->ts_enabled) return fail(S2_ERR_INVALID, "time-split and pipelined voice ranges are exclusive");
+    if (n_sub > 1 && b->split.enabled) return fail(S2_ERR_INVALID, "time-split and pipelined voice ranges are exclusive");
     CUDA_TRY(cudaSetDevice(b->device));
-    { int rc = s2_bank_sync(b); if (rc == S2_OK) rc = apply_staged_table(b); if (rc) return rc; }
-    if (n_sub > 1) {
-        for (int k = 0; k < n_sub; k++) {
-            if (!b->sub[k]) CUDA_TRY(cudaStreamCreateWithFlags(&b->sub[k], cudaStreamNonBlocking));
-            if (!b->ev_sub[k]) CUDA_TRY(cudaEventCreateWithFlags(&b->ev_sub[k], cudaEventDisableTiming));
-            CUDA_TRY(cudaEventRecord(b->ev_sub[k], b->sub[k]));
-        }
-        if (!b->mix) {
-            int prio_lo = 0, prio_hi = 0;
-            CUDA_TRY(cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi));
-            CUDA_TRY(cudaStreamCreateWithPriority(&b->mix, cudaStreamNonBlocking, prio_hi));
-        }
-        if (!b->upload) CUDA_TRY(cudaStreamCreateWithFlags(&b->upload, cudaStreamNonBlocking));
-        for (int k = 0; k < n_sub; k++)
-            for (int q = 0; q < 2; q++)
-                if (!b->ev_gather[k][q]) {
-                    CUDA_TRY(cudaEventCreateWithFlags(&b->ev_gather[k][q], cudaEventDisableTiming));
-                    CUDA_TRY(cudaEventRecord(b->ev_gather[k][q], b->sub[k]));
-                }
-        for (int i = 0; i < kMixBufs; i++)
-            if (!b->ev_mix[i]) CUDA_TRY(cudaEventCreateWithFlags(&b->ev_mix[i], cudaEventDisableTiming));
-        for (int i = 0; i < 2; i++) {
-            if (!b->ev_stage[i]) CUDA_TRY(cudaEventCreateWithFlags(&b->ev_stage[i], cudaEventDisableTiming));
-            if (!b->d_stage2[i]) CUDA_TRY(cudaMalloc(&b->d_stage2[i], b->n_voices * sizeof(uint32_t)));
-        }
-        if (!b->ev_tail) CUDA_TRY(cudaEventCreateWithFlags(&b->ev_tail, cudaEventDisableTiming));
-    }
+    { int rc = s2_bank_sync(b); if (rc == S2_OK) rc = settle_edits(b); if (rc) return rc; }
+    if (n_sub > 1) { int rc = b->pipe.create(n_sub, b->n_voices); if (rc) return rc; }
     b->n_sub = n_sub;
-    b->step = 0;
-    b->table_step = 0;
-    b->table_pending = -1;
+    b->pipe.step = 0;
+    b->pipe.table_step = 0;
+    b->pipe.table_pending = -1;
     return S2_OK;
 }
 
@@ -913,28 +909,22 @@ int s2_bank_set_time_split(s2_bank* b, int enable) {
     if (!b) return fail(S2_ERR_INVALID, "null bank");
     CUDA_TRY(cudaSetDevice(b->device));
     { int rc = s2_bank_sync(b); if (rc) return rc; }
-    if (!enable) { b->ts_enabled = false; return S2_OK; }
+    if (!enable) { b->split.enabled = false; return S2_OK; }
     if (b->filter_kind > S2_FILTER_BIQUAD_LP)
         return fail(S2_ERR_INVALID, "time-split rendering knows the one-pole and the second-order low-pass filters");
     if (b->n_voices > kTsMaxVoices)
         return fail(S2_ERR_INVALID, "time-split rendering is for narrow banks (<= %zu voices)", kTsMaxVoices);
     if (b->n_sub > 1) return fail(S2_ERR_INVALID, "time-split and pipelined voice ranges are exclusive");
-    if (!b->ts) CUDA_TRY(cudaStreamCreateWithFlags(&b->ts, cudaStreamNonBlocking));
-    for (int i = 0; i < kTsBufs; i++) {
-        if (!b->d_seg_phase[i]) CUDA_TRY(cudaMalloc(&b->d_seg_phase[i], b->n_voices * 96 * sizeof(float)));
-        if (!b->ev_k1[i]) CUDA_TRY(cudaEventCreateWithFlags(&b->ev_k1[i], cudaEventDisableTiming));
-        if (!b->ev_k2[i]) CUDA_TRY(cudaEventCreateWithFlags(&b->ev_k2[i], cudaEventDisableTiming));
-    }
-    if (!b->ev_main) CUDA_TRY(cudaEventCreateWithFlags(&b->ev_main, cudaEventDisableTiming));
-    b->ts_enabled = true;
-    b->ts_main_dirty = true;
-    b->ts_step = 0;
+    { int rc = b->split.create(b->n_voices); if (rc) return rc; }
+    b->split.enabled = true;
+    b->split.main_dirty = true;
+    b->split.step = 0;
     return S2_OK;
 }
 
 int s2_bank_time_split_blocks(s2_bank* b, uint64_t* blocks) {
     if (!b || !blocks) return fail(S2_ERR_INVALID, "null argument");
-    *blocks = b->ts_blocks;
+    *blocks = b->split.blocks;
     return S2_OK;
 }
 
@@ -943,9 +933,9 @@ int s2_bank_join(s2_bank* b, void* stream) {
     if (b->n_sub <= 1) return S2_OK;       // everything already is on the bank's stream
     CUDA_TRY(cudaSetDevice(b->device));
     cudaStream_t st = (cudaStream_t)stream;
-    for (int k = 0; k < b->n_sub; k++) CUDA_TRY(cudaStreamWaitEvent(st, b->ev_sub[k], 0));
-    CUDA_TRY(cudaEventRecord(b->ev_tail, b->mix));
-    CUDA_TRY(cudaStreamWaitEvent(st, b->ev_tail, 0));
+    for (int k = 0; k < b->n_sub; k++) CUDA_TRY(cudaStreamWaitEvent(st, b->pipe.ev_sub[k], 0));
+    CUDA_TRY(cudaEventRecord(b->pipe.ev_tail, b->pipe.mix));
+    CUDA_TRY(cudaStreamWaitEvent(st, b->pipe.ev_tail, 0));
     return S2_OK;
 }
 
@@ -1158,12 +1148,7 @@ int s2_synth_render_score(s2_synth* s, const s2_note_event* events, size_t n_eve
     }
     if (frames == 0) return S2_OK;
     CUDA_TRY(cudaSetDevice(s->device));
-    if (frames > s->score_cap) {
-        if (s->d_score) CUDA_TRY(cudaFree(s->d_score));
-        s->d_score = nullptr; s->score_cap = 0;
-        CUDA_TRY(cudaMalloc(&s->d_score, frames * sizeof(float)));
-        s->score_cap = frames;
-    }
+    { int rc = grow(s->bank, &s->d_score, 1, s->score_cap, frames); if (rc) return rc; }
     size_t pos = 0, i = 0;
     while (pos < frames) {
         while (i < n_events && score_quantise(events[i].frame) <= pos) {

@@ -82,13 +82,13 @@ cudaError_t launch_ts_render(const RenderArgs& a, uint32_t filter_kind, bool mov
 cudaError_t launch_ts_mix_rows(const float* rows, uint32_t n_rows, size_t row_stride, uint32_t frames, float* bus,
                                cudaStream_t stream);
 // one kernel, fixed summation order; partial row w starts at partials + w * row_stride.  With `counters` (kBusCounters
-// zeroed words owned by the bank, launches on one stream at a time) and 4 * frames floats of scratch, wide banks
-// take the four-frames-per-lane form.
+// zeroed words owned by the bank, launches on one stream at a time) and `scratch` of bus_scratch_floats(n_warps,
+// frames) floats, wide banks take the four-frames-per-lane form.
 constexpr uint32_t kBusCounters = 1024;
-cudaError_t launch_bus_reduce(const float* partials, uint32_t n_warps, size_t row_stride, uint32_t frames,
-                              float* scratch, float* bus, cudaStream_t stream, unsigned int* counters = nullptr,
-                              size_t scratch_floats = 0);
-uint32_t bus_segments(uint32_t n_warps);
+cudaError_t launch_bus_reduce(const float* partials, uint32_t n_warps, size_t row_stride, uint32_t frames, float* bus,
+                              cudaStream_t stream, unsigned int* counters = nullptr, float* scratch = nullptr);
+// floats of scratch the four-frames-per-lane form reads for this shape; 0 where that form does not apply
+size_t bus_scratch_floats(uint32_t n_rows, uint32_t frames);
 // release_row[slot] = staged[voice_of_slot[slot]]  (bulk note-off table given in voice order)
 cudaError_t launch_gather_u32(const uint32_t* staged, const float* row_index_bits, uint32_t* dst_row,
                               uint32_t n, cudaStream_t stream);

@@ -593,8 +593,6 @@ render_kernel(const RenderArgs a) {
 // machine whose every slot is taken by long-running render blocks.  The 4,096 short blocks of the two-stage
 // form it replaces queued for those slots one by one and cost ~30 us of step time for 19 us of work; 128 blocks
 // of 8 warps need one slot each and displace next to nothing (it is latency-bound at ~20 us, off the critical path).
-constexpr uint32_t kBusSegWarps = 64;      // (scratch sizing of the callers: segments of the former first stage)
-
 __global__ void __launch_bounds__(256) bus_reduce_kernel(const float* __restrict__ partials, uint32_t n_rows,
                                                          size_t row_stride, uint32_t frames, float* __restrict__ bus) {
     __shared__ float sm[8][33];
@@ -729,16 +727,17 @@ cudaError_t launch_render(const RenderArgs& a, uint32_t filter_kind, int trace, 
     }
 }
 
-uint32_t bus_segments(uint32_t n_warps) { return (n_warps + kBusSegWarps - 1) / kBusSegWarps; }
+size_t bus_scratch_floats(uint32_t n_rows, uint32_t frames) {
+    const bool wide = n_rows >= 512u && (frames & 127u) == 0u && frames / 128u <= kBusCounters;
+    return wide ? (size_t)kRedSplit * frames : 0;
+}
 
-cudaError_t launch_bus_reduce(const float* partials, uint32_t n_warps, size_t row_stride, uint32_t frames,
-                              float* scratch, float* bus, cudaStream_t stream, unsigned int* counters,
-                              size_t scratch_floats) {
+cudaError_t launch_bus_reduce(const float* partials, uint32_t n_warps, size_t row_stride, uint32_t frames, float* bus,
+                              cudaStream_t stream, unsigned int* counters, float* scratch) {
     if (frames == 0) return cudaSuccess;
     auto al16 = [](const void* q) { return (reinterpret_cast<uintptr_t>(q) & 15u) == 0u; };
-    const bool wide = counters != nullptr && n_warps >= 512u && (frames & 127u) == 0u && frames / 128u <= kBusCounters &&
-                      (row_stride & 3u) == 0u && scratch_floats >= (size_t)kRedSplit * frames &&
-                      al16(partials) && al16(scratch) && al16(bus);
+    const bool wide = counters != nullptr && scratch != nullptr && bus_scratch_floats(n_warps, frames) != 0 &&
+                      (row_stride & 3u) == 0u && al16(partials) && al16(scratch) && al16(bus);
     if (wide)
         bus_reduce_wide_kernel<<<frames / 128u * kRedSplit, 256, 0, stream>>>(partials, n_warps, row_stride, frames, scratch,
                                                                               counters, bus);
