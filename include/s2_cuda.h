@@ -106,6 +106,11 @@ size_t s2_bank_voices(const s2_bank* bank);
 
 /* Replace one voice (note_on into slot `index`, synth.rs:61-70: fresh state, offset from desc). */
 int s2_bank_set_voice(s2_bank* bank, size_t index, const s2_voice_desc* voice);
+/* Bulk note_on (synth.rs:61-70 for many voices): entry j replaces voice indices[j] with voices[j], with the same
+   effect as s2_bank_set_voice(bank, indices[j], &voices[j]) called for j = 0, 1, ..., n-1.  A repeated index: the
+   last entry wins.  Host arrays, copied before the call returns.  Every entry is validated first; on error nothing
+   changes.  Asynchronous in every mode: it never waits for the bank's renders.  n = 0 does nothing. */
+int s2_bank_set_voices(s2_bank* bank, size_t n, const uint32_t* indices, const s2_voice_desc* voices);
 /* note_off for slot `index` (synth.rs:72-80): release_frame_offset = current_frame_offset. */
 int s2_bank_release_voice(s2_bank* bank, size_t index);
 
@@ -152,11 +157,13 @@ int s2_bank_render_bus_host_async(s2_bank* bank, size_t frames, float* d_voice_o
  *   - render calls return at once and are ordered among themselves; their outputs are complete after
  *     s2_bank_sync(), or, on a stream of the caller's, after s2_bank_join(bank, stream);
  *   - the caller must not reuse an output buffer the bank may still be writing (join first);
- *   - s2_bank_set_releases is pipelined too (each range applies the table before its next render);
+ *   - s2_bank_set_releases is pipelined too (each range applies the table before its next render), and
+ *     so is s2_bank_set_voices (each range that receives entries writes them between its renders);
  *     every other entry (set_voice, release_voice, get/set_state, trace) drains the pipeline first;
  *   - edits take effect in call order, as in the default mode: set_voice, release_voice, a trace or a
- *     pipeline change after s2_bank_set_releases applies the table first, so a later edit of a voice's
- *     note-off is never overwritten by an earlier table;
+ *     pipeline change after s2_bank_set_releases applies the table first, and s2_bank_set_voices writes
+ *     its release offsets into a table staged before it, so a later edit of a voice's note-off is never
+ *     overwritten by an earlier table;
  *   - s2_bank_trace_phase returns after its render has finished;
  *   - s2_bank_render_bus_host_async makes the bank's own stream (given at creation) wait for the copy.
  * n_sub = 1 (default) keeps everything on the bank's stream.

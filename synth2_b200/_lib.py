@@ -56,6 +56,7 @@ SYMBOLS = {
     "s2_bank_destroy": (None, [_vp]),
     "s2_bank_voices": (_sz, [_vp]),
     "s2_bank_set_voice": (_i, [_vp, _sz, _vp]),
+    "s2_bank_set_voices": (_i, [_vp, _sz, _vp, _vp]),
     "s2_bank_release_voice": (_i, [_vp, _sz]),
     "s2_bank_set_releases": (_i, [_vp, _vp]),
     "s2_bank_render": (_i, [_vp, _sz, _vp, _sz, _vp]),

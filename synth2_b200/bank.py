@@ -70,6 +70,18 @@ class VoiceBank:
         voice = np.ascontiguousarray(voice, dtype=VOICE_DESC).reshape(-1)[:1]
         check(lib().s2_bank_set_voice(self._h, int(index), ptr(voice)))
 
+    def set_voices(self, indices, voices: np.ndarray):
+        """Bulk note_on: the same as set_voice(indices[j], voices[j]) for j = 0, 1, ... in order (the last entry of a
+        repeated index wins), applied on the GPU without waiting for the bank's renders."""
+        idx = np.asarray(indices).reshape(-1)
+        if idx.size and (idx.min() < 0 or idx.max() > 0xFFFFFFFF):
+            raise IndexError("voice index out of range")
+        idx = np.ascontiguousarray(idx, dtype=np.uint32)
+        voices = np.ascontiguousarray(voices, dtype=VOICE_DESC).reshape(-1)
+        if voices.size != idx.size:
+            raise ValueError(f"{idx.size} indices for {voices.size} voices")
+        check(lib().s2_bank_set_voices(self._h, idx.size, ptr(idx), ptr(voices)))
+
     def release_voice(self, index: int):
         check(lib().s2_bank_release_voice(self._h, int(index)))
 

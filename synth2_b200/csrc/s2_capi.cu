@@ -114,6 +114,15 @@ void pack_state(const s2_voice_state& s, float* col, size_t pitch) {
     col[S_FL_KEY * pitch] = ubits(kNoKey);
 }
 
+// A note-on: the voice's parameter column and a fresh state (st::Layer::default(), synth.rs:68) at its frame offset.
+void pack_note_on(const s2_voice_desc& d, uint32_t index, float* pcol, float* scol, size_t pitch) {
+    pack_voice(d, index, pcol, pitch);
+    s2_voice_state st;
+    memset(&st, 0, sizeof st);
+    st.frame_offset = d.frame_offset;
+    pack_state(st, scol, pitch);
+}
+
 struct VoiceBook {           // host mirror of what the device will hold, O(1) per render
     uint32_t start_offset;   // frame offset when the voice was (re)started
     uint64_t start_total;    // bank->total_frames at that moment
@@ -195,6 +204,39 @@ struct Pipeline {
     }
 };
 
+// Staging of s2_bank_set_voices: batch i is packed into page-locked buffer r = i % kBatchBufs, sent with one copy to
+// device buffer r and scattered from there, so the caller's arrays are free on return and the copy never waits for
+// a pageable-memory bounce.  Buffer r is reused once its copy (host side) and its scatters (device side) have run.
+constexpr int kBatchBufs = 4;
+
+struct VoiceBatches {
+    float* h[kBatchBufs] = {};             // page-locked
+    float* d[kBatchBufs] = {};
+    size_t h_cap = 0, d_cap = 0;           // floats, each buffer
+    cudaEvent_t ev_copied[kBatchBufs] = {};    // the copy out of h[r] has finished
+    cudaEvent_t ev_read[kBatchBufs][8] = {};   // voice range k's scatter out of d[r] has finished (pipelined)
+    uint64_t next = 0;
+    std::vector<uint32_t> stamp;           // per voice: the batch generation that last kept an entry of it
+    uint32_t gen = 0;
+
+    int create() {
+        for (int r = 0; r < kBatchBufs; r++) {
+            CUDA_TRY(make_event(ev_copied[r]));
+            for (int k = 0; k < 8; k++) CUDA_TRY(make_event(ev_read[r][k]));
+        }
+        return S2_OK;
+    }
+
+    void release() {
+        for (int r = 0; r < kBatchBufs; r++) {
+            destroy(ev_copied[r]);
+            for (int k = 0; k < 8; k++) destroy(ev_read[r][k]);
+            if (h[r]) cudaFreeHost(h[r]);
+            cudaFree(d[r]);
+        }
+    }
+};
+
 // Time-split mode (s2_bank_set_time_split, s2_kernel_ts.cu): narrow one-pole banks render a block as 32 time
 // segments per voice.  The phase pre-pass runs on its own stream, ahead of the renders.
 struct TimeSplit {
@@ -252,6 +294,7 @@ struct s2_bank {
     int n_sub = 1;                // voice ranges of the pipelined mode; 1 = everything on the bank's stream
     Pipeline pipe;
     TimeSplit split;
+    VoiceBatches batches;
     uint64_t total_frames = 0;
     uint64_t max_offset = 0;     // upper bound of any active voice's frame offset
     size_t n_sine = 0;
@@ -266,6 +309,15 @@ uint32_t current_offset(const s2_bank* b, size_t i) {
     return o > 0xFFFFFFFFull ? 0xFFFFFFFFu : (uint32_t)o;   // saturating_add, synth.rs:197
 }
 
+// The host mirrors of a voice replaced by s2_bank_set_voice(s), updated at call time in call order.
+void note_voice(s2_bank* b, size_t index, const s2_voice_desc& d) {
+    if (b->book[index].osc_kind == S2_OSC_SINE) b->n_sine--;
+    if (d.osc_kind == S2_OSC_SINE) b->n_sine++;
+    b->book[index] = {d.frame_offset, b->total_frames, d.active ? 1u : 0u, d.osc_kind};
+    if (!b->split.descs.empty()) b->split.descs[index] = d;
+    if (d.active && d.frame_offset > b->max_offset) b->max_offset = d.frame_offset;
+}
+
 // Waits (on the host) for everything the bank has issued on its internal streams.
 int bank_drain(s2_bank* b) {
     for (int k = 0; k < b->n_sub && b->n_sub > 1; k++) CUDA_TRY(cudaStreamSynchronize(b->pipe.sub[k]));
@@ -275,18 +327,19 @@ int bank_drain(s2_bank* b) {
     return S2_OK;
 }
 
-// Grows the n device buffers bufs[0..n) to `need` floats each; they share the capacity `cap`.  The bank's internal
-// streams may still use the old buffers, so the bank (if any) is drained before they are freed.  A failed
-// allocation leaves that buffer null and cap 0.
-int grow(s2_bank* b, float** bufs, int n, size_t& cap, size_t need) {
+// Grows the n device buffers bufs[0..n) (pinned: page-locked host buffers) to `need` floats each; they share the
+// capacity `cap`.  The bank's internal streams may still use the old buffers, so the bank (if any) is drained before
+// they are freed.  A failed allocation leaves that buffer null and cap 0.
+int grow(s2_bank* b, float** bufs, int n, size_t& cap, size_t need, bool pinned = false) {
     if (need <= cap) return S2_OK;
     if (b) { int rc = bank_drain(b); if (rc) return rc; }
     for (int i = 0; i < n; i++) {
-        if (bufs[i]) CUDA_TRY(cudaFree(bufs[i]));
+        if (bufs[i]) CUDA_TRY(pinned ? cudaFreeHost(bufs[i]) : cudaFree(bufs[i]));
         bufs[i] = nullptr;
     }
     cap = 0;
-    for (int i = 0; i < n; i++) CUDA_TRY(cudaMalloc(&bufs[i], need * sizeof(float)));
+    for (int i = 0; i < n; i++)
+        CUDA_TRY(pinned ? cudaMallocHost(&bufs[i], need * sizeof(float)) : cudaMalloc(&bufs[i], need * sizeof(float)));
     cap = need;
     return S2_OK;
 }
@@ -717,6 +770,7 @@ void s2_bank_destroy(s2_bank* b) {
     cudaStreamSynchronize(b->stream);
     b->pipe.release();
     b->split.release();
+    b->batches.release();
     cudaFree(b->d_params);
     cudaFree(b->d_state);
     cudaFree(b->d_partials);
@@ -736,22 +790,104 @@ int s2_bank_set_voice(s2_bank* b, size_t index, const s2_voice_desc* voice) {
     if ((rc = settle_edits(b)) != S2_OK) return rc;    // pipelined mode: per-voice edits are not pipelined
     float hp[s2::P_COUNT], hs[s2::S_COUNT];
     const size_t slot = b->slot_of_voice[index];   // the voice keeps its slot (a changed kind makes that warp mixed)
-    pack_voice(*voice, (uint32_t)index, hp, 1);
-    s2_voice_state st;
-    memset(&st, 0, sizeof st);            // st::Layer::default(), synth.rs:68
-    st.frame_offset = voice->frame_offset;
-    pack_state(st, hs, 1);
+    pack_note_on(*voice, (uint32_t)index, hp, hs, 1);
     // one 4-byte element per SoA row
     CUDA_TRY(cudaMemcpy2DAsync(b->d_params + slot, b->vpad * sizeof(float), hp, sizeof(float), sizeof(float),
                                s2::P_COUNT, cudaMemcpyHostToDevice, b->stream));
     CUDA_TRY(cudaMemcpy2DAsync(b->d_state + slot, b->vpad * sizeof(float), hs, sizeof(float), sizeof(float),
                                s2::S_COUNT, cudaMemcpyHostToDevice, b->stream));
     CUDA_TRY(cudaStreamSynchronize(b->stream));   // hp/hs live on this stack frame
-    if (b->book[index].osc_kind == S2_OSC_SINE) b->n_sine--;
-    if (voice->osc_kind == S2_OSC_SINE) b->n_sine++;
-    b->book[index] = {voice->frame_offset, b->total_frames, voice->active ? 1u : 0u, voice->osc_kind};
-    if (!b->split.descs.empty()) b->split.descs[index] = *voice;
-    if (voice->active && voice->frame_offset > b->max_offset) b->max_offset = voice->frame_offset;
+    note_voice(b, index, *voice);
+    return S2_OK;
+}
+
+int s2_bank_set_voices(s2_bank* b, size_t n, const uint32_t* indices, const s2_voice_desc* voices) {
+    if (!b) return fail(S2_ERR_INVALID, "null bank");
+    if (n == 0) return S2_OK;
+    if (!indices || !voices) return fail(S2_ERR_INVALID, "null argument");
+    for (size_t j = 0; j < n; j++) {
+        if (indices[j] >= b->n_voices) return fail(S2_ERR_INVALID, "entry %zu: voice index %u out of range", j, indices[j]);
+        int rc = validate_voice(voices[j], indices[j], b->filter_kind);
+        if (rc) return rc;
+    }
+    CUDA_TRY(cudaSetDevice(b->device));
+    VoiceBatches& vb = b->batches;
+    Pipeline& pl = b->pipe;
+    { int rc = vb.create(); if (rc) return rc; }
+
+    // The last entry of each index wins: walking backwards, an index is kept the first time it is met.  The kept
+    // entries are then bucketed by voice range (one range unless pipelined), each bucket contiguous in the batch.
+    if (vb.stamp.size() != b->n_voices) vb.stamp.assign(b->n_voices, 0u);
+    if (++vb.gen == 0) { std::fill(vb.stamp.begin(), vb.stamp.end(), 0u); vb.gen = 1; }
+    const int n_ranges = b->n_sub;
+    uint32_t bound[9];
+    for (int k = 0; k <= n_ranges; k++) bound[k] = n_ranges > 1 ? sub_begin(b, k) : (k ? (uint32_t)b->n_voices : 0u);
+    std::vector<uint32_t> kept;
+    std::vector<uint8_t> range_of;
+    size_t count[8] = {}, begin[8] = {};
+    for (size_t j = n; j-- > 0;) {
+        if (vb.stamp[indices[j]] == vb.gen) continue;
+        vb.stamp[indices[j]] = vb.gen;
+        const uint32_t slot = b->slot_of_voice[indices[j]];
+        int k = 0;
+        while (slot >= bound[k + 1]) k++;
+        kept.push_back((uint32_t)j);
+        range_of.push_back((uint8_t)k);
+        count[k]++;
+    }
+    for (int k = 1; k < n_ranges; k++) begin[k] = begin[k - 1] + count[k - 1];
+    const size_t m = kept.size();
+    const size_t need = (size_t)(s2::P_COUNT + s2::S_COUNT + 1) * m;
+
+    const int r = (int)(vb.next % (uint64_t)kBatchBufs);
+    if (need > vb.h_cap) {
+        for (int i = 0; i < kBatchBufs; i++) CUDA_TRY(cudaEventSynchronize(vb.ev_copied[i]));   // no copy reads them
+        int rc = grow(b, vb.h, kBatchBufs, vb.h_cap, need, true);
+        if (rc) return rc;
+    }
+    { int rc = grow(b, vb.d, kBatchBufs, vb.d_cap, need); if (rc) return rc; }
+    CUDA_TRY(cudaEventSynchronize(vb.ev_copied[r]));   // h[r] is free again (long since, in steady state)
+    float* hb = vb.h[r];
+    size_t fill[8];
+    std::copy(begin, begin + 8, fill);
+    for (size_t i = 0; i < m; i++) {
+        const uint32_t j = kept[i];
+        const size_t e = fill[range_of[i]]++;
+        pack_note_on(voices[j], indices[j], hb + e, hb + (size_t)s2::P_COUNT * m + e, m);
+        hb[(size_t)(s2::P_COUNT + s2::S_COUNT) * m + e] = ubits(b->slot_of_voice[indices[j]]);
+    }
+
+    if (n_ranges == 1) {
+        // one stream (time-split included): copy and scatter in order on the bank's stream
+        CUDA_TRY(cudaMemcpyAsync(vb.d[r], hb, need * sizeof(float), cudaMemcpyHostToDevice, b->stream));
+        CUDA_TRY(cudaEventRecord(vb.ev_copied[r], b->stream));
+        CUDA_TRY(s2::launch_set_voices(vb.d[r], (uint32_t)m, 0, (uint32_t)m, b->d_params, b->d_state, (uint32_t)b->vpad,
+                                       nullptr, b->stream));
+        g_launches.fetch_add(1, std::memory_order_relaxed);
+        b->split.main_dirty = true;   // the next phase pre-pass reads the fresh phases
+    } else {
+        // Pipelined: the copy on the upload stream, then each range that has entries scatters them on its own
+        // stream, between its renders.  No range waits for another.  A pending note-off table is applied by the
+        // ranges' next renders: the scatter writes the note-ons' release offsets into it too (after it has landed).
+        for (int k = 0; k < n_ranges; k++) CUDA_TRY(cudaStreamWaitEvent(pl.upload, vb.ev_read[r][k], 0));   // d[r] free
+        CUDA_TRY(cudaMemcpyAsync(vb.d[r], hb, need * sizeof(float), cudaMemcpyHostToDevice, pl.upload));
+        CUDA_TRY(cudaEventRecord(vb.ev_copied[r], pl.upload));
+        const int q = pl.table_pending;
+        for (int k = 0; k < n_ranges; k++) {
+            if (!count[k]) continue;
+            cudaStream_t sk = pl.sub[k];
+            CUDA_TRY(cudaStreamWaitEvent(sk, vb.ev_copied[r], 0));
+            if (q >= 0) CUDA_TRY(cudaStreamWaitEvent(sk, pl.ev_stage[q], 0));
+            CUDA_TRY(s2::launch_set_voices(vb.d[r], (uint32_t)m, (uint32_t)begin[k], (uint32_t)count[k], b->d_params,
+                                           b->d_state, (uint32_t)b->vpad, q >= 0 ? pl.d_staging[q] : nullptr, sk));
+            g_launches.fetch_add(1, std::memory_order_relaxed);
+            CUDA_TRY(cudaEventRecord(vb.ev_read[r][k], sk));
+            if (q >= 0) CUDA_TRY(cudaEventRecord(pl.ev_gather[k][q], sk));   // a superseding table waits for it
+            CUDA_TRY(cudaEventRecord(pl.ev_sub[k], sk));
+        }
+    }
+    vb.next++;
+    for (size_t j = 0; j < n; j++) note_voice(b, indices[j], voices[j]);
     return S2_OK;
 }
 
@@ -783,8 +919,9 @@ int s2_bank_set_releases(s2_bank* b, const uint32_t* h_release) {
             pl.table_step--;
             return s2_bank_set_releases(b, h_release);
         }
-        if (pl.table_step >= 2)     // buffer q still feeds the gathers of the table staged two uploads ago
-            for (int k = 0; k < b->n_sub; k++) CUDA_TRY(cudaStreamWaitEvent(pl.upload, pl.ev_gather[k][q], 0));
+        // buffer q may still feed the renders that apply the table staged two uploads ago, or, when this table
+        // supersedes one, the s2_bank_set_voices scatters that wrote into it
+        for (int k = 0; k < b->n_sub; k++) CUDA_TRY(cudaStreamWaitEvent(pl.upload, pl.ev_gather[k][q], 0));
         CUDA_TRY(cudaMemcpyAsync(pl.d_staging[q], h_release, b->n_voices * sizeof(uint32_t), cudaMemcpyHostToDevice, pl.upload));
         CUDA_TRY(cudaEventRecord(pl.ev_stage[q], pl.upload));
         pl.table_pending = q;
@@ -977,13 +1114,16 @@ uint32_t synth_current(const s2_synth* s, int i) {
     return s->pending[i].frame_offset;
 }
 
+// The note-ons since the last render, as one batch on the bank's stream (no host wait).
 int synth_flush(s2_synth* s) {
-    for (int i = 0; i < kNumVoices; i++) {
-        if (!s->dirty[i]) continue;
-        int rc = s2_bank_set_voice(s->bank, (size_t)i, &s->pending[i]);
-        if (rc) return rc;
-        s->dirty[i] = false;
-    }
+    uint32_t idx[kNumVoices];
+    s2_voice_desc ds[kNumVoices];
+    size_t n = 0;
+    for (int i = 0; i < kNumVoices; i++)
+        if (s->dirty[i]) { idx[n] = (uint32_t)i; ds[n++] = s->pending[i]; }
+    int rc = s2_bank_set_voices(s->bank, n, idx, ds);
+    if (rc) return rc;
+    for (int i = 0; i < kNumVoices; i++) s->dirty[i] = false;
     return S2_OK;
 }
 

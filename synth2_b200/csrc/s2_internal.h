@@ -92,5 +92,10 @@ size_t bus_scratch_floats(uint32_t n_rows, uint32_t frames);
 // release_row[slot] = staged[voice_of_slot[slot]]  (bulk note-off table given in voice order)
 cudaError_t launch_gather_u32(const uint32_t* staged, const float* row_index_bits, uint32_t* dst_row,
                               uint32_t n, cudaStream_t stream);
+// Bulk note-on (s2_bank_set_voices).  `batch` holds m entries column-major: [P_COUNT][m] parameters, [S_COUNT][m] fresh
+// state, then [m] target slots (u32 bits).  Entries [begin, begin + count) are written to their slots of params /
+// state; with `staged_release` (a pending note-off table in voice order) also staged_release[P_ROW] = P_RELEASE.
+cudaError_t launch_set_voices(const float* batch, uint32_t m, uint32_t begin, uint32_t count, float* params,
+                              float* state, uint32_t vpad, uint32_t* staged_release, cudaStream_t stream);
 
 }  // namespace s2

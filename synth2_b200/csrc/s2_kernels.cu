@@ -695,6 +695,31 @@ cudaError_t launch_gather_u32(const uint32_t* staged, const float* row_index_bit
     return cudaGetLastError();
 }
 
+// Bulk note-on: thread j takes entry e = begin + j of the packed batch (one column per entry, read coalesced across
+// the entries) and writes its P_COUNT + S_COUNT words at its slot.  A pending note-off table gets the entry's release
+// offset at the entry's voice index, so that the render prologue that applies the table keeps the note-on's value.
+__global__ void set_voices_kernel(const float* __restrict__ batch, uint32_t m, uint32_t begin, uint32_t count,
+                                  float* __restrict__ params, float* __restrict__ state, uint32_t vpad,
+                                  uint32_t* __restrict__ staged_release) {
+    const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= count) return;
+    const size_t e = begin + j;
+    const size_t slot = __float_as_uint(batch[(size_t)(P_COUNT + S_COUNT) * m + e]);
+#pragma unroll
+    for (int k = 0; k < P_COUNT; k++) params[(size_t)k * vpad + slot] = batch[(size_t)k * m + e];
+#pragma unroll
+    for (int k = 0; k < S_COUNT; k++) state[(size_t)k * vpad + slot] = batch[(size_t)(P_COUNT + k) * m + e];
+    if (staged_release != nullptr)
+        staged_release[__float_as_uint(batch[(size_t)P_ROW * m + e])] = __float_as_uint(batch[(size_t)P_RELEASE * m + e]);
+}
+
+cudaError_t launch_set_voices(const float* batch, uint32_t m, uint32_t begin, uint32_t count, float* params,
+                              float* state, uint32_t vpad, uint32_t* staged_release, cudaStream_t stream) {
+    if (count == 0) return cudaSuccess;
+    set_voices_kernel<<<(count + 255) / 256, 256, 0, stream>>>(batch, m, begin, count, params, state, vpad, staged_release);
+    return cudaGetLastError();
+}
+
 uint32_t render_warps(uint32_t n_voices) { return (n_voices + 31u) / 32u; }
 
 static_assert((size_t)kWarpsPerBlock * warp_smem_floats() * sizeof(float) + 4096 <= 48 * 1024,
