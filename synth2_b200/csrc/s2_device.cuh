@@ -11,6 +11,8 @@
 #include "s2_math.h"
 #include "s2_cutoff.h"
 
+#include <type_traits>
+
 // The biquad's products and sums are rounded separately, as the source reads (dsp_filters.rs:116-128).  A
 // fused (FFMA) form was tried and rejected: a resonant low-cutoff biquad in f32 direct form amplifies
 // per-frame rounding differences by ~1/(1-r) (~10^3 at 100 Hz, damping 0.2), enough to pass the 1e-4 bar.
@@ -28,6 +30,17 @@ namespace s2 {
 static __device__ const uint32_t d_sin_bits[1024] = {
 #include "sin_table_bits.inc"
 };
+
+// Oscillator-kind dispatch: fn(std::integral_constant<int, K>, args...) for the first K of the list equal to k, the
+// last K of the list for any other k.  The list is the set of loop variants a call site instantiates.  The loop's
+// arguments are passed through rather than captured: a lambda that captures the render kernel's locals by reference
+// changes its register allocation (e.g. 8 B of spills appear or vanish, instruction counts move by up to 5 %).
+template <int K, int... Ks, class Fn, class... A>
+__device__ __forceinline__ void with_kind(int k, Fn&& fn, A&&... args) {
+    if constexpr (sizeof...(Ks) == 0) fn(std::integral_constant<int, K>{}, args...);
+    else if (k == K) fn(std::integral_constant<int, K>{}, args...);
+    else with_kind<Ks...>(k, fn, args...);
+}
 
 // ------------------------------------------------------------------------------------------
 // Per-lane voice description, decoded once per launch.
@@ -124,6 +137,15 @@ __device__ __forceinline__ SegEnv seg_env(const E& e, uint32_t n) {
 }
 __device__ __forceinline__ float seg_eval(const SegEnv& s, float x) {
     return __fadd_rn(__fmul_rn(s.es, __fadd_rn(x, s.nex0)), s.ey0);
+}
+// The envelope at frame offset n (x = its f32 image) of a walk that keeps its current segment in `s`: the line inside
+// the segment, the stage chain at a boundary, after which `s` is the next frame's segment.
+template <class E>
+__device__ __forceinline__ float seg_walk(SegEnv& s, const E& e, uint32_t n, float x) {
+    if (n < s.nend) return seg_eval(s, x);
+    const float g = env_x16(e, x);
+    s = seg_env(e, n + 1u);
+    return g;
 }
 
 // fmod(t, 1) for t in [0, 2) (the fast paths: 0 <= phase < 1, 0 <= 1/P < 1): t - 1 is exact there, and as
@@ -441,9 +463,9 @@ __device__ __forceinline__ float osc_step(uint32_t kind, const OscC& o, float& p
 // equal to the IEEE quotient for all 65,536 possible values (tests/test_oracle_kats.py).
 // (q * 2) - 1 is one fma because q * 2 is exact.
 constexpr float kNoiseHi = 0x1.0001p-16f, kNoiseEps = 0x1p-45f;
+__device__ __forceinline__ uint32_t noise_hash(uint32_t rot, uint32_t n) { return (rot ^ n) * 0x9e3779b9u; }
 __device__ __forceinline__ float noise_fast(uint32_t rot, uint32_t n) {
-    const uint32_t h = (rot ^ n) * 0x9e3779b9u;
-    const float v = __uint2float_rn(h & 0xffffu);
+    const float v = __uint2float_rn(noise_hash(rot, n) & 0xffffu);
     const float q = __fmaf_rn(v, kNoiseHi, kNoiseEps);
     return __fmaf_rn(q, 2.0f, -1.0f);
 }
@@ -538,14 +560,30 @@ struct FastV {
     float P, d, slope, nhalf, ts1, ts2;
     // patch
     float gain, namt;
-    // filter of a resting cutoff: one-pole c0 = k, c1 = 1 - k; second order c0 = 2*alpha, c1 = 2*beta, c2 = 2*gamma
-    float c0, c1, c2;
+    // filter of a resting cutoff (fl_bits unused)
+    FiltC fc;
     // amp envelope segment of the lane's current frame: g = es * (x + nex0) + ey0 for frame offsets [.., seg_end)
     float es, nex0, ey0;
     uint32_t seg_end;
     // carried state
-    float ph, x1, x2, y1, y2;
+    float ph;
+    FiltS fs;
 };
+
+__device__ __forceinline__ void set_osc(FastV& F, const OscC& o) {
+    F.P = o.P; F.d = o.d; F.slope = o.slope; F.nhalf = -o.half; F.ts1 = o.ts1; F.ts2 = o.ts2;
+}
+__device__ __forceinline__ OscC osc_of(const FastV& F) {
+    OscC o;
+    o.P = F.P; o.d = F.d; o.slope = F.slope; o.half = -F.nhalf; o.ts1 = F.ts1; o.ts2 = F.ts2; o.fo_bits = 0;
+    return o;
+}
+
+// es * (x + nex0) + ey0 for frames (x.x, x.y): an envelope segment's line (SegEnv), the add through an fma by one
+// (see the hazard note)
+__device__ __forceinline__ float2 seg_line2(float es, float nex0, float ey0, float2 x, float one) {
+    return s2c::vaddp(pmul2(splat2(es), padd2(x, splat2(nex0))), splat2(ey0), one);
+}
 
 // How a chunk evaluates the amp envelope.
 enum { G_CONST = 0,      // every frame of the chunk lies in a segment of slope 0 (sustain, end): g = ey0
@@ -620,11 +658,42 @@ __device__ __forceinline__ float2 input2(const FastV& F, float2 osc2, uint32_t h
     return padd2(padd2(osc2, splat2(F.gain)), NAMT0 ? nz2 : padd2(nz2, splat2(F.namt)));
 }
 
+// The filter input of one frame, u = (osc + gain) + (noise + amount), as input2
+__device__ __forceinline__ float input1(const FastV& F, float osc, uint32_t rot, uint32_t n) {
+    return __fadd_rn(__fadd_rn(osc, F.gain), __fadd_rn(noise_fast(rot, n), F.namt));
+}
+
+// One frame of one voice, x16 semantics in the fast forms (osc_step without the `%`, noise_fast), filter coefficients
+// c: the phase step, waveform, filter input and filter step.  Returns the filter's output.
+template <int FILTER, int KIND>
+__device__ __forceinline__ float voice_frame(FastV& F, const FiltC& c, uint32_t kind, uint32_t rot, uint32_t n,
+                                             const float* sintab) {
+    const float osc = osc_step<KIND, false>(kind, osc_of(F), F.ph, sintab);
+    return filt_step<FILTER>(input1(F, osc, rot, n), c, F.fs);
+}
+
+// Frames (i, i + 1) of one voice in the time-packed loops, filter coefficients ca / cb and noise hash words ha / hb of
+// the two frames.  The two recurrences (phase, filter) stay scalar — a packed op has twice the latency — while
+// everything that is feed-forward (waveform, noise map, gain / noise combine, the filter's input product, output gain)
+// is computed for both frames in one packed instruction.  Element-wise rounding is identical to the scalar form.
+// gain() gives the amp envelope of the two frames, evaluated after the filter step.  hbig = (P / 2) * 2^60 (wave2).
+template <int FILTER, int KIND, bool NAMT0, int TRACE, class Gain>
+__device__ __forceinline__ float2 voice_pair(FastV& F, const FiltC& ca, const FiltC& cb, uint32_t ha, uint32_t hb,
+                                             float hbig, uint32_t kind, const float* sintab, Gain&& gain) {
+    // phase recurrence, two frames (try3/oscillators.rs:377-381; see osc_step)
+    const float pa = F.ph;
+    const float pb = wrap_unit(__fadd_rn(pa, F.d));
+    F.ph = wrap_unit(__fadd_rn(pb, F.d));
+    const float2 ph2 = make_float2(pa, pb);
+    const float2 osc2 = wave2<KIND>(F, ph2, hbig, kind, sintab);
+    const float2 y2 = filt_step2<FILTER>(input2<NAMT0>(F, osc2, ha, hb), ca, cb, F.fs);
+    // envelope (old/simdtest.rs:270-330) and output gain (process.rs:373-378)
+    const float2 g2 = gain();
+    return TRACE == TRACE_PHASE ? ph2 : pmul2(y2, g2);
+}
+
 // Time-packed fast chunk: 32 frames of one voice per lane with period, cutoff and (G_CONST / G_LINE) amp-envelope
-// segment constant.  The two recurrences (phase, filter) stay scalar — a packed op has twice the latency — while
-// everything that is feed-forward (waveform, noise map, gain / noise combine, envelope, output gain, the filter's
-// input product) is computed for frames (i, i + 1) of the voice in one packed instruction.  Element-wise rounding
-// is identical to the scalar form.
+// segment constant, two frames per step (voice_pair).
 // FASTHASH: the noise amount is +0.0 and the voice's frame offset and rotated seed are multiples of 8 (seeds below
 // 2^27 rotate to multiples of 32), so (seed' ^ (offset + i)) == (seed' ^ offset) + i and the hash of frame i is one
 // add with an immediate.
@@ -636,56 +705,37 @@ __device__ __forceinline__ void chunk_fast_tp(FastV& F, const EnvQ* __restrict__
     float2 xf2 = make_float2(__uint2float_rn(n0), __uint2float_rn(n0 + 1u));       // exact: n0 + 32 <= 2^24
     SegEnv sg = {0.0f, 0.0f, 0.0f, 0u, 0u, 0};
     if (GMODE == G_ANY) sg = seg_env(*amp, n0);
-    FiltS fs = {F.x1, F.x2, F.y1, F.y2};
-    FiltC fc;
-    fc.c0 = F.c0; fc.c1 = F.c1; fc.c2 = F.c2; fc.fl_bits = 0;
-    float ph = F.ph;
     // 8 frames per trip: long enough to overlap neighbouring frames, short enough for the instruction cache
 #pragma unroll 1
     for (int jt = 0; jt < kChunk / S2_TRIP; jt++) {
     // FASTHASH: nb ^ i == nb + i for i < 8, so the hash of frame i is nb * C + i * C: one multiply per trip and
     // one add with an immediate per frame
-    const uint32_t nbc = (rot ^ n) * 0x9e3779b9u;
+    const uint32_t nbc = noise_hash(rot, n);
 #pragma unroll
     for (int jj = 0; jj < S2_TRIP / 4; jj++) {
         const int j = (S2_TRIP / 4) * jt + jj;
         float o4[4];
 #pragma unroll
         for (int h = 0; h < 2; h++) {
-            // ---- phase recurrence, two frames (try3/oscillators.rs:377-381; see osc_step)
-            const float pa = ph;
-            const float pb = wrap_unit(__fadd_rn(pa, F.d));
-            ph = wrap_unit(__fadd_rn(pb, F.d));
-            const float2 ph2 = make_float2(pa, pb);
-            const float2 osc2 = wave2<KIND>(F, ph2, hbig, kind, sintab);
-            // ---- noise (try3/hashnoise.rs:33-68)
             const uint32_t fi = 4u * jj + 2u * h;                 // frame index inside the trip (compile-time)
-            const uint32_t ha = FASTHASH ? nbc + fi * 0x9e3779b9u : (rot ^ (n + fi)) * 0x9e3779b9u;
-            const uint32_t hb = FASTHASH ? nbc + (fi + 1u) * 0x9e3779b9u : (rot ^ (n + fi + 1u)) * 0x9e3779b9u;
-            const float2 u2 = input2<FASTHASH>(F, osc2, ha, hb);
-            // ---- filter recurrence
-            const float2 y2 = filt_step2<FILTER>(u2, fc, fc, fs);
-            // ---- envelope segment (old/simdtest.rs:270-330) and output gain (process.rs:373-378)
-            float2 g2;
-            if (GMODE == G_CONST) g2 = splat2(F.ey0);
-            else if (GMODE == G_LINE) {
-                // es * (x + nex0) + ey0, the add through an fma by one (see the hazard note)
-                g2 = s2c::vaddp(pmul2(splat2(F.es), padd2(xf2, splat2(F.nex0))), splat2(F.ey0), one);
-                xf2 = padd2(xf2, splat2(2.0f));
-            } else {
-                const uint32_t ne = n + fi;
-                if (ne + 2u <= sg.nend) {
+            const uint32_t ha = FASTHASH ? nbc + fi * 0x9e3779b9u : noise_hash(rot, n + fi);
+            const uint32_t hb = FASTHASH ? nbc + (fi + 1u) * 0x9e3779b9u : noise_hash(rot, n + fi + 1u);
+            const float2 out2 = voice_pair<FILTER, KIND, FASTHASH, TRACE>(F, F.fc, F.fc, ha, hb, hbig, kind, sintab, [&] {
+                if (GMODE == G_CONST) return splat2(F.ey0);
+                float2 g2;
+                if (GMODE == G_LINE) {
+                    g2 = seg_line2(F.es, F.nex0, F.ey0, xf2, one);
+                } else if (n + fi + 2u <= sg.nend) {
                     // both frames inside the current segment: its line, bit-exact (see SegEnv)
-                    g2.x = seg_eval(sg, xf2.x);
-                    g2.y = seg_eval(sg, xf2.y);
+                    g2 = make_float2(seg_eval(sg, xf2.x), seg_eval(sg, xf2.y));
                 } else {
-                    const AmpEdge e = amp_at_boundary(amp, xf2.x, xf2.y, ne + 2u);
+                    const AmpEdge e = amp_at_boundary(amp, xf2.x, xf2.y, n + fi + 2u);
                     g2 = e.g;
                     sg = e.sg;
                 }
                 xf2 = padd2(xf2, splat2(2.0f));
-            }
-            const float2 out2 = TRACE == TRACE_PHASE ? ph2 : pmul2(y2, g2);
+                return g2;
+            });
             o4[2 * h] = out2.x;
             o4[2 * h + 1] = out2.y;
         }
@@ -693,15 +743,13 @@ __device__ __forceinline__ void chunk_fast_tp(FastV& F, const EnvQ* __restrict__
     }
     n += (uint32_t)S2_TRIP;
     }
-    F.ph = ph;
-    F.x1 = fs.x1; F.x2 = fs.x2; F.y1 = fs.y1; F.y2 = fs.y2;
 }
 
 // Per-lane inputs of a moving-cutoff chunk (registers, valid for one chunk).
 struct MovV {
     CutP cp;
     float mes, mnex0, mey0;      // the mod envelope's segment line (the whole chunk lies inside it)
-    bool moving;                 // false: this lane's cutoff rests (F.c0 .. F.c2) while others of the warp move
+    bool moving;                 // false: this lane's cutoff rests (F.fc) while others of the warp move
 };
 
 // Moving-cutoff chunk, packed: the period is constant but the mod envelope is in a ramp, so the cutoff — and with
@@ -727,45 +775,32 @@ __device__ __forceinline__ void chunk_modcut_pk(FastV& F, const MovV& mv, const 
     const float hbig = __fmul_rn(-F.nhalf, 0x1p60f);
     uint32_t n = n0;
     float2 xf2 = make_float2(__uint2float_rn(n0), __uint2float_rn(n0 + 1u));
-    FiltS fs = {F.x1, F.x2, F.y1, F.y2};
-    float ph = F.ph;
 #pragma unroll 1
     for (int j = 0; j < kChunk / 4; j++) {
         float o4[4];
 #pragma unroll
         for (int h = 0; h < 2; h++) {
             // the mod envelope's line at the two frame offsets
-            const float2 m2 = s2c::vaddp(pmul2(splat2(mv.mes), padd2(xf2, splat2(mv.mnex0))), splat2(mv.mey0), one);
+            const float2 m2 = seg_line2(mv.mes, mv.mnex0, mv.mey0, xf2, one);
             float2 c0, c1, c2;
             if (SHARED) {
                 c0 = *reinterpret_cast<const float2*>(ctab + 4 * j + 2 * h);
                 c1 = *reinterpret_cast<const float2*>(ctab + 32 + 4 * j + 2 * h);
                 c2 = *reinterpret_cast<const float2*>(ctab + 64 + 4 * j + 2 * h);
-                if (!mv.moving) { c0 = splat2(F.c0); c1 = splat2(F.c1); c2 = splat2(F.c2); }
             } else if (FILTER == FILT_ONE_POLE) {
                 c0 = s2c::exp_neg_fast<float2>(s2c::theta_at<float2>(m2, mv.cp.amt, mv.cp.theta0));
                 c1 = pfma2(c0, splat2(-one), splat2(1.0f));               // 1 - k, one rounding (exact product)
                 c2 = splat2(0.0f);
-                if (!mv.moving) { c0 = splat2(F.c0); c1 = splat2(F.c1); }
             } else {
                 float2 s2, co2;
                 window_frame_sincos<float2>(W, mv.cp, one, m2, &s2, &co2);
                 s2c::biquad_lp_hp<FILTER == FILT_BIQUAD_HP, float2>(s2, co2, mv.cp.hd, one, &c0, &c1, &c2);
-                if (!mv.moving) { c0 = splat2(F.c0); c1 = splat2(F.c1); c2 = splat2(F.c2); }
             }
-            FiltC ca, cb;
-            ca.c0 = c0.x; ca.c1 = c1.x; ca.c2 = c2.x;
-            cb.c0 = c0.y; cb.c1 = c1.y; cb.c2 = c2.y;
-            const float pa = ph;
-            const float pb = wrap_unit(__fadd_rn(pa, F.d));
-            ph = wrap_unit(__fadd_rn(pb, F.d));
-            const float2 ph2 = make_float2(pa, pb);
-            const float2 osc2 = wave2<KIND>(F, ph2, hbig, kind, sintab);
-            const uint32_t ha = (rot ^ n) * 0x9e3779b9u, hb = (rot ^ (n + 1u)) * 0x9e3779b9u;
-            const float2 u2 = input2<false>(F, osc2, ha, hb);
-            const float2 y2 = filt_step2<FILTER>(u2, ca, cb, fs);
-            const float2 g2 = s2c::vaddp(pmul2(splat2(F.es), padd2(xf2, splat2(F.nex0))), splat2(F.ey0), one);
-            const float2 out2 = TRACE == TRACE_PHASE ? ph2 : pmul2(y2, g2);
+            if (!mv.moving) { c0 = splat2(F.fc.c0); c1 = splat2(F.fc.c1); c2 = splat2(F.fc.c2); }
+            const FiltC ca = {c0.x, c1.x, c2.x, 0u}, cb = {c0.y, c1.y, c2.y, 0u};
+            const float2 out2 = voice_pair<FILTER, KIND, false, TRACE>(F, ca, cb, noise_hash(rot, n), noise_hash(rot, n + 1u),
+                                                                       hbig, kind, sintab,
+                                                                       [&] { return seg_line2(F.es, F.nex0, F.ey0, xf2, one); });
             o4[2 * h] = out2.x;
             o4[2 * h + 1] = out2.y;
             n += 2u;
@@ -773,8 +808,6 @@ __device__ __forceinline__ void chunk_modcut_pk(FastV& F, const MovV& mv, const 
         }
         *reinterpret_cast<float4*>(row + 4 * j) = make_float4(o4[0], o4[1], o4[2], o4[3]);
     }
-    F.ph = ph;
-    F.x1 = fs.x1; F.x2 = fs.x2; F.y1 = fs.y1; F.y2 = fs.y2;
 }
 
 // The same chunk when no aligned lane pair (2i, 2i + 1) holds two moving lanes (s2_bank_create lays the slots out that
@@ -805,11 +838,9 @@ __device__ __forceinline__ void chunk_modcut_pr(FastV& F, const MovV& mv, const 
     const float hbig = __fmul_rn(-F.nhalf, 0x1p60f);
     uint32_t n = n0;
     float2 xf2 = make_float2(__uint2float_rn(n0), __uint2float_rn(n0 + 1u));
-    FiltS fs = {F.x1, F.x2, F.y1, F.y2};
-    float ph = F.ph;
 #pragma unroll 1
     for (int j = 0; j < kChunk / 4; j++) {
-        const float2 m2 = s2c::vaddp(pmul2(splat2(mes), padd2(xa2, splat2(mnex0))), splat2(mey0), one);
+        const float2 m2 = seg_line2(mes, mnex0, mey0, xa2, one);
         float2 s2, co2;
         window_frame_sincos<float2>(Wa, cp, one, m2, &s2, &co2);
         const float2 q2 = s2c::quotient_of<float2>(s2, cp.hd, one);
@@ -822,20 +853,11 @@ __device__ __forceinline__ void chunk_modcut_pr(FastV& F, const MovV& mv, const 
         for (int h = 0; h < 2; h++) {
             float2 c0, c1, c2;
             s2c::biquad_from_q_cos<FILTER == FILT_BIQUAD_HP, float2>(h ? qo : q2, h ? coo : co2, one, &c0, &c1, &c2);
-            if (!mv.moving) { c0 = splat2(F.c0); c1 = splat2(F.c1); c2 = splat2(F.c2); }
-            FiltC ca, cb;
-            ca.c0 = c0.x; ca.c1 = c1.x; ca.c2 = c2.x;
-            cb.c0 = c0.y; cb.c1 = c1.y; cb.c2 = c2.y;
-            const float pa = ph;
-            const float pb = wrap_unit(__fadd_rn(pa, F.d));
-            ph = wrap_unit(__fadd_rn(pb, F.d));
-            const float2 ph2 = make_float2(pa, pb);
-            const float2 osc2 = wave2<KIND>(F, ph2, hbig, kind, sintab);
-            const uint32_t ha = (rot ^ n) * 0x9e3779b9u, hb = (rot ^ (n + 1u)) * 0x9e3779b9u;
-            const float2 u2 = input2<false>(F, osc2, ha, hb);
-            const float2 y2 = filt_step2<FILTER>(u2, ca, cb, fs);
-            const float2 g2 = s2c::vaddp(pmul2(splat2(F.es), padd2(xf2, splat2(F.nex0))), splat2(F.ey0), one);
-            const float2 out2 = TRACE == TRACE_PHASE ? ph2 : pmul2(y2, g2);
+            if (!mv.moving) { c0 = splat2(F.fc.c0); c1 = splat2(F.fc.c1); c2 = splat2(F.fc.c2); }
+            const FiltC ca = {c0.x, c1.x, c2.x, 0u}, cb = {c0.y, c1.y, c2.y, 0u};
+            const float2 out2 = voice_pair<FILTER, KIND, false, TRACE>(F, ca, cb, noise_hash(rot, n), noise_hash(rot, n + 1u),
+                                                                       hbig, kind, sintab,
+                                                                       [&] { return seg_line2(F.es, F.nex0, F.ey0, xf2, one); });
             o4[2 * h] = out2.x;
             o4[2 * h + 1] = out2.y;
             n += 2u;
@@ -843,8 +865,6 @@ __device__ __forceinline__ void chunk_modcut_pr(FastV& F, const MovV& mv, const 
         }
         *reinterpret_cast<float4*>(row + 4 * j) = make_float4(o4[0], o4[1], o4[2], o4[3]);
     }
-    F.ph = ph;
-    F.x1 = fs.x1; F.x2 = fs.x2; F.y1 = fs.y1; F.y2 = fs.y2;
 }
 
 // Moving-cutoff chunk, one frame at a time: any alignment, any filter, windows made on demand (valid or not).
@@ -858,33 +878,22 @@ __device__ __forceinline__ void chunk_modcut_sc(FastV& F, const EnvQ* __restrict
                                                 float one, uint32_t kind, uint32_t rot, uint32_t n0,
                                                 float* __restrict__ row, const float* sintab, const float* __restrict__ ctab) {
     SegEnv sa = seg_env(*amp, n0);
-    OscC o;
-    o.P = F.P; o.d = F.d; o.slope = F.slope; o.half = -F.nhalf; o.ts1 = F.ts1; o.ts2 = F.ts2; o.fo_bits = 0;
-    FiltS fs = {F.x1, F.x2, F.y1, F.y2};
-    FiltC fc;
-    fc.c0 = F.c0; fc.c1 = F.c1; fc.c2 = F.c2; fc.fl_bits = 0;
+    FiltC fc = F.fc;
     s2c::Window W;
     window_none(W);
-    float ph = F.ph;
     uint32_t n = n0;
     float xf = __uint2float_rn(n0);                               // exact: n0 + 32 <= 2^24
 #pragma unroll 1
     for (int i = 0; i < kChunk; i++) {
-        float g;
-        if (n < sa.nend) g = seg_eval(sa, xf); else { g = env_x16(*amp, xf); sa = seg_env(*amp, n + 1u); }
+        const float g = seg_walk(sa, *amp, n, xf);
         if (SHARED) { fc.c0 = ctab[i]; fc.c1 = ctab[32 + i]; fc.c2 = ctab[64 + i]; }
         else if (mv.moving) moving_coefs<FILTER>(fc, W, sm, mv.cp, one, n, seg_eval(sm, xf));
-        const float ph0 = ph;
-        const float osc = osc_step<KIND, false>(kind, o, ph, sintab);
-        const float nz = noise_fast(rot, n);
-        const float u = __fadd_rn(__fadd_rn(osc, F.gain), __fadd_rn(nz, F.namt));
-        const float y = filt_step<FILTER>(u, fc, fs);
+        const float ph0 = F.ph;
+        const float y = voice_frame<FILTER, KIND>(F, fc, kind, rot, n, sintab);
         row[i] = TRACE == TRACE_PHASE ? ph0 : __fmul_rn(y, g);
         n += 1u;
         xf = __fadd_rn(xf, 1.0f);
     }
-    F.ph = ph;
-    F.x1 = fs.x1; F.x2 = fs.x2; F.y1 = fs.y1; F.y2 = fs.y2;
 }
 
 // One frame per lane: the filter coefficients of frames n0 .. n0 + 31 of a cutoff trajectory shared by the warp.

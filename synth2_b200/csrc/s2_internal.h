@@ -57,7 +57,6 @@ struct RenderArgs {
                            // without the lane-pair help (chunk_modcut_pk only)
 };
 
-constexpr int kWarpsPerBlock = 1;
 constexpr int kChunk = 32;          // frames per compute chunk (classification granularity)
 // The render kernel's tile is 32 voices x 64 frames = two chunks: a warp then writes 256 contiguous bytes per output
 // row per visit.  128 bytes per row per visit tops out at 5.1 TB/s of write bandwidth on this part whatever the

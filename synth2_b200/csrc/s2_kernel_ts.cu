@@ -75,12 +75,22 @@ template <int FILTER, bool GCONST>
 __device__ __forceinline__ void ts_chunk_kind(FastV& F, const EnvQ* amp, float one, uint32_t kind, uint32_t rot, uint32_t n,
                                               float* row, const float* sintab) {
     constexpr int G = GCONST ? G_CONST : G_ANY;
-    switch (kind) {                       // warp-uniform: a warp is one voice
-    case 0: chunk_fast_tp<FILTER, 0, G, false, TRACE_NONE>(F, amp, one, kind, rot, n, row, sintab); break;
-    case 1: chunk_fast_tp<FILTER, 1, G, false, TRACE_NONE>(F, amp, one, kind, rot, n, row, sintab); break;
-    case 2: chunk_fast_tp<FILTER, 2, G, false, TRACE_NONE>(F, amp, one, kind, rot, n, row, sintab); break;
-    default: chunk_fast_tp<FILTER, 3, G, false, TRACE_NONE>(F, amp, one, kind, rot, n, row, sintab); break;
+    // warp-uniform: a warp is one voice
+    with_kind<0, 1, 2, 3>((int)kind, [](auto K, auto&&... args) { chunk_fast_tp<FILTER, K, G, false, TRACE_NONE>(args...); },
+                          F, amp, one, kind, rot, n, row, sintab);
+}
+
+// Write-back of the 32 x 32 tile of frames c .. c + 31 of every segment: tile row r = segment r (128-byte runs)
+__device__ __forceinline__ void ts_store_tile(const float* tile, int lane, float* __restrict__ gout, uint32_t L, uint32_t c) {
+    const int q = lane >> 3, c4 = (lane & 7) * 4;
+    __syncwarp();
+#pragma unroll
+    for (int i = 0; i < 8; i++) {
+        const int r = 4 * i + q;
+        const float4 val = *reinterpret_cast<const float4*>(tile + r * kTsTileStride + c4);
+        __stcs(reinterpret_cast<float4*>(gout + (size_t)r * L + c + c4), val);
     }
+    __syncwarp();
 }
 
 // 2x2 real matrices (row-major) in binary64 for the biquad's segment maps
@@ -99,30 +109,25 @@ __device__ __forceinline__ M22 shfl_up(const M22& m, int off) {
 // accumulates the product of the per-frame state maps — k_n for the one-pole, M_n = [[2g_n, -2b_n], [1, 0]] for
 // the biquad — which is the segment's map for the scan.  WRITE: second sweep, output through the tile.
 template <int FILTER, bool WRITE>
-__device__ __forceinline__ void ts_moving_sweep(const EnvP& A, const EnvP& M, float lpf, float amt_lpf, float damp,
-                                                float sr, float one, const OscC& oc, uint32_t kind, uint32_t rot, float gain,
-                                                float namt, uint32_t nl, uint32_t L, float& ph, FiltS& fs, float& kprod,
-                                                M22& mprod, float* tile, int lane, float* __restrict__ gout,
+__device__ __forceinline__ void ts_moving_sweep(FastV& F, const Lane& V, float sr, float one, uint32_t nl, uint32_t L,
+                                                float& kprod, M22& mprod, float* tile, int lane, float* __restrict__ gout,
                                                 const float* sintab) {
-    const int q = lane >> 3, c4 = (lane & 7) * 4;
     float* row = tile + lane * kTsTileStride;
-    SegEnv sa = seg_env(A, nl);
+    SegEnv sa = seg_env(V.amp, nl);
     uint32_t n = nl;
     float xf = __uint2float_rn(nl);
     FiltC fc;
     fc.c0 = fc.c1 = fc.c2 = 0.0f; fc.fl_bits = kNoKey;
     MovG mg;
-    movg_init(mg, lpf, amt_lpf, damp, sr);
-    mg.sm = seg_env(M, nl);
+    movg_init(mg, V.lpf, V.amt_lpf, V.damp, sr);
+    mg.sm = seg_env(V.mod, nl);
     for (uint32_t c = 0; c < L; c += kChunk) {
 #pragma unroll 1
         for (int i = 0; i < kChunk; i++) {
-            if (n >= mg.sm.nend) mg.sm = seg_env(M, n);
+            if (n >= mg.sm.nend) mg.sm = seg_env(V.mod, n);
             const float m = seg_eval(mg.sm, xf);
-            x16_coefs<FILTER>(fc, mg, M, lpf, amt_lpf, damp, sr, one, n, m);
-            const float osc = osc_step<-1, false>(kind, oc, ph, sintab);
-            const float u = __fadd_rn(__fadd_rn(osc, gain), __fadd_rn(noise_fast(rot, n), namt));
-            const float y = filt_step<FILTER>(u, fc, fs);
+            x16_coefs<FILTER>(fc, mg, V.mod, V.lpf, V.amt_lpf, V.damp, sr, one, n, m);
+            const float y = voice_frame<FILTER, -1>(F, fc, V.kind, V.rot, n, sintab);
             if (!WRITE) {
                 if (FILTER == 0) kprod = __fmul_rn(kprod, fc.c0);
                 else {                                        // M_n * mprod
@@ -131,23 +136,12 @@ __device__ __forceinline__ void ts_moving_sweep(const EnvP& A, const EnvP& M, fl
                     mprod = t;
                 }
             } else {
-                float g;
-                if (n < sa.nend) g = seg_eval(sa, xf); else { g = env_x16(A, xf); sa = seg_env(A, n + 1u); }
-                row[i] = __fmul_rn(y, g);
+                row[i] = __fmul_rn(y, seg_walk(sa, V.amp, n, xf));
             }
             n += 1u;
             xf = __fadd_rn(xf, 1.0f);
         }
-        if (WRITE) {
-            __syncwarp();
-#pragma unroll
-            for (int i = 0; i < 8; i++) {
-                const int r = 4 * i + q;                      // tile row = segment r
-                const float4 val = *reinterpret_cast<const float4*>(tile + r * kTsTileStride + c4);
-                __stcs(reinterpret_cast<float4*>(gout + (size_t)r * L + c + c4), val);
-            }
-            __syncwarp();
-        }
+        if (WRITE) ts_store_tile(tile, lane, gout, L, c);
     }
 }
 
@@ -166,7 +160,6 @@ __global__ void __launch_bounds__(32) ts_render_kernel(const RenderArgs a, const
     const uint32_t L = frames / kSegs;
     const uint32_t orow = __float_as_uint(P[P_ROW * vp]);
     float* __restrict__ gout = a.voice_out + (size_t)orow * a.row_stride;
-    const int q = lane >> 3, c4 = (lane & 7) * 4;
 
     if (__float_as_uint(P[P_ACTIVE * vp]) == 0u) {
         // inactive voices render silence (their state does not move)
@@ -174,33 +167,27 @@ __global__ void __launch_bounds__(32) ts_render_kernel(const RenderArgs a, const
             __stcs(reinterpret_cast<float4*>(gout + t), make_float4(0.0f, 0.0f, 0.0f, 0.0f));
         return;
     }
-    const uint32_t kind = __float_as_uint(P[P_KIND * vp]);
+    const Lane V = load_lane(P, vp, sr, __float_as_uint(P[P_RELEASE * vp]));
+    const uint32_t kind = V.kind, rot = V.rot;
     if (kind == 3u) {
         for (int i = lane; i < 1024; i += 32) sintab[i] = __uint_as_float(d_sin_bits[i]);
     }
-    const uint32_t seed = __float_as_uint(P[P_SEED * vp]);
-    const uint32_t rot = (seed << 5) | (seed >> 27);
-    const uint32_t release = __float_as_uint(P[P_RELEASE * vp]);
-    EnvP A, M;
-    make_env(A, P[P_AA * vp], P[P_AD * vp], P[P_AS * vp], P[P_AR * vp], release, sr);
-    make_env(M, P[P_MA * vp], P[P_MD * vp], P[P_MS * vp], P[P_MR * vp], release, sr);
-    const EnvQ Aq = compact(A);
+    const EnvQ Aq = compact(V.amp);
     float* __restrict__ S = a.state + slot;
     const uint32_t n0 = __float_as_uint(S[S_OFFSET * vp]);
 
     // constants of the block: the host admitted this voice because its period and cutoff do not move
-    const float amt_lpf = P[P_AMT_LPF * vp];
-    const float m = (amt_lpf != 0.0f && env_stage(M, __uint2float_rn(n0)) == 2) ? M.S : 0.0f;
-    const float fl = modulate_freq(P[P_LPF * vp], m, amt_lpf);
+    const float m = (V.amt_lpf != 0.0f && env_stage(V.mod, __uint2float_rn(n0)) == 2) ? V.mod.S : 0.0f;
+    const float fl = modulate_freq(V.lpf, m, V.amt_lpf);
     OscC oc;
     FiltC fc;
-    make_osc(oc, P[P_PITCH * vp], sr);
-    make_filt<FILTER>(fc, fl, P[P_DAMP * vp], sr);
+    make_osc(oc, V.pitch, sr);
+    make_filt<FILTER>(fc, fl, V.damp, sr);
 
     FastV F;
-    F.P = oc.P; F.d = oc.d; F.slope = oc.slope; F.nhalf = -oc.half; F.ts1 = oc.ts1; F.ts2 = oc.ts2;
-    F.gain = P[P_GAIN * vp]; F.namt = P[P_NOISE * vp];
-    F.c0 = fc.c0; F.c1 = fc.c1; F.c2 = fc.c2;
+    set_osc(F, oc);
+    F.gain = V.gain; F.namt = V.namt;
+    F.fc = fc;
     F.es = 0.0f; F.nex0 = 0.0f; F.ey0 = 1.0f; F.seg_end = 0u;
     const float* __restrict__ sp = seg_phase + (size_t)slot * (3 * kSegs);
     const float ph0 = sp[lane];
@@ -217,23 +204,19 @@ __global__ void __launch_bounds__(32) ts_render_kernel(const RenderArgs a, const
             float pa = sp[kSegs + lane], pb = sp[2 * kSegs + lane];
             const float oa = osc_step<-1, false>(kind, oc, pa, sintab);
             const float ob = osc_step<-1, false>(kind, oc, pb, sintab);
-            x1_in = __fadd_rn(__fadd_rn(oa, F.gain), __fadd_rn(noise_fast(rot, nl - 1u), F.namt));
-            x2_in = __fadd_rn(__fadd_rn(ob, F.gain), __fadd_rn(noise_fast(rot, nl - 2u), F.namt));
+            x1_in = input1(F, oa, rot, nl - 1u);
+            x2_in = input1(F, ob, rot, nl - 2u);
         }
     }
 
     // ---- sweep 1: zero-state response of the segment (gain and output are irrelevant)
     float kprod = 1.0f;
     M22 mprod = {1.0, 0.0, 0.0, 1.0};
+    F.ph = ph0;
+    F.fs = {x1_in, x2_in, 0.0f, 0.0f};
     if (MOVING) {
-        float ph = ph0;
-        FiltS fs = {x1_in, x2_in, 0.0f, 0.0f};
-        ts_moving_sweep<FILTER, false>(A, M, P[P_LPF * vp], amt_lpf, P[P_DAMP * vp], sr, a.one, oc, kind, rot, F.gain, F.namt,
-                                       nl, L, ph, fs, kprod, mprod, tile, lane, gout, sintab);
-        F.y1 = fs.y1; F.y2 = fs.y2;
+        ts_moving_sweep<FILTER, false>(F, V, sr, a.one, nl, L, kprod, mprod, tile, lane, gout, sintab);
     } else {
-        F.ph = ph0;
-        F.x1 = x1_in; F.x2 = x2_in; F.y1 = 0.0f; F.y2 = 0.0f;
         for (uint32_t c = 0; c < L; c += kChunk) ts_chunk_kind<FILTER, true>(F, &Aq, a.one, kind, rot, nl + c, row, sintab);
     }
 
@@ -242,7 +225,7 @@ __global__ void __launch_bounds__(32) ts_render_kernel(const RenderArgs a, const
     if (FILTER == 0) {
         const float last = S[S_LAST * vp];
         float Kc = MOVING ? kprod : (float)exp((double)L * log((double)fc.c0));   // k^L (one value per voice)
-        float Yc = F.y1;
+        float Yc = F.fs.y1;
 #pragma unroll
         for (int off = 1; off < 32; off <<= 1) {
             const float Kp = __shfl_up_sync(0xffffffffu, Kc, off);
@@ -265,7 +248,7 @@ __global__ void __launch_bounds__(32) ts_render_kernel(const RenderArgs a, const
                 base = mul(base, base);
             }
         }
-        double z1 = (double)F.y1, z2 = (double)F.y2;          // zero-state response of this segment
+        double z1 = (double)F.fs.y1, z2 = (double)F.fs.y2;          // zero-state response of this segment
 #pragma unroll
         for (int off = 1; off < 32; off <<= 1) {
             const M22 Mp = shfl_up(Mc, off);
@@ -286,30 +269,19 @@ __global__ void __launch_bounds__(32) ts_render_kernel(const RenderArgs a, const
     }
 
     // ---- sweep 2: the reference recurrence from the true start state, written out
+    F.ph = ph0;
+    F.fs = {x1_in, x2_in, y1_in, y2_in};
     if (MOVING) {
-        float ph = ph0;
-        FiltS fs = {x1_in, x2_in, y1_in, y2_in};
-        ts_moving_sweep<FILTER, true>(A, M, P[P_LPF * vp], amt_lpf, P[P_DAMP * vp], sr, a.one, oc, kind, rot, F.gain, F.namt,
-                                      nl, L, ph, fs, kprod, mprod, tile, lane, gout, sintab);
-        F.x1 = fs.x1; F.x2 = fs.x2; F.y1 = fs.y1; F.y2 = fs.y2;
+        ts_moving_sweep<FILTER, true>(F, V, sr, a.one, nl, L, kprod, mprod, tile, lane, gout, sintab);
     } else {
-        F.ph = ph0;
-        F.x1 = x1_in; F.x2 = x2_in; F.y1 = y1_in; F.y2 = y2_in;
         for (uint32_t c = 0; c < L; c += kChunk) {
             ts_chunk_kind<FILTER, false>(F, &Aq, a.one, kind, rot, nl + c, row, sintab);
-            __syncwarp();
-#pragma unroll
-            for (int i = 0; i < 8; i++) {
-                const int r = 4 * i + q;                      // tile row = segment r
-                const float4 val = *reinterpret_cast<const float4*>(tile + r * kTsTileStride + c4);
-                __stcs(reinterpret_cast<float4*>(gout + (size_t)r * L + c + c4), val);
-            }
-            __syncwarp();
+            ts_store_tile(tile, lane, gout, L, c);
         }
     }
     if (lane == 31) {
-        if (FILTER == 0) S[S_LAST * vp] = F.y1;
-        else { S[S_X1 * vp] = F.x1; S[S_X2 * vp] = F.x2; S[S_Y1 * vp] = F.y1; S[S_Y2 * vp] = F.y2; }
+        if (FILTER == 0) S[S_LAST * vp] = F.fs.y1;
+        else { S[S_X1 * vp] = F.fs.x1; S[S_X2 * vp] = F.fs.x2; S[S_Y1 * vp] = F.fs.y1; S[S_Y2 * vp] = F.fs.y2; }
         S[S_OFFSET * vp] = __uint_as_float(n0 + frames);      // n0 + frames <= 2^24 (host check)
     }
 }

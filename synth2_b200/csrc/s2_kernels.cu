@@ -12,8 +12,6 @@
 // Reference line numbers are relative to /root/reference/components/s2_lib/src/.
 #include "s2_device.cuh"
 
-#include <type_traits>
-
 // Register cap of the render kernel, as a minimum of resident one-warp blocks per SM: 16 blocks = 65,536 / (16 * 32)
 // = 128 registers.  Shared memory (14.8 KB + 1 KB per block) already limits an SM to 14 blocks — the 13.8 a
 // 65,536-voice bank needs — so nothing is lost against the 96 registers of round 1, and the chunk-level state
@@ -65,23 +63,20 @@ __device__ __forceinline__ void fast_tile(int gmode, bool fasthash, FastV& F, co
 // 65,536 voices = 13.8 one-warp blocks per SM: without pipelining all of them must be resident at once (a
 // second wave would serialise: measured +20 % time at 144 registers, where only 13 fit).
 template <int FILTER, int TRACE>
-__global__ void __launch_bounds__(kWarpsPerBlock * 32, S2_MINBLOCKS)
+__global__ void __launch_bounds__(32, S2_MINBLOCKS)
 render_kernel(const RenderArgs a) {
     extern __shared__ __align__(16) float smem[];
-    const int warp = threadIdx.x >> 5;
-    const int lane = threadIdx.x & 31;
+    const int lane = threadIdx.x;
     constexpr int kRows = 32;
-    constexpr int kTileFloats = kRows * kTileStride;
-    float* wsm = smem + warp * warp_smem_floats();
-    float* tile = wsm;
-    float* cold_base = wsm + kTileFloats;
-    float* sintab = smem + kWarpsPerBlock * warp_smem_floats();
+    float* tile = smem;
+    float* cold_base = smem + kRows * kTileStride;
+    float* sintab = smem + warp_smem_floats();
     if (a.has_sine) {
-        for (int i = threadIdx.x; i < 1024; i += kWarpsPerBlock * 32) sintab[i] = __uint_as_float(d_sin_bits[i]);
+        for (int i = lane; i < 1024; i += 32) sintab[i] = __uint_as_float(d_sin_bits[i]);
         __syncthreads();
     }
 
-    const uint32_t vbase = a.slot_begin + (blockIdx.x * kWarpsPerBlock + warp) * kRows;
+    const uint32_t vbase = a.slot_begin + blockIdx.x * kRows;
     if (vbase >= a.slot_end) return;
     const uint32_t vp = a.vpad;
     const float sr = a.sample_rate;
@@ -92,7 +87,7 @@ render_kernel(const RenderArgs a) {
 
     uint32_t kind, rot, n;
     bool active;
-    FastV F;
+    FastV F{};
     {
         const uint32_t v = vbase + lane;
         const bool exists = v < a.slot_end;
@@ -120,10 +115,10 @@ render_kernel(const RenderArgs a) {
         F.ph = __float_as_uint(S[S_HAS_PHASE * vp]) != 0u ? S[S_PHASE * vp] : 0.0f;   // process.rs:316
         n = __float_as_uint(S[S_OFFSET * vp]);
         if (FILTER == 0) {
-            F.y1 = S[S_LAST * vp]; F.x1 = 0.0f; F.x2 = 0.0f; F.y2 = 0.0f;
+            F.fs.y1 = S[S_LAST * vp];
         } else {
-            F.x1 = S[S_X1 * vp]; F.x2 = S[S_X2 * vp];
-            F.y1 = S[S_Y1 * vp]; F.y2 = S[S_Y2 * vp];
+            F.fs.x1 = S[S_X1 * vp]; F.fs.x2 = S[S_X2 * vp];
+            F.fs.y1 = S[S_Y1 * vp]; F.fs.y2 = S[S_Y2 * vp];
         }
         F.gain = L.gain;
         F.namt = L.namt;
@@ -139,9 +134,6 @@ render_kernel(const RenderArgs a) {
         C.fc = fc;
         C.n_safe = 0u;
         C.msg.es = C.msg.nex0 = C.msg.ey0 = 0.0f; C.msg.nbeg = 1u; C.msg.nend = 0u; C.msg.stage = 4;
-        F.P = 0.0f; F.d = 0.0f; F.slope = 0.0f; F.nhalf = 0.0f; F.ts1 = 0.0f; F.ts2 = 0.0f;
-        F.c0 = 0.0f; F.c1 = 0.0f; F.c2 = 0.0f;
-        F.es = 0.0f; F.nex0 = 0.0f; F.ey0 = 0.0f;
         F.seg_end = active ? 0u : 0xffffffffu;
     }
     bool lane_gconst = true;          // the lane's current amp segment (F.es ..) is a sustain / end stage
@@ -217,7 +209,7 @@ render_kernel(const RenderArgs a) {
     // this warp's partial row of the mix, from launch parameters and the block index only (uniform registers: a
     // pointer kept live across the chunk loop is spilled under the register cap and reloaded from local memory)
     auto bus_row = [&]() -> float* {
-        return a.bus_partials + (size_t)(a.slot_begin / (uint32_t)kRows + blockIdx.x * (uint32_t)kWarpsPerBlock + (uint32_t)warp) * a.frames;
+        return a.bus_partials + (size_t)(a.slot_begin / (uint32_t)kRows + blockIdx.x) * a.frames;
     };
     // (16-byte stores into the partial row: needs frames % 4 == 0 and an aligned base)
     const bool bus_wide_ok = a.bus_partials != nullptr && a.n_voices > 32u && (frames & 3u) == 0u &&
@@ -321,8 +313,8 @@ render_kernel(const RenderArgs a) {
                             if (!sane) n_safe = 0u;
                             lane_fast = sane && n + kChunk <= n_safe;
                             // publish into the lane's registers
-                            F.P = oc.P; F.d = oc.d; F.slope = oc.slope; F.nhalf = -oc.half; F.ts1 = oc.ts1; F.ts2 = oc.ts2;
-                            F.c0 = fc.c0; F.c1 = fc.c1; F.c2 = fc.c2;
+                            set_osc(F, oc);
+                            F.fc = fc;
                         } else if (!mconst && C.amt_osc == 0.0f && n + kChunk <= sm.nend) {
                             // the mod envelope ramps through the whole chunk and only the cutoff follows it: the period
                             // is the per-voice constant sr / pitch -> moving-cutoff chunk
@@ -331,7 +323,7 @@ render_kernel(const RenderArgs a) {
                             if (oc.d < 1.0f && oc.P > 1.0f) {
                                 lane_semi = true;
                                 C.msg = sm;
-                                F.P = oc.P; F.d = oc.d; F.slope = oc.slope; F.nhalf = -oc.half; F.ts1 = oc.ts1; F.ts2 = oc.ts2;
+                                set_osc(F, oc);
                             }
                         }
                         C.n_safe = n_safe;
@@ -379,13 +371,8 @@ render_kernel(const RenderArgs a) {
                 const uint32_t n_chunks = reps ? reps * (kTile / (uint32_t)kChunk) : 1u;
                 uint32_t hh = h0, ts = t0;
                 for (uint32_t k = 0; k < n_chunks; k++) {
-                    switch (wkind) {
-                    case 0: fast_tile<FILTER, 0, TRACE>(gmode, fasthash, F, &C.amp, one, kind, rot, n, row + hh, sintab); break;
-                    case 1: fast_tile<FILTER, 1, TRACE>(gmode, fasthash, F, &C.amp, one, kind, rot, n, row + hh, sintab); break;
-                    case 2: fast_tile<FILTER, 2, TRACE>(gmode, fasthash, F, &C.amp, one, kind, rot, n, row + hh, sintab); break;
-                    case 3: fast_tile<FILTER, 3, TRACE>(gmode, fasthash, F, &C.amp, one, kind, rot, n, row + hh, sintab); break;
-                    default: fast_tile<FILTER, -1, TRACE>(gmode, fasthash, F, &C.amp, one, kind, rot, n, row + hh, sintab); break;
-                    }
+                    with_kind<0, 1, 2, 3, -1>(wkind, [](auto K, auto&&... args) { fast_tile<FILTER, K, TRACE>(args...); },
+                                              gmode, fasthash, F, &C.amp, one, kind, rot, n, row + hh, sintab);
                     if (TRACE != TRACE_PHASE && seg_left < (uint32_t)kChunk) edge_gain(edge, hh, n);
                     n += kChunk;
                     hh += (uint32_t)kChunk;
@@ -413,6 +400,7 @@ render_kernel(const RenderArgs a) {
                 SegEnv sm = C.msg;
                 mv.mes = sm.es; mv.mnex0 = sm.nex0; mv.mey0 = sm.ey0;
                 constexpr bool kPackable = FILTER == FILT_ONE_POLE || FILTER == FILT_BIQUAD_LP || FILTER == FILT_BIQUAD_HP;
+                constexpr bool kPairable = FILTER == FILT_BIQUAD_LP || FILTER == FILT_BIQUAD_HP;
                 // the packed forms take the amp envelope as one line through the chunk (as G_LINE); a lane with a stage
                 // boundary inside the chunk takes a gain of 1 and edge_gain afterwards
                 auto amp_line = [&]() {
@@ -421,36 +409,38 @@ render_kernel(const RenderArgs a) {
                         F.es = sg.es; F.nex0 = sg.nex0; F.ey0 = sg.ey0; F.seg_end = sg.nend;
                         lane_gconst = sg.stage == 2 || sg.stage == 4;
                     }
-                    return active && F.seg_end - n < (uint32_t)kChunk;
+                    const bool edge = active && F.seg_end - n < (uint32_t)kChunk;
+                    if (edge) { F.es = 0.0f; F.nex0 = 0.0f; F.ey0 = 1.0f; }
+                    return edge;
                 };
+                const bool packable = a.force_path == 0u || a.force_path == 3u;
                 if (filt_uniform) {
                     // one cutoff trajectory for the whole warp: 32 frames' coefficients, one per lane, once; the
-                    // packed loop reads them
+                    // chunk reads them
                     const Cold& CL = *reinterpret_cast<const Cold*>(cold_base + leader * kColdWords);
                     const uint32_t n_lead = __shfl_sync(0xffffffffu, n, leader);   // inactive lanes hold other offsets
                     const CutP cpl = cutp_of(CL.lpf, CL.theta0, CL.amt_lpf, CL.damp, sr, rsr);
                     const SegEnv sml = CL.msg;
                     modcut_coefficients<FILTER>(sml, cpl, one, n_lead, lane, ctab);
                     __syncwarp();
-                    if (a.force_path == 0u || a.force_path == 3u) {
+                    if (packable) {
                         const bool edge = amp_line();
-                        if (edge) { F.es = 0.0f; F.nex0 = 0.0f; F.ey0 = 1.0f; }
                         s2c::Window W;
                         window_none(W);
-                        switch (wkind) {
-                        case 0: chunk_modcut_pk<FILTER, 0, TRACE, true>(F, mv, W, one, kind, rot, n, crow, sintab, ctab); break;
-                        case 1: chunk_modcut_pk<FILTER, 1, TRACE, true>(F, mv, W, one, kind, rot, n, crow, sintab, ctab); break;
-                        default: chunk_modcut_pk<FILTER, -1, TRACE, true>(F, mv, W, one, kind, rot, n, crow, sintab, ctab); break;
-                        }
+                        with_kind<0, 1, -1>(wkind, [](auto K, auto&&... args) { chunk_modcut_pk<FILTER, K, TRACE, true>(args...); },
+                                            F, mv, W, one, kind, rot, n, crow, sintab, ctab);
                         if (TRACE != TRACE_PHASE) edge_gain(edge, h0, n);
                     } else {
                         chunk_modcut_sc<FILTER, -1, TRACE, true>(F, &C.amp, mv, sm, one, kind, rot, n, crow, sintab, ctab);
                     }
                     __syncwarp();          // ctab is rewritten by the next moving-cutoff chunk
                 } else {
-                    // packed: the moving lanes aligned and (second-order filters) with a valid window.  Otherwise one
-                    // frame at a time.
-                    bool packed = false, edge = false;
+                    // each lane's own coefficients: packed where every moving lane is aligned and (second-order filters)
+                    // has a valid window, paired where moreover no lane pair (2i, 2i + 1) holds two moving lanes (the
+                    // resting lane of a pair helps); otherwise one frame at a time
+                    enum { ONE_FRAME, PACKED, PAIRED };
+                    int form = ONE_FRAME;
+                    bool edge = false;
                     s2c::Window W;
                     window_none(W);
                     if constexpr (kPackable) {
@@ -463,35 +453,23 @@ render_kernel(const RenderArgs a) {
                                 ok = W.valid != 0u;
                             }
                         }
-                        packed = (a.force_path == 0u || a.force_path == 3u) && __all_sync(0xffffffffu, ok);
-                    }
-                    if (packed) {
-                        if constexpr (kPackable) {
-                            if (edge) { F.es = 0.0f; F.nex0 = 0.0f; F.ey0 = 1.0f; }
-                            // no lane pair (2i, 2i + 1) with two moving lanes: the resting lane of a pair helps
+                        if (packable && __all_sync(0xffffffffu, ok)) {
                             const uint32_t mmask = __ballot_sync(0xffffffffu, mv.moving);
-                            bool paired = false;
-                            if constexpr (FILTER != FILT_ONE_POLE) paired = (mmask & (mmask >> 1) & 0x55555555u) == 0u && a.force_path != 3u;
-                            if (paired) {
-                                if constexpr (FILTER != FILT_ONE_POLE) {
-                                    switch (wkind) {
-                                    case 0: chunk_modcut_pr<FILTER, 0, TRACE>(F, mv, W, one, kind, rot, n, crow, sintab); break;
-                                    case 1: chunk_modcut_pr<FILTER, 1, TRACE>(F, mv, W, one, kind, rot, n, crow, sintab); break;
-                                    default: chunk_modcut_pr<FILTER, -1, TRACE>(F, mv, W, one, kind, rot, n, crow, sintab); break;
-                                    }
-                                }
-                            } else {
-                                switch (wkind) {
-                                case 0: chunk_modcut_pk<FILTER, 0, TRACE>(F, mv, W, one, kind, rot, n, crow, sintab); break;
-                                case 1: chunk_modcut_pk<FILTER, 1, TRACE>(F, mv, W, one, kind, rot, n, crow, sintab); break;
-                                default: chunk_modcut_pk<FILTER, -1, TRACE>(F, mv, W, one, kind, rot, n, crow, sintab); break;
-                                }
-                            }
-                            if (TRACE != TRACE_PHASE) edge_gain(edge, h0, n);
+                            form = kPairable && (mmask & (mmask >> 1) & 0x55555555u) == 0u && a.force_path != 3u ? PAIRED : PACKED;
                         }
+                    }
+                    if (form == PAIRED) {
+                        if constexpr (kPairable)
+                            with_kind<0, 1, -1>(wkind, [](auto K, auto&&... args) { chunk_modcut_pr<FILTER, K, TRACE>(args...); },
+                                                F, mv, W, one, kind, rot, n, crow, sintab);
+                    } else if (form == PACKED) {
+                        if constexpr (kPackable)
+                            with_kind<0, 1, -1>(wkind, [](auto K, auto&&... args) { chunk_modcut_pk<FILTER, K, TRACE>(args...); },
+                                                F, mv, W, one, kind, rot, n, crow, sintab);
                     } else {
                         chunk_modcut_sc<FILTER, -1, TRACE, false>(F, &C.amp, mv, sm, one, kind, rot, n, crow, sintab, nullptr);
                     }
+                    if (TRACE != TRACE_PHASE && form != ONE_FRAME) edge_gain(edge, h0, n);
                 }
                 n += kChunk;
                 semi_left -= (uint32_t)kChunk;
@@ -504,17 +482,13 @@ render_kernel(const RenderArgs a) {
                     FiltC fc = C.fc;
                     MovG mg;
                     movg_init(mg, L.lpf, L.amt_lpf, L.damp, sr);
-                    float ph = F.ph;
-                    FiltS fs = {F.x1, F.x2, F.y1, F.y2};
                     for (uint32_t i = 0; i < cnt; i++) {
                         const bool scalar_sem = tc + i >= f16;
-                        crow[i] = general_frame<FILTER, TRACE>(L, sr, one, n, scalar_sem, oc, fc, mg, ph, fs, sintab);
+                        crow[i] = general_frame<FILTER, TRACE>(L, sr, one, n, scalar_sem, oc, fc, mg, F.ph, F.fs, sintab);
                         n += 1u;
                     }
                     C.oc = oc;
                     C.fc = fc;
-                    F.ph = ph;
-                    F.x1 = fs.x1; F.x2 = fs.x2; F.y1 = fs.y1; F.y2 = fs.y2;
                     C.n_safe = 0u;         // oc/fc may have moved: republish through the classifier
                 }
                 fast_left = semi_left = seg_left = 0u;
@@ -570,10 +544,10 @@ render_kernel(const RenderArgs a) {
         const uint32_t start = __float_as_uint(S[S_OFFSET * vp]);
         const uint32_t nxt = start + frames < start ? 0xffffffffu : start + frames;   // saturating (synth.rs:197)
         S[S_OFFSET * vp] = __uint_as_float(nxt);
-        if (FILTER == 0) S[S_LAST * vp] = F.y1;
+        if (FILTER == 0) S[S_LAST * vp] = F.fs.y1;
         else {
-            S[S_X1 * vp] = F.x1; S[S_X2 * vp] = F.x2;
-            S[S_Y1 * vp] = F.y1; S[S_Y2 * vp] = F.y2;
+            S[S_X1 * vp] = F.fs.x1; S[S_X2 * vp] = F.fs.x2;
+            S[S_Y1 * vp] = F.fs.y1; S[S_Y2 * vp] = F.fs.y2;
         }
         const OscC oc = C.oc;
         const FiltC fc = C.fc;
@@ -722,15 +696,14 @@ cudaError_t launch_set_voices(const float* batch, uint32_t m, uint32_t begin, ui
 
 uint32_t render_warps(uint32_t n_voices) { return (n_voices + 31u) / 32u; }
 
-static_assert((size_t)kWarpsPerBlock * warp_smem_floats() * sizeof(float) + 4096 <= 48 * 1024,
+static_assert(warp_smem_floats() * sizeof(float) + 4096 <= 48 * 1024,
               "the render kernel's dynamic shared memory must stay under the 48 KB that needs no opt-in");
 
+// One warp per block (DESIGN.md section 4.2).
 template <int FILTER, int TRACE>
 static cudaError_t launch_t(const RenderArgs& a, cudaStream_t stream) {
-    const uint32_t n_warps = render_warps(a.slot_end - a.slot_begin);
-    const uint32_t blocks = (n_warps + kWarpsPerBlock - 1) / kWarpsPerBlock;
-    const size_t smem = (size_t)kWarpsPerBlock * warp_smem_floats() * sizeof(float) + (a.has_sine ? 4096 : 0);
-    render_kernel<FILTER, TRACE><<<blocks, kWarpsPerBlock * 32, smem, stream>>>(a);
+    const size_t smem = warp_smem_floats() * sizeof(float) + (a.has_sine ? 4096 : 0);
+    render_kernel<FILTER, TRACE><<<render_warps(a.slot_end - a.slot_begin), 32, smem, stream>>>(a);
     return cudaGetLastError();
 }
 
