@@ -138,6 +138,34 @@ int s2_bank_set_releases(s2_bank* bank, const uint32_t* h_release);
 int s2_bank_render(s2_bank* bank, size_t frames, float* d_voice_out, size_t row_stride,
                    float* d_bus_out);
 
+/*
+ * Per-voice level meters.  Same as s2_bank_render, and for every active voice v also accumulates, in caller voice
+ * order:
+ *   d_sum_sq[v] += sum over this call's frames of y*y          (binary64 array, 8-byte aligned)
+ *   d_peak[v]    = max(d_peak[v], |y|) compared as magnitude bits (binary32 array, 4-byte aligned)
+ * d_voice_out and d_bus_out may both be NULL (meters only: no per-voice stores at all).
+ *
+ * The caller owns both device arrays (n_voices entries each); zeroing them starts a window (a block, a whole render,
+ * ...).  Note-ons, releases and state edits never touch them: a meter follows the voice index, not the note.
+ *   peak     exact: bits(peak) = max_u32(bits(peak), bits(y) & 0x7fffffff) over every rendered frame, the
+ *            `frames % 16` scalar-tail frames included, so a NaN sample ranks above +inf and reads back as NaN (a
+ *            second-order filter whose cutoff passes Nyquist blows up; a sweep wants to see it).
+ *   sum_sq   within 1e-6 relative of the exact sum of squares while every |y| < 2^64; non-finite once a square
+ *            overflows binary32 or a sample is NaN.  Deterministic: squares in binary32, a fixed pairwise tree over
+ *            each 64-frame tile counted from the call's first frame, tile totals added in binary64 to a per-call
+ *            total that is added to the meter.  Its bits depend only on the voice's parameters and state, `frames`
+ *            and the prior meter: the same with or without rows and bus, in the default and the pipelined modes.
+ * Inactive voices (and padding) leave their entries bit for bit unchanged.  Asynchronous on the bank's stream;
+ * pipelined, each voice range updates its own voices on its own stream, and the meters are complete after
+ * s2_bank_sync / s2_bank_join, like the rows.  Time-split mode: a metered block takes the default path (it is not
+ * counted by s2_bank_time_split_blocks).  A metered render issues the same kernel launches as the same plain render
+ * (in time-split mode: as the plain render on the default path).
+ * A NULL bank, a NULL meter or a misaligned meter returns S2_ERR_INVALID with nothing enqueued; every other check
+ * is s2_bank_render's.
+ */
+int s2_bank_render_metered(s2_bank* bank, size_t frames, float* d_voice_out, size_t row_stride,
+                           float* d_bus_out, double* d_sum_sq, float* d_peak);
+
 /* Same, then copies the bus to HOST memory and synchronises the stream (Synth::sample shape). */
 int s2_bank_render_bus_host(s2_bank* bank, size_t frames, float* d_voice_out, size_t row_stride,
                             float* h_bus_out);

@@ -60,6 +60,7 @@ SYMBOLS = {
     "s2_bank_release_voice": (_i, [_vp, _sz]),
     "s2_bank_set_releases": (_i, [_vp, _vp]),
     "s2_bank_render": (_i, [_vp, _sz, _vp, _sz, _vp]),
+    "s2_bank_render_metered": (_i, [_vp, _sz, _vp, _sz, _vp, _vp, _vp]),
     "s2_bank_render_bus_host": (_i, [_vp, _sz, _vp, _sz, _vp]),
     "s2_bank_render_bus_host_async": (_i, [_vp, _sz, _vp, _sz, _vp]),
     "s2_bank_get_state": (_i, [_vp, _vp]),

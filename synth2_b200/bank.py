@@ -90,9 +90,22 @@ class VoiceBank:
         check(lib().s2_bank_set_releases(self._h, ptr(release_offsets)))
 
     # -- rendering (device buffers: anything with .data_ptr(), or a raw address)
-    def render(self, frames: int, voice_out=None, row_stride: int = 0, bus_out=None):
+    def render(self, frames: int, voice_out=None, row_stride: int = 0, bus_out=None, sum_sq=None, peak=None):
+        """Render `frames` frames.  With `sum_sq` and `peak` (per-voice meters, given together: float64 and float32 device
+        tensors of n_voices, or raw addresses) every active voice also adds its sum of y*y to sum_sq and raises peak to
+        its largest |y| (s2_bank_render_metered); voice_out and bus_out may then both be None."""
         row_stride = _row_stride(voice_out, frames, row_stride)
-        check(lib().s2_bank_render(self._h, int(frames), ptr(voice_out), row_stride, ptr(bus_out)))
+        if sum_sq is None and peak is None:
+            check(lib().s2_bank_render(self._h, int(frames), ptr(voice_out), row_stride, ptr(bus_out)))
+            return
+        if sum_sq is None or peak is None:
+            raise ValueError("sum_sq and peak are given together")
+        for m, dtype in ((sum_sq, "float64"), (peak, "float32")):
+            if hasattr(m, "data_ptr") and (str(m.dtype) != "torch." + dtype or m.numel() != self.n_voices
+                                           or not m.is_contiguous()):
+                raise ValueError(f"a meter is a contiguous {dtype} tensor of {self.n_voices} entries")
+        check(lib().s2_bank_render_metered(self._h, int(frames), ptr(voice_out), row_stride, ptr(bus_out),
+                                           ptr(sum_sq), ptr(peak)))
 
     def render_bus_host(self, frames: int, voice_out=None, row_stride: int = 0, out: np.ndarray = None):
         """Render and return the mono mix in host memory (the `Synth::sample` shape)."""

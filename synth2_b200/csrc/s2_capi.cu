@@ -366,8 +366,10 @@ int settle_edits(s2_bank* b) {
     return rc ? rc : apply_staged_table(b);
 }
 
-// Every RenderArgs field from the bank, for the whole slot range, without bus partials or a staged table.
-s2::RenderArgs base_args(const s2_bank* b, size_t frames, float* d_voice_out, size_t row_stride) {
+// Every RenderArgs field from the bank, for the whole slot range, without bus partials or a staged table.  A plain
+// render is a metered one with null meters.
+s2::RenderArgs base_args(const s2_bank* b, size_t frames, float* d_voice_out, size_t row_stride, double* d_sum_sq,
+                         uint32_t* d_peak) {
     s2::RenderArgs a;
     a.params = b->d_params;
     a.state = b->d_state;
@@ -385,6 +387,8 @@ s2::RenderArgs base_args(const s2_bank* b, size_t frames, float* d_voice_out, si
     a.force_path = b->force_path;
     a.staged_release = nullptr;
     a.release_row = nullptr;
+    a.sum_sq = d_sum_sq;
+    a.peak = d_peak;
     return a;
 }
 
@@ -415,11 +419,12 @@ uint32_t sub_begin(const s2_bank* b, int k) {
     return (uint32_t)(s < b->n_voices ? s : b->n_voices);
 }
 
-int bank_render_pipelined(s2_bank* b, size_t frames, float* d_voice_out, size_t row_stride, float* d_bus_out) {
+int bank_render_pipelined(s2_bank* b, size_t frames, float* d_voice_out, size_t row_stride, float* d_bus_out,
+                          double* d_sum_sq, uint32_t* d_peak) {
     Pipeline& pl = b->pipe;
     const uint32_t n_warps = s2::render_warps((uint32_t)b->n_voices);
     const int p = (int)(pl.step % (uint64_t)kMixBufs);
-    s2::RenderArgs a = base_args(b, frames, d_voice_out, row_stride);
+    s2::RenderArgs a = base_args(b, frames, d_voice_out, row_stride, d_sum_sq, d_peak);
     if (d_bus_out) {
         int rc = grow(b, pl.d_partials, kMixBufs, pl.partials_cap, partials_floats(n_warps, frames));
         if (rc) return rc;
@@ -464,8 +469,9 @@ float host_ms_as_samples(float ms, float sr) { return sr * (ms / 1000.0f); }
 // block (no pitch modulation).  Returns 0 = no, 1 = yes and every cutoff rests too (mod envelope unused by the
 // cutoff, or in sustain / end until the block ends), 2 = yes but some cutoff follows a ramping mod envelope
 // (per-frame coefficients).  Conservative: anything unsure renders the general way.
-int ts_block_class(const s2_bank* b, size_t frames, const float* d_voice_out) {
+int ts_block_class(const s2_bank* b, size_t frames, const float* d_voice_out, bool metered) {
     if (!b->split.enabled || !d_voice_out) return 0;                            // the mix is summed from the rows
+    if (metered) return 0;                                                      // the time-split kernels have no meters
     if (frames < 1024 || (frames & 1023u) != 0 || frames > (1u << 24)) return 0;   // 32 segments of whole chunks
     const float sr = (float)b->sample_rate;
     int cls = 1;
@@ -497,7 +503,7 @@ int bank_render_time_split(s2_bank* b, size_t frames, float* d_voice_out, size_t
                            bool moving) {
     TimeSplit& ts = b->split;
     const int p = (int)(ts.step % (uint64_t)kTsBufs);
-    const s2::RenderArgs a = base_args(b, frames, d_voice_out, row_stride);
+    const s2::RenderArgs a = base_args(b, frames, d_voice_out, row_stride, nullptr, nullptr);
     if (ts.main_dirty) {
         // the pre-pass reads the carried phase: order it after whatever the bank's stream wrote
         CUDA_TRY(cudaEventRecord(ts.ev_main, b->stream));
@@ -530,7 +536,7 @@ int bank_render_time_split(s2_bank* b, size_t frames, float* d_voice_out, size_t
 }
 
 int bank_render_impl(s2_bank* b, size_t frames, float* d_voice_out, size_t row_stride, float* d_bus_out,
-                     int trace) {
+                     int trace, double* d_sum_sq = nullptr, uint32_t* d_peak = nullptr) {
     if (!b) return fail(S2_ERR_INVALID, "null bank");
     if (frames == 0) return S2_OK;
     if (frames > 0x7FFFFFFFull) return fail(S2_ERR_INVALID, "frames %zu too large for one call", frames);
@@ -550,18 +556,19 @@ int bank_render_impl(s2_bank* b, size_t frames, float* d_voice_out, size_t row_s
     }
     CUDA_TRY(cudaSetDevice(b->device));
     if (trace == s2::TRACE_NONE) {
-        const int cls = ts_block_class(b, frames, d_voice_out);
+        const int cls = ts_block_class(b, frames, d_voice_out, d_sum_sq != nullptr);
         if (cls) return bank_render_time_split(b, frames, d_voice_out, row_stride, d_bus_out, cls == 2);
     }
     b->split.main_dirty = true;   // the general kernels below move the carried phase on the bank's stream
-    if (b->n_sub > 1 && trace == s2::TRACE_NONE) return bank_render_pipelined(b, frames, d_voice_out, row_stride, d_bus_out);
+    if (b->n_sub > 1 && trace == s2::TRACE_NONE)
+        return bank_render_pipelined(b, frames, d_voice_out, row_stride, d_bus_out, d_sum_sq, d_peak);
     if (b->n_sub > 1) {   // a trace: it renders the whole bank on the bank's stream
         int rc = settle_edits(b);
         if (rc) return rc;
     }
 
     const uint32_t n_warps = s2::render_warps((uint32_t)b->n_voices);
-    s2::RenderArgs a = base_args(b, frames, d_voice_out, row_stride);
+    s2::RenderArgs a = base_args(b, frames, d_voice_out, row_stride, d_sum_sq, d_peak);
     if (d_bus_out) {
         if (n_warps == 1) {
             a.bus_partials = d_bus_out;   // a single warp sums its voices in index order: that IS the bus
@@ -945,6 +952,16 @@ int s2_bank_set_releases(s2_bank* b, const uint32_t* h_release) {
 
 int s2_bank_render(s2_bank* b, size_t frames, float* d_voice_out, size_t row_stride, float* d_bus_out) {
     return bank_render_impl(b, frames, d_voice_out, row_stride, d_bus_out, s2::TRACE_NONE);
+}
+
+int s2_bank_render_metered(s2_bank* b, size_t frames, float* d_voice_out, size_t row_stride, float* d_bus_out,
+                           double* d_sum_sq, float* d_peak) {
+    if (!b) return fail(S2_ERR_INVALID, "null bank");
+    if (!d_sum_sq || !d_peak) return fail(S2_ERR_INVALID, "null meter (sum_sq and peak are both required)");
+    if (((uintptr_t)d_sum_sq & 7u) != 0 || ((uintptr_t)d_peak & 3u) != 0)
+        return fail(S2_ERR_INVALID, "sum_sq must be 8-byte and peak 4-byte aligned");
+    return bank_render_impl(b, frames, d_voice_out, row_stride, d_bus_out, s2::TRACE_NONE, d_sum_sq,
+                            reinterpret_cast<uint32_t*>(d_peak));
 }
 
 int s2_bank_trace_phase(s2_bank* b, size_t frames, float* d_phase_out, size_t row_stride) {

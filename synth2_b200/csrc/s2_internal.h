@@ -32,7 +32,9 @@ enum StateIdx {
 };
 constexpr uint32_t kNoKey = 0x7fc00001u;   // a NaN payload no frequency can have
 
-enum TraceMode { TRACE_NONE = 0, TRACE_PHASE = 1 };
+// TRACE_METER: a render exactly as TRACE_NONE that also accumulates the per-voice meters of RenderArgs (sum_sq, peak);
+// launch_render takes it for a TRACE_NONE launch whose meters are set.
+enum TraceMode { TRACE_NONE = 0, TRACE_PHASE = 1, TRACE_METER = 2 };
 
 struct RenderArgs {
     const float* params;   // [P_COUNT][vpad]
@@ -55,6 +57,11 @@ struct RenderArgs {
     uint32_t force_path;   // test hook (S2_FORCE_PATH): 0 = normal, 1 = moving-cutoff chunks one frame at a time,
                            // 2 = every chunk through the general per-frame path, 3 = packed moving-cutoff chunks
                            // without the lane-pair help (chunk_modcut_pk only)
+    // Per-voice meters (s2_bank_render_metered), indexed by the caller's voice index, or both nullptr: every active
+    // voice adds its sum of y*y over the launch's frames to sum_sq and raises peak to its largest |y| (magnitude
+    // bits).  Last, so that the fields above keep their parameter offsets in the unmetered kernels.
+    double* sum_sq;
+    uint32_t* peak;
 };
 
 constexpr int kChunk = 32;          // frames per compute chunk (classification granularity)

@@ -40,6 +40,48 @@ __device__ __forceinline__ void tree_sum_rows(float4 (&val)[N], float2& b01, flo
     b23 = make_float2(val[0].z, val[0].w);
 }
 
+// Shared memory of a metered launch (TRACE_METER), after the warp's tiles: each lane's running meters, double
+// sum_sq[32] then uint32 peak[32].  Kept there rather than in registers, which the chunk loops use up to the cap.
+constexpr int kMeterFloats = 32 * 2 + 32;
+__device__ __forceinline__ double* meter_sum(float* smem) { return reinterpret_cast<double*>(smem + warp_smem_floats()); }
+__device__ __forceinline__ uint32_t* meter_peak(float* smem) { return reinterpret_cast<uint32_t*>(smem + warp_smem_floats() + 64); }
+
+// Meters of one 64-frame tile row (the lane's own): squares in binary32, summed by a fixed pairwise tree over the 64
+// columns counted from the tile's first frame, the tile total added to the binary64 running total; the peak is the
+// largest magnitude as bits (sign cleared), so a NaN ranks above +inf.  A partial tile zeroes its columns from `cnt`
+// on first (other lanes read only the first `cnt`).  One tree for every tile of every write-back: the total's bits
+// do not depend on whether rows or a bus are stored.
+__device__ __forceinline__ void meter_row(float* row, uint32_t cnt, float one, double& sum_sq, uint32_t& peak) {
+    if (cnt < (uint32_t)kTileFrames)
+        for (uint32_t c = cnt; c < (uint32_t)kTileFrames; c++) row[c] = 0.0f;
+    constexpr uint32_t m = 0x7fffffffu;
+    uint32_t pk = peak;
+    float2 half[2];
+#pragma unroll
+    for (int hh = 0; hh < 2; hh++) {
+        float2 s[16];
+#pragma unroll
+        for (int i = 0; i < 8; i++) {
+            const float4 v = *reinterpret_cast<const float4*>(row + 32 * hh + 4 * i);
+            s[2 * i] = pmul2(make_float2(v.x, v.y), make_float2(v.x, v.y));
+            s[2 * i + 1] = pmul2(make_float2(v.z, v.w), make_float2(v.z, v.w));
+            pk = __vimax3_u32(pk, __float_as_uint(v.x) & m, __float_as_uint(v.y) & m);
+            pk = __vimax3_u32(pk, __float_as_uint(v.z) & m, __float_as_uint(v.w) & m);
+        }
+        // the first level adds two products: vaddp, which ptxas cannot fuse with the multiplies (s2_cutoff.h)
+#pragma unroll
+        for (int i = 0; i < 16; i += 2) s[i] = s2c::vaddp(s[i], s[i + 1], one);
+#pragma unroll
+        for (int w = 2; w < 16; w <<= 1)
+#pragma unroll
+            for (int i = 0; i + w < 16; i += 2 * w) s[i] = padd2(s[i], s[i + w]);
+        half[hh] = s[0];
+    }
+    const float2 t = padd2(half[0], half[1]);
+    sum_sq = __dadd_rn(sum_sq, (double)__fadd_rn(t.x, t.y));
+    peak = pk;
+}
+
 // One fast chunk of a kind-uniform (or mixed, KIND = -1) warp, by envelope mode and hash form.
 // Instruction-cache budget: an SM holds 32 KB of instructions (L1.5; 6 KB per scheduler in L0) and its warps sit in
 // different loops (two oscillator kinds x envelope modes); once the loops in flight plus the per-chunk code outgrow
@@ -70,7 +112,12 @@ render_kernel(const RenderArgs a) {
     constexpr int kRows = 32;
     float* tile = smem;
     float* cold_base = smem + kRows * kTileStride;
-    float* sintab = smem + warp_smem_floats();
+    constexpr bool kMeter = TRACE == TRACE_METER;
+    float* sintab = smem + warp_smem_floats() + (kMeter ? kMeterFloats : 0);
+    if constexpr (kMeter) {
+        meter_sum(smem)[lane] = 0.0;
+        meter_peak(smem)[lane] = 0u;
+    }
     if (a.has_sine) {
         for (int i = lane; i < 1024; i += 32) sintab[i] = __uint_as_float(d_sin_bits[i]);
         __syncthreads();
@@ -214,8 +261,9 @@ render_kernel(const RenderArgs a) {
     // (16-byte stores into the partial row: needs frames % 4 == 0 and an aligned base)
     const bool bus_wide_ok = a.bus_partials != nullptr && a.n_voices > 32u && (frames & 3u) == 0u &&
                              (reinterpret_cast<uintptr_t>(a.bus_partials) & 15u) == 0u;
-    const bool simple_store = (gout == nullptr || all_rows) && (a.bus_partials == nullptr || bus_wide_ok) &&
-                              (gout != nullptr || a.bus_partials != nullptr);
+    bool simple_store = (gout == nullptr || all_rows) && (a.bus_partials == nullptr || bus_wide_ok);
+    if constexpr (!kMeter) simple_store = simple_store && (gout != nullptr || a.bus_partials != nullptr);
+    // (a metered launch without rows or a bus stores nothing per tile and takes the runs too)
     // Write-back of a full tile at frame ts.  ROWS: every tile row has an output row; MIX: per-warp partial sums of
     // a wide bank — each lane adds its 16 rows as two pairwise trees of packed adds, then the two q-groups are added
     // by one butterfly shuffle (a fixed tree: deterministic).  `checked`: rows may be missing (rp == 0).
@@ -379,7 +427,15 @@ render_kernel(const RenderArgs a) {
                     if (reps && hh == kTile) {
                         if (!active) { clear_chunk(row); clear_chunk(row + kChunk); }
                         __syncwarp();
-                        store_tile(ts, gout != nullptr, a.bus_partials != nullptr, false);
+                        if constexpr (kMeter) {
+                            // the lane's own row of the finished tile into its meters (inactive lanes reduce their
+                            // cleared rows: no divergence)
+                            if (gout != nullptr || a.bus_partials != nullptr)
+                                store_tile(ts, gout != nullptr, a.bus_partials != nullptr, false);
+                            meter_row(row, kTile, one, meter_sum(smem)[lane], meter_peak(smem)[lane]);
+                        } else {
+                            store_tile(ts, gout != nullptr, a.bus_partials != nullptr, false);
+                        }
                         __syncwarp();      // every lane is done reading the tile before the next one overwrites it
                         hh = 0u;
                         ts += kTile;
@@ -534,6 +590,7 @@ render_kernel(const RenderArgs a) {
                 gbus[t0 + c] = acc;
             }
         }
+        if constexpr (kMeter) meter_row(row, tcnt, one, meter_sum(smem)[lane], meter_peak(smem)[lane]);
         __syncwarp();      // every lane is done reading the tile before the next one overwrites it
     }
 
@@ -557,6 +614,12 @@ render_kernel(const RenderArgs a) {
         S[S_FL_KEY * vp] = __uint_as_float(fc.fl_bits);
         S[S_DAMP_KEY * vp] = C.damp;
         S[S_FC_C0 * vp] = fc.c0; S[S_FC_C1 * vp] = fc.c1; S[S_FC_C2 * vp] = fc.c2;
+        if constexpr (kMeter) {
+            // a voice is one lane of one launch, and a voice range's launches are stream-ordered: no atomics
+            const uint32_t r = C.out_row;
+            a.sum_sq[r] = __dadd_rn(a.sum_sq[r], meter_sum(smem)[lane]);
+            a.peak[r] = max(a.peak[r], meter_peak(smem)[lane]);
+        }
     }
 }
 
@@ -696,20 +759,26 @@ cudaError_t launch_set_voices(const float* batch, uint32_t m, uint32_t begin, ui
 
 uint32_t render_warps(uint32_t n_voices) { return (n_voices + 31u) / 32u; }
 
-static_assert(warp_smem_floats() * sizeof(float) + 4096 <= 48 * 1024,
+static_assert((warp_smem_floats() + kMeterFloats) * sizeof(float) + 4096 <= 48 * 1024,
               "the render kernel's dynamic shared memory must stay under the 48 KB that needs no opt-in");
+// A bank of 65,536 voices without sine voices needs 13.8 blocks per SM resident at once, metered or not: 14 blocks of
+// the metered size plus the 1 KB the runtime reserves per block (128-byte granules) fit the 228 KB of an SM.
+static_assert(14 * (((warp_smem_floats() + kMeterFloats) * sizeof(float) + 127) / 128 * 128 + 1024) <= 228 * 1024,
+              "a metered launch must keep 14 resident blocks per SM");
 
 // One warp per block (DESIGN.md section 4.2).
 template <int FILTER, int TRACE>
 static cudaError_t launch_t(const RenderArgs& a, cudaStream_t stream) {
-    const size_t smem = warp_smem_floats() * sizeof(float) + (a.has_sine ? 4096 : 0);
+    const size_t smem = (warp_smem_floats() + (TRACE == TRACE_METER ? kMeterFloats : 0)) * sizeof(float) +
+                        (a.has_sine ? 4096 : 0);
     render_kernel<FILTER, TRACE><<<render_warps(a.slot_end - a.slot_begin), 32, smem, stream>>>(a);
     return cudaGetLastError();
 }
 
 template <int FILTER>
 static cudaError_t launch_f(const RenderArgs& a, int trace, cudaStream_t stream) {
-    return trace == TRACE_PHASE ? launch_t<FILTER, TRACE_PHASE>(a, stream) : launch_t<FILTER, TRACE_NONE>(a, stream);
+    if (trace == TRACE_PHASE) return launch_t<FILTER, TRACE_PHASE>(a, stream);
+    return a.sum_sq ? launch_t<FILTER, TRACE_METER>(a, stream) : launch_t<FILTER, TRACE_NONE>(a, stream);
 }
 
 cudaError_t launch_render(const RenderArgs& a, uint32_t filter_kind, int trace, cudaStream_t stream) {
