@@ -101,8 +101,33 @@ void s2_default_voice(s2_voice_desc* out);
    stream) on which all work of this bank is enqueued. */
 int s2_bank_create(int device, uint32_t sample_rate, uint32_t filter_kind, size_t n_voices,
                    const s2_voice_desc* voices, void* stream, s2_bank** out);
+/*
+ * Mixed-filter bank: voice i renders through filter filter_kinds[i] (S2_FILTER_*).  Otherwise exactly
+ * s2_bank_create.  One bank then holds any patch the library renders (a sweep over filter types, a multitimbral
+ * host's parts), and one kernel launch renders every kind.
+ *   - Kinds are fixed per voice for the bank's life.  Every other entry (set_voice, set_voices, release_voice,
+ *     set_releases, get/set state, trace, pipelining, meters, s2_bank_reduce_bus) works unchanged; a note-on keeps
+ *     the voice's kind.  To change kinds, build a new bank (get/set state migrates the voices).
+ *   - Validation uses each voice's own kind: damping > 0 is required of second-order voices only.  A bad kind, a NULL
+ *     filter_kinds or a bad voice returns S2_ERR_INVALID before anything is allocated.
+ *   - Rows, meters and carried state of each voice are bit-identical to those of the same voice in a bank of its kind
+ *     made by s2_bank_create, given the same calls in the same order, in every mode.
+ *   - Bus: banks of up to 32 voices add in the reference's order, sequentially from 0.0 in voice order, in every
+ *     mode; with more than one kind the rows are rendered first (into an internal scratch when d_voice_out is NULL)
+ *     and added by one more kernel launch.  Wider banks: as s2_bank_render (deterministic, the same bits in the
+ *     default and pipelined modes, in no particular voice order).
+ *   - A mixed bank whose voices all share one kind is s2_bank_create with that kind, bit for bit.
+ *   - Voices are grouped by kind into whole warps of 32 slots, so a bank of K kinds may hold up to 31 * (K - 1)
+ *     padding slots.  The pipelined voice ranges are cut in slots: a narrow bank with several kinds may have more
+ *     non-empty ranges, so more launches per render, than a bank of one kind of the same width.
+ *   - s2_bank_set_time_split(bank, 1) on a bank of more than one kind returns S2_ERR_INVALID.
+ */
+int s2_bank_create_mixed(int device, uint32_t sample_rate, size_t n_voices, const s2_voice_desc* voices,
+                         const uint32_t* filter_kinds, void* stream, s2_bank** out);
 void s2_bank_destroy(s2_bank* bank);
 size_t s2_bank_voices(const s2_bank* bank);
+/* n_voices entries, in voice order.  Works for every bank: a single-kind bank reports its kind for every voice. */
+int s2_bank_filter_kinds(const s2_bank* bank, uint32_t* out);
 
 /* Replace one voice (note_on into slot `index`, synth.rs:61-70: fresh state, offset from desc). */
 int s2_bank_set_voice(s2_bank* bank, size_t index, const s2_voice_desc* voice);

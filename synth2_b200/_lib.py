@@ -53,8 +53,10 @@ SYMBOLS = {
     "s2_note_to_pitch": (_f, [_u8]),
     "s2_default_voice": (None, [_vp]),
     "s2_bank_create": (_i, [_i, _u32, _u32, _sz, _vp, _vp, C.POINTER(_vp)]),
+    "s2_bank_create_mixed": (_i, [_i, _u32, _sz, _vp, _vp, _vp, C.POINTER(_vp)]),
     "s2_bank_destroy": (None, [_vp]),
     "s2_bank_voices": (_sz, [_vp]),
+    "s2_bank_filter_kinds": (_i, [_vp, _vp]),
     "s2_bank_set_voice": (_i, [_vp, _sz, _vp]),
     "s2_bank_set_voices": (_i, [_vp, _sz, _vp, _vp]),
     "s2_bank_release_voice": (_i, [_vp, _sz]),

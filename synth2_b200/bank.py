@@ -25,6 +25,11 @@ def _row_stride(buf, frames: int, given: int) -> int:
     return int(buf.stride(0)) if hasattr(buf, "stride") else int(frames)
 
 
+def _stream_ptr(stream):
+    """A torch stream, a raw cudaStream_t or None (the default stream) as the library's `void* stream`."""
+    return None if stream is None else C.c_void_p(getattr(stream, "cuda_stream", stream))
+
+
 def default_voice(n: int = 1) -> np.ndarray:
     """`Synth::default_config()` (synth.rs:125-152) as n inactive voice descriptions."""
     one = np.zeros(1, dtype=VOICE_DESC)
@@ -35,17 +40,44 @@ def default_voice(n: int = 1) -> np.ndarray:
 class VoiceBank:
     def __init__(self, voices: np.ndarray, sample_rate: int = 48000,
                  filter_kind: int = _lib.FILTER_ONE_POLE, device: int = 0, stream=None):
+        voices = self._setup(voices, sample_rate, filter_kind, device)
+        check(lib().s2_bank_create(self.device, self.sample_rate, self.filter_kind, self.n_voices,
+                                   ptr(voices), _stream_ptr(stream), C.byref(self._h)))
+
+    def _setup(self, voices, sample_rate, filter_kind, device) -> np.ndarray:
+        """The handle and fields every bank has, before s2_bank_create(_mixed) fills the handle; returns the voices
+        as the contiguous array the library reads."""
         voices = np.ascontiguousarray(voices, dtype=VOICE_DESC)
         self._h = C.c_void_p()
         self.n_voices = int(voices.shape[0])
         self.sample_rate = int(sample_rate)
         self.filter_kind = int(filter_kind)
         self.device = int(device)
-        stream_ptr = None
-        if stream is not None:
-            stream_ptr = C.c_void_p(getattr(stream, "cuda_stream", stream))
-        check(lib().s2_bank_create(self.device, self.sample_rate, self.filter_kind, self.n_voices,
-                                   ptr(voices), stream_ptr, C.byref(self._h)))
+        return voices
+
+    @classmethod
+    def mixed(cls, voices: np.ndarray, filter_kinds, sample_rate: int = 48000, device: int = 0, stream=None):
+        """A bank whose voice i renders through filter filter_kinds[i] (s2_bank_create_mixed).  `filter_kind` is then
+        the kind of voice 0; `filter_kinds` has them all."""
+        voices = np.asarray(voices).reshape(-1)
+        kinds = np.asarray(filter_kinds).reshape(-1)
+        if kinds.size != voices.size:
+            raise ValueError(f"{kinds.size} filter kinds for {voices.size} voices")
+        if kinds.size and (kinds.min() < 0 or kinds.max() > 0xFFFFFFFF):
+            raise ValueError("filter kind out of range")
+        kinds = np.ascontiguousarray(kinds, dtype=np.uint32)
+        self = cls.__new__(cls)
+        voices = self._setup(voices, sample_rate, kinds[0] if kinds.size else 0, device)
+        check(lib().s2_bank_create_mixed(self.device, self.sample_rate, self.n_voices, ptr(voices), ptr(kinds),
+                                         _stream_ptr(stream), C.byref(self._h)))
+        return self
+
+    @property
+    def filter_kinds(self) -> np.ndarray:
+        """The filter kind of every voice, in voice order (np.uint32)."""
+        out = np.zeros(self.n_voices, dtype=np.uint32)
+        check(lib().s2_bank_filter_kinds(self._h, ptr(out)))
+        return out
 
     # -- lifetime
     def close(self):
@@ -144,8 +176,7 @@ class VoiceBank:
 
     def join(self, stream=None):
         """Make `stream` (a torch stream, a raw cudaStream_t, or None = default) wait for the bank's work."""
-        sp = None if stream is None else C.c_void_p(getattr(stream, "cuda_stream", stream))
-        check(lib().s2_bank_join(self._h, sp))
+        check(lib().s2_bank_join(self._h, _stream_ptr(stream)))
 
     # -- carried state
     def get_state(self) -> np.ndarray:

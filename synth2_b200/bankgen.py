@@ -7,7 +7,7 @@ rank can generate exactly its own voice range and the oracle and the GPU see ide
 """
 import numpy as np
 
-from ._lib import NO_RELEASE, OSC_SAW, OSC_SQUARE, VOICE_DESC
+from ._lib import FILTER_BIQUAD_BP, NO_RELEASE, OSC_SAW, OSC_SQUARE, VOICE_DESC
 from .bank import note_to_pitch
 
 _M = np.uint64(0xFFFFFFFFFFFFFFFF)
@@ -133,6 +133,32 @@ def make_sweep_bank(gpu_index: int, render_frames: int, first_variant: int = 0, 
     b["frame_offset"] = 0
     b["active"] = 1
     return b
+
+
+SWEEP_FILTER_KINDS = 6                # S2_FILTER_ONE_POLE .. S2_FILTER_FIRST_ORDER_HP
+
+
+def make_mixed_sweep_bank(gpu_index: int, render_frames: int, first_variant: int = 0, n_variants: int = None,
+                          sample_rate: int = 48000, kind=OSC_SAW):
+    """Config 5's sweep with the filter kind as a fourth axis: the variants of make_sweep_bank, each (cutoff, damping)
+    cell of 32 detunes rendered through filter kind `cell % 6` (the cells cycle through the six kinds, and the 32
+    detunes of a cell keep one kind, so they still fill one warp with one cutoff trajectory).  Returns (voices,
+    filter_kinds).
+
+    Band-pass voices read `damping` as their quality factor Q, and their coefficients need theta / (2 Q) below pi / 2
+    (dsp_filters.rs:197-207, tan); they keep a margin of two, theta / (2 Q) <= pi / 4, i.e. a cutoff of at most
+    Q * sample_rate / 4: their cutoff is clamped to that limit (and to 0.45 * sample_rate), and their mod amount to
+    the room left below it.  The other kinds keep make_sweep_bank's values.
+    """
+    b = make_sweep_bank(gpu_index, render_frames, first_variant, n_variants, sample_rate, kind)
+    vid = np.arange(first_variant, first_variant + b.shape[0], dtype=np.int64)
+    kinds = ((vid // SWEEP_AXIS) % SWEEP_FILTER_KINDS).astype(np.uint32)
+    bp = kinds == FILTER_BIQUAD_BP
+    limit = np.minimum(0.45 * float(sample_rate), b["damping"][bp].astype(np.float64) * float(sample_rate) / 4.0)
+    cutoff = np.minimum(b["lpf_freq_hz"][bp].astype(np.float64), limit).astype(np.float32)
+    b["lpf_freq_hz"][bp] = cutoff
+    b["mod_env_to_lpf_freq"][bp] = np.clip(np.log2(limit / cutoff.astype(np.float64)), 0.0, 1.5).astype(np.float32)
+    return b, kinds
 
 
 def default_bank(n: int) -> np.ndarray:

@@ -14,7 +14,7 @@ CSRC = PKG / "csrc"
 LIB = PKG / "libs2cuda.so"
 SOURCES = [CSRC / "s2_kernels.cu", CSRC / "s2_kernel_ts.cu", CSRC / "s2_capi.cu",
            CSRC / "s2_patch.cpp", CSRC / "s2_player.cpp", CSRC / "s2_nccl.cpp"]
-DEPS = SOURCES + [CSRC / "s2_internal.h", CSRC / "s2_device.cuh", CSRC / "s2_math.h", CSRC / "s2_cutoff.h",
+DEPS = SOURCES + [CSRC / "s2_internal.h", CSRC / "s2_render_body.inc", CSRC / "s2_device.cuh", CSRC / "s2_math.h", CSRC / "s2_cutoff.h",
                   CSRC / "sin_table_bits.inc",
                   PKG.parent / "include" / "s2_cuda.h"]
 

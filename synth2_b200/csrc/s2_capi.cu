@@ -272,8 +272,9 @@ struct s2_bank {
     int device = 0;
     cudaStream_t stream = nullptr;
     uint32_t sample_rate = 0;
-    uint32_t filter_kind = 0;
+    uint32_t filter_kind = 0;    // the kind of every voice, or of voice 0 of a mixed-filter bank
     size_t n_voices = 0;
+    size_t n_slots = 0;          // n_voices plus the padding slots of a mixed-filter bank
     size_t vpad = 0;
     float* d_params = nullptr;
     float* d_state = nullptr;
@@ -288,8 +289,13 @@ struct s2_bank {
     // 32 lanes of a warp run the same code for as long as possible, then dealt over the voice ranges; output
     // rows, state get/set and per-voice calls keep the caller's indices.  Banks of <= 32 voices keep
     // the identity order, which also keeps the bus sum in the reference's voice order.
+    // Mixed-filter banks: kinds are grouped, each group but the last padded to whole warps of 32 slots with padding
+    // slots (voice_of_slot = P_ROW = kPadRow, inactive).
     std::vector<uint32_t> slot_of_voice, voice_of_slot;
     bool identity = true;
+    std::vector<uint32_t> voice_kind;   // filter kind of each voice
+    uint32_t n_kinds = 1;               // distinct kinds; above 1 the render takes the mixed kernel
+    uint8_t* d_warp_kinds = nullptr;    // [n_slots / 32 rounded up] filter kind of each warp
     uint32_t force_path = 0;      // test hook (S2_FORCE_PATH, see RenderArgs)
     int n_sub = 1;                // voice ranges of the pipelined mode; 1 = everything on the bank's stream
     Pipeline pipe;
@@ -353,7 +359,7 @@ int apply_staged_table(s2_bank* b) {
     CUDA_TRY(cudaStreamWaitEvent(b->stream, pl.ev_stage[pl.table_pending], 0));
     CUDA_TRY(s2::launch_gather_u32(pl.d_staging[pl.table_pending], b->d_params + (size_t)s2::P_ROW * b->vpad,
                                    reinterpret_cast<uint32_t*>(b->d_params + (size_t)s2::P_RELEASE * b->vpad),
-                                   (uint32_t)b->n_voices, b->stream));
+                                   (uint32_t)b->n_slots, b->stream));
     g_launches.fetch_add(1, std::memory_order_relaxed);
     CUDA_TRY(cudaStreamSynchronize(b->stream));   // the staging buffer is free again before the next upload
     pl.table_pending = -1;
@@ -375,7 +381,7 @@ s2::RenderArgs base_args(const s2_bank* b, size_t frames, float* d_voice_out, si
     a.state = b->d_state;
     a.n_voices = (uint32_t)b->n_voices;
     a.slot_begin = 0;
-    a.slot_end = (uint32_t)b->n_voices;
+    a.slot_end = (uint32_t)b->n_slots;
     a.vpad = (uint32_t)b->vpad;
     a.sample_rate = (float)b->sample_rate;
     a.frames = (uint32_t)frames;
@@ -389,6 +395,7 @@ s2::RenderArgs base_args(const s2_bank* b, size_t frames, float* d_voice_out, si
     a.release_row = nullptr;
     a.sum_sq = d_sum_sq;
     a.peak = d_peak;
+    a.warp_kinds = b->n_kinds > 1 ? b->d_warp_kinds : nullptr;
     return a;
 }
 
@@ -411,24 +418,44 @@ int mix_partials(const s2_bank* b, float* partials, uint32_t n_warps, size_t fra
     return S2_OK;
 }
 
+// Multi-kind banks of up to 32 voices span several warps (one per kind).  Their bus is added from the rows, in voice
+// order from +0.0 as a one-warp bank adds it, after the render: into `a` go the caller's rows, or else a scratch of
+// n_voices rows of `frames` rounded up to 16 bytes in `scratch`.
+bool bus_from_rows(const s2_bank* b) { return b->n_kinds > 1 && b->n_voices <= 32; }
+size_t scratch_row_stride(size_t frames) { return (frames + 3) & ~(size_t)3; }
+
+void rows_for_bus(s2::RenderArgs& a, float* scratch, size_t frames) {
+    if (a.voice_out) return;
+    a.voice_out = scratch;
+    a.row_stride = scratch_row_stride(frames);
+}
+
+int mix_rows(const s2_bank* b, const s2::RenderArgs& a, size_t frames, float* bus, cudaStream_t st) {
+    CUDA_TRY(s2::launch_ts_mix_rows(a.voice_out, (uint32_t)b->n_voices, a.row_stride, (uint32_t)frames, bus, st));
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    return S2_OK;
+}
+
 uint32_t sub_begin(const s2_bank* b, int k) {
     // contiguous slot ranges, multiples of 64 slots so that warps (32 or 64 slots) never straddle two
-    const uint64_t groups = (b->n_voices + 63) / 64;
+    const uint64_t groups = (b->n_slots + 63) / 64;
     const uint64_t g = groups * (uint64_t)k / (uint64_t)b->n_sub;
     const uint64_t s = g * 64;
-    return (uint32_t)(s < b->n_voices ? s : b->n_voices);
+    return (uint32_t)(s < b->n_slots ? s : b->n_slots);
 }
 
 int bank_render_pipelined(s2_bank* b, size_t frames, float* d_voice_out, size_t row_stride, float* d_bus_out,
                           double* d_sum_sq, uint32_t* d_peak) {
     Pipeline& pl = b->pipe;
-    const uint32_t n_warps = s2::render_warps((uint32_t)b->n_voices);
+    const uint32_t n_warps = s2::render_warps((uint32_t)b->n_slots);
     const int p = (int)(pl.step % (uint64_t)kMixBufs);
     s2::RenderArgs a = base_args(b, frames, d_voice_out, row_stride, d_sum_sq, d_peak);
     if (d_bus_out) {
-        int rc = grow(b, pl.d_partials, kMixBufs, pl.partials_cap, partials_floats(n_warps, frames));
+        const size_t need = bus_from_rows(b) ? b->n_voices * scratch_row_stride(frames) : partials_floats(n_warps, frames);
+        int rc = grow(b, pl.d_partials, kMixBufs, pl.partials_cap, need);
         if (rc) return rc;
-        a.bus_partials = pl.d_partials[p];
+        if (bus_from_rows(b)) rows_for_bus(a, pl.d_partials[p], frames);
+        else a.bus_partials = pl.d_partials[p];
     }
     uint32_t* release_row = reinterpret_cast<uint32_t*>(b->d_params + (size_t)s2::P_RELEASE * b->vpad);
     for (int k = 0; k < b->n_sub; k++) {
@@ -452,7 +479,8 @@ int bank_render_pipelined(s2_bank* b, size_t frames, float* d_voice_out, size_t 
     pl.table_pending = -1;
     if (d_bus_out) {
         for (int k = 0; k < b->n_sub; k++) CUDA_TRY(cudaStreamWaitEvent(pl.mix, pl.ev_sub[k], 0));
-        int rc = mix_partials(b, a.bus_partials, n_warps, frames, d_bus_out, pl.mix);
+        int rc = bus_from_rows(b) ? mix_rows(b, a, frames, d_bus_out, pl.mix)
+                                  : mix_partials(b, a.bus_partials, n_warps, frames, d_bus_out, pl.mix);
         if (rc) return rc;
         CUDA_TRY(cudaEventRecord(pl.ev_mix[p], pl.mix));
     }
@@ -567,9 +595,13 @@ int bank_render_impl(s2_bank* b, size_t frames, float* d_voice_out, size_t row_s
         if (rc) return rc;
     }
 
-    const uint32_t n_warps = s2::render_warps((uint32_t)b->n_voices);
+    const uint32_t n_warps = s2::render_warps((uint32_t)b->n_slots);
     s2::RenderArgs a = base_args(b, frames, d_voice_out, row_stride, d_sum_sq, d_peak);
-    if (d_bus_out) {
+    if (d_bus_out && bus_from_rows(b)) {
+        int rc = grow(b, &b->d_partials, 1, b->partials_cap, b->n_voices * scratch_row_stride(frames));
+        if (rc) return rc;
+        rows_for_bus(a, b->d_partials, frames);
+    } else if (d_bus_out) {
         if (n_warps == 1) {
             a.bus_partials = d_bus_out;   // a single warp sums its voices in index order: that IS the bus
         } else {
@@ -583,11 +615,177 @@ int bank_render_impl(s2_bank* b, size_t frames, float* d_voice_out, size_t row_s
     // the next pipelined render launches on the sub-streams, which do not wait for the bank's stream
     if (b->n_sub > 1) CUDA_TRY(cudaStreamSynchronize(b->stream));
     if (d_bus_out) {
-        int rc = mix_partials(b, a.bus_partials, n_warps, frames, d_bus_out, b->stream);
+        int rc = bus_from_rows(b) ? mix_rows(b, a, frames, d_bus_out, b->stream)
+                                  : mix_partials(b, a.bus_partials, n_warps, frames, d_bus_out, b->stream);
         if (rc) return rc;
     }
     b->total_frames += frames;
     b->max_offset += frames;
+    return S2_OK;
+}
+
+// The order of one filter kind's voices `ids` (ascending voice indices) in their slots.  Groups of up to 32 voices
+// keep the voice order, which for a bank of one kind keeps the bus sum in the reference's voice order.
+void order_kind_group(const s2_voice_desc* voices, std::vector<uint32_t>& ids) {
+    const size_t n = ids.size();
+    if (n <= 32) return;
+    // (inactive last) x oscillator kind x when the amp envelope comes to rest: the 32 voices of a warp then leave
+    // the envelope ramps together instead of waiting for the slowest of a random draw.  Stable: a patch sweep
+    // keeps the variants of one cutoff trajectory next to each other.
+    // NOT a key: whether the cutoff follows the mod envelope.  Grouping the followers halves the warps that run
+    // moving-cutoff chunks, but a step is one launch per voice range and a range's launches run in order: the
+    // ranges of followers (1.9x the work per frame for 200 ms) fall behind the others and finish alone on a
+    // part-filled machine.  Measured on the bench bank, first 20 blocks: 6.2 ms grouped and contiguous, 7.1 ms
+    // grouped and dealt over the ranges, against mixed warps (every warp pays, all ranges in step).
+    struct Key { uint32_t kind; float amp_rest; };
+    auto key = [&](uint32_t v) -> Key {
+        const s2_voice_desc& d = voices[v];
+        return {d.active ? d.osc_kind : 4u, d.amp_attack_ms + d.amp_decay_ms};
+    };
+    std::stable_sort(ids.begin(), ids.end(), [&](uint32_t x, uint32_t y) {
+        const Key a = key(x);
+        const Key c = key(y);
+        if (a.kind != c.kind) return a.kind < c.kind;
+        return a.amp_rest < c.amp_rest;
+    });
+    // Instead the followers are PAIRED with voices whose cutoff rests: inside each kind, walking the sorted
+    // order, a follower and a non-follower that are next in line share an aligned lane pair (2i, 2i + 1), and the
+    // resting lane computes half of its partner's moving coefficients (chunk_modcut_pr).  Voices left without
+    // a partner come after the pairs, in the sorted order.
+    auto follows = [&](uint32_t v) { return voices[v].active && voices[v].mod_env_to_lpf_freq != 0.0f; };
+    std::vector<uint32_t> out, fq, nq;
+    out.reserve(n);
+    size_t g0 = 0;
+    while (g0 < n) {
+        size_t g1 = g0;
+        while (g1 < n && key(ids[g1]).kind == key(ids[g0]).kind) g1++;
+        fq.clear(); nq.clear();
+        size_t fi = 0, ni = 0;             // queue heads
+        for (size_t i = g0; i < g1; i++) {
+            const uint32_t v = ids[i];
+            (follows(v) ? fq : nq).push_back(v);
+            if (fi < fq.size() && ni < nq.size()) {
+                if (out.size() & 1u) { out.push_back(nq[ni++]); continue; }    // keep the pairs on even slots
+                out.push_back(fq[fi++]);
+                out.push_back(nq[ni++]);
+            }
+        }
+        // the unpaired: merge the two leftovers back into the sorted order
+        std::vector<uint32_t> left(fq.begin() + fi, fq.end());
+        left.insert(left.end(), nq.begin() + ni, nq.end());
+        std::stable_sort(left.begin(), left.end(), [&](uint32_t x, uint32_t y) { return key(x).amp_rest < key(y).amp_rest; });
+        out.insert(out.end(), left.begin(), left.end());
+        g0 = g1;
+    }
+    ids.swap(out);
+}
+
+// The bank's slots: voice_of_slot, with kPadRow for a padding slot.  Voices are grouped by filter kind (stably, in
+// kind order), each group is ordered by order_kind_group, and every group but the last is padded to whole warps of 32
+// slots, so that each warp runs one filter.  With one kind there is no padding.
+std::vector<uint32_t> layout_slots(const s2_voice_desc* voices, const std::vector<uint32_t>& kinds) {
+    std::vector<uint32_t> slots;
+    slots.reserve(kinds.size());
+    std::vector<uint32_t> ids;
+    for (uint32_t k = S2_FILTER_ONE_POLE; k <= S2_FILTER_FIRST_ORDER_HP; k++) {
+        ids.clear();
+        for (size_t v = 0; v < kinds.size(); v++)
+            if (kinds[v] == k) ids.push_back((uint32_t)v);
+        if (ids.empty()) continue;
+        while (slots.size() & 31u) slots.push_back(s2::kPadRow);
+        order_kind_group(voices, ids);
+        slots.insert(slots.end(), ids.begin(), ids.end());
+    }
+    // Deal the sorted warps (32 slots each) round-robin into 8 bins laid out one after the other: every contiguous
+    // eighth / quarter / half of the slot range — the voice ranges of s2_bank_set_pipeline — then holds the same
+    // mix of kinds and envelope lengths, so the ranges' streams advance together.
+    const size_t full_warps = slots.size() / 32;
+    if (full_warps >= 16) {
+        std::vector<uint32_t> dealt;
+        dealt.reserve(slots.size());
+        for (size_t bin = 0; bin < 8; bin++)
+            for (size_t w = bin; w < full_warps; w += 8)
+                dealt.insert(dealt.end(), slots.begin() + w * 32, slots.begin() + (w + 1) * 32);
+        dealt.insert(dealt.end(), slots.begin() + full_warps * 32, slots.end());
+        slots.swap(dealt);
+    }
+    return slots;
+}
+
+// s2_bank_create and s2_bank_create_mixed once their arguments are checked: `kinds` holds one valid filter kind per
+// voice.  Nothing is allocated on the device before every voice has passed validation.
+int bank_create(int device, uint32_t sample_rate, std::vector<uint32_t> kinds, const s2_voice_desc* voices,
+                void* stream, s2_bank** out) {
+    const size_t n_voices = kinds.size();
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
+        return fail(S2_ERR_NO_DEVICE, "no CUDA device (this library has no CPU path)");
+    if (device < 0 || device >= ndev) return fail(S2_ERR_NO_DEVICE, "device %d out of range (%d)", device, ndev);
+    for (size_t i = 0; i < n_voices; i++) {
+        int rc = validate_voice(voices[i], i, kinds[i]);
+        if (rc) return rc;
+    }
+    std::vector<uint32_t> voice_of_slot = layout_slots(voices, kinds);
+    if (voice_of_slot.size() > 0x7FFFFFE0ull) return fail(S2_ERR_INVALID, "too many voices");
+    CUDA_TRY(cudaSetDevice(device));
+
+    s2_bank* b = new (std::nothrow) s2_bank;
+    if (!b) return fail(S2_ERR_NOMEM, "out of host memory");
+    b->device = device;
+    b->stream = (cudaStream_t)stream;
+    b->sample_rate = sample_rate;
+    b->filter_kind = kinds[0];
+    b->n_voices = n_voices;
+    b->n_slots = voice_of_slot.size();
+    b->vpad = (b->n_slots + 63) & ~(size_t)63;
+    b->book.resize(n_voices);
+    if (n_voices <= kTsMaxVoices) b->split.descs.assign(voices, voices + n_voices);
+    if (const char* f = getenv("S2_FORCE_PATH")) b->force_path = (f[0] >= '1' && f[0] <= '3') ? (uint32_t)(f[0] - '0') : 0u;   // test hook
+
+    b->voice_of_slot.swap(voice_of_slot);
+    b->slot_of_voice.resize(n_voices);
+    for (size_t s = 0; s < b->n_slots; s++) {
+        const uint32_t v = b->voice_of_slot[s];
+        if (v != s) b->identity = false;
+        if (v != s2::kPadRow) b->slot_of_voice[v] = (uint32_t)s;
+    }
+    std::vector<uint8_t> warp_kinds((b->n_slots + 31) / 32);
+    for (size_t w = 0; w < warp_kinds.size(); w++) warp_kinds[w] = (uint8_t)kinds[b->voice_of_slot[w * 32]];   // never padding
+    uint32_t seen = 0;
+    for (uint32_t k : kinds) seen |= 1u << k;
+    b->n_kinds = (uint32_t)__builtin_popcount(seen);
+    b->voice_kind.swap(kinds);
+
+    std::vector<float> hp((size_t)s2::P_COUNT * b->vpad, 0.0f), hs((size_t)s2::S_COUNT * b->vpad, 0.0f);
+    for (size_t s = 0; s < b->n_slots; s++)
+        if (b->voice_of_slot[s] == s2::kPadRow) hp[(size_t)s2::P_ROW * b->vpad + s] = ubits(s2::kPadRow);   // inactive: zeros
+    for (size_t i = 0; i < n_voices; i++) {
+        const size_t slot = b->slot_of_voice[i];
+        pack_voice(voices[i], (uint32_t)i, hp.data() + slot, b->vpad);
+        s2_voice_state st;
+        memset(&st, 0, sizeof st);
+        st.frame_offset = voices[i].frame_offset;
+        pack_state(st, hs.data() + slot, b->vpad);
+        b->book[i] = {voices[i].frame_offset, 0, voices[i].active ? 1u : 0u, voices[i].osc_kind};
+        if (voices[i].active && voices[i].frame_offset > b->max_offset) b->max_offset = voices[i].frame_offset;
+        if (voices[i].osc_kind == S2_OSC_SINE) b->n_sine++;
+    }
+    cudaError_t e = cudaMalloc(&b->d_params, hp.size() * sizeof(float));
+    if (e == cudaSuccess) e = cudaMalloc(&b->d_state, hs.size() * sizeof(float));
+    if (e == cudaSuccess) e = cudaMalloc(&b->d_bus_counters, s2::kBusCounters * sizeof(unsigned int));
+    if (e == cudaSuccess) e = cudaMemsetAsync(b->d_bus_counters, 0, s2::kBusCounters * sizeof(unsigned int), b->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(b->d_params, hp.data(), hp.size() * sizeof(float), cudaMemcpyHostToDevice, b->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(b->d_state, hs.data(), hs.size() * sizeof(float), cudaMemcpyHostToDevice, b->stream);
+    if (e == cudaSuccess && b->n_kinds > 1) e = cudaMalloc(&b->d_warp_kinds, warp_kinds.size());
+    if (e == cudaSuccess && b->n_kinds > 1)
+        e = cudaMemcpyAsync(b->d_warp_kinds, warp_kinds.data(), warp_kinds.size(), cudaMemcpyHostToDevice, b->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(b->stream);
+    if (e != cudaSuccess) {
+        int rc = fail(e == cudaErrorMemoryAllocation ? S2_ERR_NOMEM : S2_ERR_CUDA, "bank upload: %s", cudaGetErrorString(e));
+        s2_bank_destroy(b);
+        return rc;
+    }
+    *out = b;
     return S2_OK;
 }
 
@@ -645,129 +843,22 @@ int s2_bank_create(int device, uint32_t sample_rate, uint32_t filter_kind, size_
     if (n_voices > 0x7FFFFFE0ull) return fail(S2_ERR_INVALID, "too many voices");
     if (sample_rate == 0) return fail(S2_ERR_INVALID, "sample_rate must be > 0");
     if (filter_kind > S2_FILTER_FIRST_ORDER_HP) return fail(S2_ERR_INVALID, "filter_kind %u", filter_kind);
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
-        return fail(S2_ERR_NO_DEVICE, "no CUDA device (this library has no CPU path)");
-    if (device < 0 || device >= ndev) return fail(S2_ERR_NO_DEVICE, "device %d out of range (%d)", device, ndev);
-    for (size_t i = 0; i < n_voices; i++) {
-        int rc = validate_voice(voices[i], i, filter_kind);
-        if (rc) return rc;
-    }
-    CUDA_TRY(cudaSetDevice(device));
+    return bank_create(device, sample_rate, std::vector<uint32_t>(n_voices, filter_kind), voices, stream, out);
+}
 
-    s2_bank* b = new (std::nothrow) s2_bank;
-    if (!b) return fail(S2_ERR_NOMEM, "out of host memory");
-    b->device = device;
-    b->stream = (cudaStream_t)stream;
-    b->sample_rate = sample_rate;
-    b->filter_kind = filter_kind;
-    b->n_voices = n_voices;
-    b->vpad = (n_voices + 63) & ~(size_t)63;
-    b->book.resize(n_voices);
-    if (n_voices <= kTsMaxVoices) b->split.descs.assign(voices, voices + n_voices);
-    if (const char* f = getenv("S2_FORCE_PATH")) b->force_path = (f[0] >= '1' && f[0] <= '3') ? (uint32_t)(f[0] - '0') : 0u;   // test hook
-
-    b->voice_of_slot.resize(n_voices);
-    b->slot_of_voice.resize(n_voices);
-    for (size_t i = 0; i < n_voices; i++) b->voice_of_slot[i] = (uint32_t)i;
-    if (n_voices > 32) {
-        // (inactive last) x oscillator kind x when the amp envelope comes to rest: the 32 voices of a warp then leave
-        // the envelope ramps together instead of waiting for the slowest of a random draw.  Stable: a patch sweep
-        // keeps the variants of one cutoff trajectory next to each other.
-        // NOT a key: whether the cutoff follows the mod envelope.  Grouping the followers halves the warps that run
-        // moving-cutoff chunks, but a step is one launch per voice range and a range's launches run in order: the
-        // ranges of followers (1.9x the work per frame for 200 ms) fall behind the others and finish alone on a
-        // part-filled machine.  Measured on the bench bank, first 20 blocks: 6.2 ms grouped and contiguous, 7.1 ms
-        // grouped and dealt over the ranges, against mixed warps (every warp pays, all ranges in step).
-        struct Key { uint32_t kind; float amp_rest; };
-        std::vector<Key> keys(n_voices);
-        for (size_t i = 0; i < n_voices; i++) {
-            const s2_voice_desc& d = voices[i];
-            keys[i] = {d.active ? d.osc_kind : 4u, d.amp_attack_ms + d.amp_decay_ms};
-        }
-        std::stable_sort(b->voice_of_slot.begin(), b->voice_of_slot.end(), [&](uint32_t x, uint32_t y) {
-            const Key& a = keys[x];
-            const Key& c = keys[y];
-            if (a.kind != c.kind) return a.kind < c.kind;
-            return a.amp_rest < c.amp_rest;
-        });
-        // Instead the followers are PAIRED with voices whose cutoff rests: inside each kind, walking the sorted
-        // order, a follower and a non-follower that are next in line share an aligned lane pair (2i, 2i + 1), and the
-        // resting lane computes half of its partner's moving coefficients (chunk_modcut_pr).  Voices left without
-        // a partner come after the pairs, in the sorted order.
-        {
-            auto follows = [&](uint32_t v) { return voices[v].active && voices[v].mod_env_to_lpf_freq != 0.0f; };
-            std::vector<uint32_t> out, fq, nq;
-            out.reserve(n_voices);
-            size_t g0 = 0;
-            while (g0 < n_voices) {
-                size_t g1 = g0;
-                while (g1 < n_voices && keys[b->voice_of_slot[g1]].kind == keys[b->voice_of_slot[g0]].kind) g1++;
-                fq.clear(); nq.clear();
-                size_t fi = 0, ni = 0;             // queue heads
-                for (size_t i = g0; i < g1; i++) {
-                    const uint32_t v = b->voice_of_slot[i];
-                    (follows(v) ? fq : nq).push_back(v);
-                    if (fi < fq.size() && ni < nq.size()) {
-                        if (out.size() & 1u) { out.push_back(nq[ni++]); continue; }    // keep the pairs on even slots
-                        out.push_back(fq[fi++]);
-                        out.push_back(nq[ni++]);
-                    }
-                }
-                // the unpaired: merge the two leftovers back into the sorted order
-                std::vector<uint32_t> left(fq.begin() + fi, fq.end());
-                left.insert(left.end(), nq.begin() + ni, nq.end());
-                std::stable_sort(left.begin(), left.end(), [&](uint32_t x, uint32_t y) { return keys[x].amp_rest < keys[y].amp_rest; });
-                out.insert(out.end(), left.begin(), left.end());
-                g0 = g1;
-            }
-            b->voice_of_slot.swap(out);
-        }
-        // Deal the sorted warps (32 slots each) round-robin into 8 bins laid out one after the other: every contiguous
-        // eighth / quarter / half of the slot range — the voice ranges of s2_bank_set_pipeline — then holds the same
-        // mix of kinds and envelope lengths, so the ranges' streams advance together.
-        const size_t full_warps = n_voices / 32;
-        if (full_warps >= 16) {
-            std::vector<uint32_t> dealt;
-            dealt.reserve(n_voices);
-            for (size_t bin = 0; bin < 8; bin++)
-                for (size_t w = bin; w < full_warps; w += 8)
-                    dealt.insert(dealt.end(), b->voice_of_slot.begin() + w * 32, b->voice_of_slot.begin() + (w + 1) * 32);
-            dealt.insert(dealt.end(), b->voice_of_slot.begin() + full_warps * 32, b->voice_of_slot.end());
-            b->voice_of_slot.swap(dealt);
-        }
-    }
-    for (size_t s = 0; s < n_voices; s++) {
-        b->slot_of_voice[b->voice_of_slot[s]] = (uint32_t)s;
-        if (b->voice_of_slot[s] != s) b->identity = false;
-    }
-
-    std::vector<float> hp((size_t)s2::P_COUNT * b->vpad, 0.0f), hs((size_t)s2::S_COUNT * b->vpad, 0.0f);
-    for (size_t i = 0; i < n_voices; i++) {
-        const size_t slot = b->slot_of_voice[i];
-        pack_voice(voices[i], (uint32_t)i, hp.data() + slot, b->vpad);
-        s2_voice_state st;
-        memset(&st, 0, sizeof st);
-        st.frame_offset = voices[i].frame_offset;
-        pack_state(st, hs.data() + slot, b->vpad);
-        b->book[i] = {voices[i].frame_offset, 0, voices[i].active ? 1u : 0u, voices[i].osc_kind};
-        if (voices[i].active && voices[i].frame_offset > b->max_offset) b->max_offset = voices[i].frame_offset;
-        if (voices[i].osc_kind == S2_OSC_SINE) b->n_sine++;
-    }
-    cudaError_t e = cudaMalloc(&b->d_params, hp.size() * sizeof(float));
-    if (e == cudaSuccess) e = cudaMalloc(&b->d_state, hs.size() * sizeof(float));
-    if (e == cudaSuccess) e = cudaMalloc(&b->d_bus_counters, s2::kBusCounters * sizeof(unsigned int));
-    if (e == cudaSuccess) e = cudaMemsetAsync(b->d_bus_counters, 0, s2::kBusCounters * sizeof(unsigned int), b->stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(b->d_params, hp.data(), hp.size() * sizeof(float), cudaMemcpyHostToDevice, b->stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(b->d_state, hs.data(), hs.size() * sizeof(float), cudaMemcpyHostToDevice, b->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(b->stream);
-    if (e != cudaSuccess) {
-        int rc = fail(e == cudaErrorMemoryAllocation ? S2_ERR_NOMEM : S2_ERR_CUDA, "bank upload: %s", cudaGetErrorString(e));
-        s2_bank_destroy(b);
-        return rc;
-    }
-    *out = b;
-    return S2_OK;
+int s2_bank_create_mixed(int device, uint32_t sample_rate, size_t n_voices, const s2_voice_desc* voices,
+                         const uint32_t* filter_kinds, void* stream, s2_bank** out) {
+    if (!out) return fail(S2_ERR_INVALID, "null out");
+    *out = nullptr;
+    if (n_voices == 0 || !voices) return fail(S2_ERR_INVALID, "empty bank");
+    if (!filter_kinds) return fail(S2_ERR_INVALID, "null filter_kinds");
+    if (n_voices > 0x7FFFFFE0ull) return fail(S2_ERR_INVALID, "too many voices");
+    if (sample_rate == 0) return fail(S2_ERR_INVALID, "sample_rate must be > 0");
+    for (size_t i = 0; i < n_voices; i++)
+        if (filter_kinds[i] > S2_FILTER_FIRST_ORDER_HP)
+            return fail(S2_ERR_INVALID, "voice %zu: filter_kind %u", i, filter_kinds[i]);
+    return bank_create(device, sample_rate, std::vector<uint32_t>(filter_kinds, filter_kinds + n_voices), voices,
+                       stream, out);
 }
 
 void s2_bank_destroy(s2_bank* b) {
@@ -783,15 +874,22 @@ void s2_bank_destroy(s2_bank* b) {
     cudaFree(b->d_partials);
     cudaFree(b->d_bus_counters);
     cudaFree(b->d_bus);
+    cudaFree(b->d_warp_kinds);
     delete b;
 }
 
 size_t s2_bank_voices(const s2_bank* b) { return b ? b->n_voices : 0; }
 
+int s2_bank_filter_kinds(const s2_bank* b, uint32_t* out) {
+    if (!b || !out) return fail(S2_ERR_INVALID, "null argument");
+    std::copy(b->voice_kind.begin(), b->voice_kind.end(), out);
+    return S2_OK;
+}
+
 int s2_bank_set_voice(s2_bank* b, size_t index, const s2_voice_desc* voice) {
     if (!b || !voice) return fail(S2_ERR_INVALID, "null argument");
     if (index >= b->n_voices) return fail(S2_ERR_INVALID, "voice index %zu out of range", index);
-    int rc = validate_voice(*voice, index, b->filter_kind);
+    int rc = validate_voice(*voice, index, b->voice_kind[index]);
     if (rc) return rc;
     CUDA_TRY(cudaSetDevice(b->device));
     if ((rc = settle_edits(b)) != S2_OK) return rc;    // pipelined mode: per-voice edits are not pipelined
@@ -814,7 +912,7 @@ int s2_bank_set_voices(s2_bank* b, size_t n, const uint32_t* indices, const s2_v
     if (!indices || !voices) return fail(S2_ERR_INVALID, "null argument");
     for (size_t j = 0; j < n; j++) {
         if (indices[j] >= b->n_voices) return fail(S2_ERR_INVALID, "entry %zu: voice index %u out of range", j, indices[j]);
-        int rc = validate_voice(voices[j], indices[j], b->filter_kind);
+        int rc = validate_voice(voices[j], indices[j], b->voice_kind[indices[j]]);
         if (rc) return rc;
     }
     CUDA_TRY(cudaSetDevice(b->device));
@@ -828,7 +926,7 @@ int s2_bank_set_voices(s2_bank* b, size_t n, const uint32_t* indices, const s2_v
     if (++vb.gen == 0) { std::fill(vb.stamp.begin(), vb.stamp.end(), 0u); vb.gen = 1; }
     const int n_ranges = b->n_sub;
     uint32_t bound[9];
-    for (int k = 0; k <= n_ranges; k++) bound[k] = n_ranges > 1 ? sub_begin(b, k) : (k ? (uint32_t)b->n_voices : 0u);
+    for (int k = 0; k <= n_ranges; k++) bound[k] = n_ranges > 1 ? sub_begin(b, k) : (k ? (uint32_t)b->n_slots : 0u);
     std::vector<uint32_t> kept;
     std::vector<uint8_t> range_of;
     size_t count[8] = {}, begin[8] = {};
@@ -945,7 +1043,7 @@ int s2_bank_set_releases(s2_bank* b, const uint32_t* h_release) {
     if (!pl.d_staging[0]) CUDA_TRY(cudaMalloc(&pl.d_staging[0], b->n_voices * sizeof(uint32_t)));
     CUDA_TRY(cudaMemcpyAsync(pl.d_staging[0], h_release, b->n_voices * sizeof(uint32_t), cudaMemcpyHostToDevice, b->stream));
     CUDA_TRY(s2::launch_gather_u32(pl.d_staging[0], b->d_params + (size_t)s2::P_ROW * b->vpad, row,
-                                   (uint32_t)b->n_voices, b->stream));
+                                   (uint32_t)b->n_slots, b->stream));
     g_launches.fetch_add(1, std::memory_order_relaxed);
     return S2_OK;
 }
@@ -1064,6 +1162,7 @@ int s2_bank_set_time_split(s2_bank* b, int enable) {
     CUDA_TRY(cudaSetDevice(b->device));
     { int rc = s2_bank_sync(b); if (rc) return rc; }
     if (!enable) { b->split.enabled = false; return S2_OK; }
+    if (b->n_kinds > 1) return fail(S2_ERR_INVALID, "time-split rendering takes banks of one filter kind");
     if (b->filter_kind > S2_FILTER_BIQUAD_LP)
         return fail(S2_ERR_INVALID, "time-split rendering knows the one-pole and the second-order low-pass filters");
     if (b->n_voices > kTsMaxVoices)

@@ -62,7 +62,14 @@ struct RenderArgs {
     // bits).  Last, so that the fields above keep their parameter offsets in the unmetered kernels.
     double* sum_sq;
     uint32_t* peak;
+    // Mixed-filter banks (s2_bank_create_mixed): the filter kind of each warp of the bank (slot / 32), or nullptr for
+    // a bank of one kind.  With it launch_render takes render_kernel_mixed, whatever its filter_kind argument says.
+    // Last, like the meters.
+    const uint8_t* warp_kinds;
 };
+
+// P_ROW of a padding slot of a mixed-filter bank: no caller voice, never active (s2_capi.cu "slots").
+constexpr uint32_t kPadRow = 0xffffffffu;
 
 constexpr int kChunk = 32;          // frames per compute chunk (classification granularity)
 // The render kernel's tile is 32 voices x 64 frames = two chunks: a warp then writes 256 contiguous bytes per output
