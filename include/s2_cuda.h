@@ -124,10 +124,40 @@ int s2_bank_create(int device, uint32_t sample_rate, uint32_t filter_kind, size_
  */
 int s2_bank_create_mixed(int device, uint32_t sample_rate, size_t n_voices, const s2_voice_desc* voices,
                          const uint32_t* filter_kinds, void* stream, s2_bank** out);
+/*
+ * Routed bank: voice i renders through filter_kinds[i] and mixes into bus bus_of_voice[i] < n_buses.  Otherwise
+ * exactly s2_bank_create_mixed.  A multitimbral host gets one mono signal per part from one bank, one launch per
+ * render and one reduction launch per summation form, however many buses there are.
+ *   - 1 <= n_buses <= S2_MAX_BUSES.  A NULL bus_of_voice, a bus >= n_buses, a bad kind or a bad voice returns
+ *     S2_ERR_INVALID before anything is allocated or any device is touched.  A bus with no voices is allowed: it is
+ *     written as +0.0 at every frame.
+ *   - A voice's bus and kind are fixed for the bank's life; a note-on keeps both.  Every other entry works unchanged
+ *     (set_voice(s), release_voice, set_releases, get/set state, trace, pipelining, time-split, meters,
+ *     s2_bank_reduce_bus).  To move a voice to another bus, build a new bank (get/set state migrates the voices).
+ *   - Bus g of s2_bank_render_buses is bit-identical to the d_bus_out of a bank made by s2_bank_create_mixed from bus
+ *     g's voices alone (same kinds, voices in the same relative order), given the same calls in the same order: at
+ *     every bus width, in the default, pipelined and time-split modes, with or without rows and meters.  So a bus of
+ *     up to 32 voices adds in the reference's order, sequentially from +0.0 in voice order.  Rows, meters and carried
+ *     state of each voice are bit-identical to those of the same voice in that bank.
+ *   - s2_bank_render's d_bus_out is the mono sum of all voices, as for a mixed bank: up to 32 voices in voice order;
+ *     wider banks a deterministic sum (the same bits in every mode) of per-warp partials by the documented trees, a
+ *     warp whose bus has at most 32 voices adding its voices in slot order.
+ *   - Layout: each bus's voices are laid out as that standalone bank's, and each bus but the last non-empty one is
+ *     padded to whole warps.  Voices are thus grouped into whole warps per (bus, kind): a bank of B buses and K kinds
+ *     may hold up to 31 * (B * K - 1) padding slots.  Time-split mode takes routed banks of one kind, as any bank.
+ *   - n_buses = 1 makes the bank s2_bank_create_mixed would make.
+ */
+#define S2_MAX_BUSES 65536u
+int s2_bank_create_routed(int device, uint32_t sample_rate, size_t n_voices, const s2_voice_desc* voices,
+                          const uint32_t* filter_kinds, const uint32_t* bus_of_voice, uint32_t n_buses,
+                          void* stream, s2_bank** out);
 void s2_bank_destroy(s2_bank* bank);
 size_t s2_bank_voices(const s2_bank* bank);
 /* n_voices entries, in voice order.  Works for every bank: a single-kind bank reports its kind for every voice. */
 int s2_bank_filter_kinds(const s2_bank* bank, uint32_t* out);
+/* *n_buses, and bus_of_voice[n_voices] in voice order (either may be NULL).  Every bank: a bank that is not routed
+   has one bus, bus 0. */
+int s2_bank_buses(const s2_bank* bank, uint32_t* n_buses, uint32_t* bus_of_voice);
 
 /* Replace one voice (note_on into slot `index`, synth.rs:61-70: fresh state, offset from desc). */
 int s2_bank_set_voice(s2_bank* bank, size_t index, const s2_voice_desc* voice);
@@ -190,6 +220,23 @@ int s2_bank_render(s2_bank* bank, size_t frames, float* d_voice_out, size_t row_
  */
 int s2_bank_render_metered(s2_bank* bank, size_t frames, float* d_voice_out, size_t row_stride,
                            float* d_bus_out, double* d_sum_sq, float* d_peak);
+
+/*
+ * Every bus of a bank (s2_bank_create_routed): s2_bank_render, or s2_bank_render_metered when d_sum_sq and d_peak are
+ * both set, with bus g written to d_buses + g * bus_stride (`frames` floats each) instead of one d_bus_out.  A bank
+ * that is not routed has one bus: its d_bus_out.
+ *   d_buses      device pointer, 16-byte aligned, bus_stride % 4 == 0 and bus_stride >= frames (the d_voice_out rules).
+ *   d_sum_sq, d_peak   both NULL or both set, as s2_bank_render_metered.
+ * Each bus's bits: see s2_bank_create_routed.  A render issues the render launches of s2_bank_render and at most three
+ * reduction launches (time-split blocks: two), for any number of buses.
+ * Multi-GPU: with bus_stride == frames the buses are one contiguous [n_buses][frames] array, and
+ * s2_bank_reduce_bus(bank, comm, root, d_buses, d_out, frames * n_buses, stream) sums them all across the GPUs in one
+ * collective call.
+ * A NULL bank, a NULL or misaligned d_buses, a bad bus_stride, one meter without the other or a misaligned meter
+ * returns S2_ERR_INVALID with nothing enqueued; every other check is s2_bank_render's.
+ */
+int s2_bank_render_buses(s2_bank* bank, size_t frames, float* d_voice_out, size_t row_stride,
+                         float* d_buses, size_t bus_stride, double* d_sum_sq, float* d_peak);
 
 /* Same, then copies the bus to HOST memory and synchronises the stream (Synth::sample shape). */
 int s2_bank_render_bus_host(s2_bank* bank, size_t frames, float* d_voice_out, size_t row_stride,

@@ -24,6 +24,7 @@ OSC_SQUARE, OSC_SAW, OSC_TRIANGLE, OSC_SINE = 0, 1, 2, 3
 FILTER_ONE_POLE, FILTER_BIQUAD_LP = 0, 1
 FILTER_BIQUAD_HP, FILTER_BIQUAD_BP, FILTER_FIRST_ORDER_LP, FILTER_FIRST_ORDER_HP = 2, 3, 4, 5
 NO_RELEASE = 0xFFFFFFFF
+MAX_BUSES = 65536
 
 # struct s2_voice_desc (80 bytes) / s2_voice_state (32 bytes), include/s2_cuda.h
 VOICE_DESC = np.dtype([
@@ -54,15 +55,18 @@ SYMBOLS = {
     "s2_default_voice": (None, [_vp]),
     "s2_bank_create": (_i, [_i, _u32, _u32, _sz, _vp, _vp, C.POINTER(_vp)]),
     "s2_bank_create_mixed": (_i, [_i, _u32, _sz, _vp, _vp, _vp, C.POINTER(_vp)]),
+    "s2_bank_create_routed": (_i, [_i, _u32, _sz, _vp, _vp, _vp, _u32, _vp, C.POINTER(_vp)]),
     "s2_bank_destroy": (None, [_vp]),
     "s2_bank_voices": (_sz, [_vp]),
     "s2_bank_filter_kinds": (_i, [_vp, _vp]),
+    "s2_bank_buses": (_i, [_vp, C.POINTER(_u32), _vp]),
     "s2_bank_set_voice": (_i, [_vp, _sz, _vp]),
     "s2_bank_set_voices": (_i, [_vp, _sz, _vp, _vp]),
     "s2_bank_release_voice": (_i, [_vp, _sz]),
     "s2_bank_set_releases": (_i, [_vp, _vp]),
     "s2_bank_render": (_i, [_vp, _sz, _vp, _sz, _vp]),
     "s2_bank_render_metered": (_i, [_vp, _sz, _vp, _sz, _vp, _vp, _vp]),
+    "s2_bank_render_buses": (_i, [_vp, _sz, _vp, _sz, _vp, _sz, _vp, _vp]),
     "s2_bank_render_bus_host": (_i, [_vp, _sz, _vp, _sz, _vp]),
     "s2_bank_render_bus_host_async": (_i, [_vp, _sz, _vp, _sz, _vp]),
     "s2_bank_get_state": (_i, [_vp, _vp]),

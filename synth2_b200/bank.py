@@ -72,6 +72,46 @@ class VoiceBank:
                                          _stream_ptr(stream), C.byref(self._h)))
         return self
 
+    @classmethod
+    def routed(cls, voices: np.ndarray, filter_kinds, bus_of_voice, n_buses: int = None, sample_rate: int = 48000,
+               device: int = 0, stream=None):
+        """A bank whose voice i renders through filter filter_kinds[i] and mixes into bus bus_of_voice[i]
+        (s2_bank_create_routed); n_buses defaults to max(bus_of_voice) + 1.  render(..., buses=...) writes every bus."""
+        voices = np.asarray(voices).reshape(-1)
+        kinds = np.asarray(filter_kinds).reshape(-1)
+        buses = np.asarray(bus_of_voice).reshape(-1)
+        if kinds.size != voices.size or buses.size != voices.size:
+            raise ValueError(f"{kinds.size} filter kinds and {buses.size} buses for {voices.size} voices")
+        if kinds.size and (kinds.min() < 0 or kinds.max() > 0xFFFFFFFF):
+            raise ValueError("filter kind out of range")
+        if buses.size and (buses.min() < 0 or buses.max() > 0xFFFFFFFF):
+            raise ValueError("bus out of range")
+        if n_buses is None:
+            n_buses = int(buses.max()) + 1 if buses.size else 1
+        if not 0 <= int(n_buses) <= 0xFFFFFFFF:
+            raise ValueError("n_buses out of range")
+        kinds = np.ascontiguousarray(kinds, dtype=np.uint32)
+        buses = np.ascontiguousarray(buses, dtype=np.uint32)
+        self = cls.__new__(cls)
+        voices = self._setup(voices, sample_rate, kinds[0] if kinds.size else 0, device)
+        check(lib().s2_bank_create_routed(self.device, self.sample_rate, self.n_voices, ptr(voices), ptr(kinds),
+                                          ptr(buses), int(n_buses), _stream_ptr(stream), C.byref(self._h)))
+        return self
+
+    @property
+    def n_buses(self) -> int:
+        """Buses of the bank: 1 unless it is routed."""
+        n = C.c_uint32(0)
+        check(lib().s2_bank_buses(self._h, C.byref(n), None))
+        return int(n.value)
+
+    @property
+    def bus_of_voice(self) -> np.ndarray:
+        """The bus of every voice, in voice order (np.uint32)."""
+        out = np.zeros(self.n_voices, dtype=np.uint32)
+        check(lib().s2_bank_buses(self._h, None, ptr(out)))
+        return out
+
     @property
     def filter_kinds(self) -> np.ndarray:
         """The filter kind of every voice, in voice order (np.uint32)."""
@@ -122,20 +162,33 @@ class VoiceBank:
         check(lib().s2_bank_set_releases(self._h, ptr(release_offsets)))
 
     # -- rendering (device buffers: anything with .data_ptr(), or a raw address)
-    def render(self, frames: int, voice_out=None, row_stride: int = 0, bus_out=None, sum_sq=None, peak=None):
+    def render(self, frames: int, voice_out=None, row_stride: int = 0, bus_out=None, sum_sq=None, peak=None,
+               buses=None, bus_stride: int = 0):
         """Render `frames` frames.  With `sum_sq` and `peak` (per-voice meters, given together: float64 and float32 device
         tensors of n_voices, or raw addresses) every active voice also adds its sum of y*y to sum_sq and raises peak to
-        its largest |y| (s2_bank_render_metered); voice_out and bus_out may then both be None."""
+        its largest |y| (s2_bank_render_metered); voice_out and bus_out may then both be None.  With `buses` (a device
+        tensor of n_buses rows, or a raw address) bus g goes to row g, `bus_stride` floats apart (default: the tensor's
+        stride(0)), instead of one bus_out (s2_bank_render_buses)."""
         row_stride = _row_stride(voice_out, frames, row_stride)
-        if sum_sq is None and peak is None:
+        if sum_sq is None and peak is None and buses is None:
             check(lib().s2_bank_render(self._h, int(frames), ptr(voice_out), row_stride, ptr(bus_out)))
             return
-        if sum_sq is None or peak is None:
+        if (sum_sq is None) != (peak is None):
             raise ValueError("sum_sq and peak are given together")
         for m, dtype in ((sum_sq, "float64"), (peak, "float32")):
             if hasattr(m, "data_ptr") and (str(m.dtype) != "torch." + dtype or m.numel() != self.n_voices
                                            or not m.is_contiguous()):
                 raise ValueError(f"a meter is a contiguous {dtype} tensor of {self.n_voices} entries")
+        if buses is not None:
+            if bus_out is not None:
+                raise ValueError("bus_out and buses are exclusive")
+            if hasattr(buses, "data_ptr") and (str(buses.dtype) != "torch.float32" or buses.dim() != 2
+                                               or buses.shape[0] != self.n_buses or buses.shape[1] < frames
+                                               or buses.stride(1) != 1):
+                raise ValueError(f"buses is a float32 tensor of {self.n_buses} rows of at least {frames} frames")
+            check(lib().s2_bank_render_buses(self._h, int(frames), ptr(voice_out), row_stride, ptr(buses),
+                                             _row_stride(buses, frames, bus_stride), ptr(sum_sq), ptr(peak)))
+            return
         check(lib().s2_bank_render_metered(self._h, int(frames), ptr(voice_out), row_stride, ptr(bus_out),
                                            ptr(sum_sq), ptr(peak)))
 

@@ -243,15 +243,15 @@ struct TimeSplit {
     bool enabled = false;
     bool main_dirty = true;               // b->stream carries state writes the pre-pass stream has not seen
     cudaStream_t stream = nullptr;        // the phase pre-pass
-    float* d_seg_phase[kTsBufs] = {};     // [n_voices][3][32] segment-start phases (and the two before) of block p
+    float* d_seg_phase[kTsBufs] = {};     // [n_slots][3][32] segment-start phases (and the two before) of block p
     cudaEvent_t ev_k1[kTsBufs] = {}, ev_k2[kTsBufs] = {}, ev_main = nullptr;
     uint64_t step = 0, blocks = 0;        // blocks: blocks rendered through the time-split kernels
     std::vector<s2_voice_desc> descs;     // host copy of the voice descriptions (banks <= kTsMaxVoices only)
 
-    int create(size_t n_voices) {
+    int create(size_t n_slots) {
         if (!stream) CUDA_TRY(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
         for (int i = 0; i < kTsBufs; i++) {
-            if (!d_seg_phase[i]) CUDA_TRY(cudaMalloc(&d_seg_phase[i], n_voices * 96 * sizeof(float)));
+            if (!d_seg_phase[i]) CUDA_TRY(cudaMalloc(&d_seg_phase[i], n_slots * 96 * sizeof(float)));
             CUDA_TRY(make_event(ev_k1[i]));
             CUDA_TRY(make_event(ev_k2[i]));
         }
@@ -264,6 +264,23 @@ struct TimeSplit {
         for (int i = 0; i < kTsBufs; i++) { destroy(ev_k1[i]); destroy(ev_k2[i]); cudaFree(d_seg_phase[i]); }
         destroy(ev_main);
     }
+};
+
+// Routed banks (s2_bank_create_routed): what the grouped bus reductions read, in one device array of 32-bit words.
+// Each bus's rows are listed once: its voices in voice order (rows of the caller, or of the time-split path) and its
+// warps in the order of a standalone bank of its voices (partial rows).  A group of spans (s2::BusSpan) is the buses
+// of one reduction form, each pointing into one of those lists.
+struct Routes {
+    uint32_t* d = nullptr;
+    // word offsets into d
+    size_t voices = 0, warps = 0, iota = 0;
+    size_t rows_voice = 0, rows_scratch = 0, partial = 0, ts_narrow = 0, ts_wide = 0;
+    // spans per group.  partial: n_rest buses, then the n_big of >= 512 warps that the four-frames-per-lane form
+    // may take
+    uint32_t n_rows = 0, n_rest = 0, n_big = 0, n_ts_narrow = 0, n_ts_wide = 0;
+    uint32_t n_scratch = 0;    // voices of the buses added from their rows (one bus-scratch row each)
+
+    const s2::BusSpan* spans(size_t off) const { return reinterpret_cast<const s2::BusSpan*>(d + off); }
 };
 
 }  // namespace
@@ -280,7 +297,8 @@ struct s2_bank {
     float* d_state = nullptr;
     float* d_partials = nullptr;
     size_t partials_cap = 0;     // floats
-    unsigned int* d_bus_counters = nullptr;   // s2::kBusCounters zeroed words of the wide bus reduction
+    unsigned int* d_bus_counters = nullptr;   // s2::kBusCounters zeroed words of the wide bus reduction per bus that
+                                              // may take it (one for a bank that is not routed)
     float* d_bus = nullptr;
     size_t bus_cap = 0;          // floats
     std::vector<VoiceBook> book;  // indexed by voice
@@ -295,7 +313,12 @@ struct s2_bank {
     bool identity = true;
     std::vector<uint32_t> voice_kind;   // filter kind of each voice
     uint32_t n_kinds = 1;               // distinct kinds; above 1 the render takes the mixed kernel
-    uint8_t* d_warp_kinds = nullptr;    // [n_slots / 32 rounded up] filter kind of each warp
+    uint8_t* d_warp_kinds = nullptr;    // [n_slots / 32 rounded up] filter kind and flags of each warp (s2::kWarpNarrowBus)
+    // Routed banks: n_buses > 1, the bus of every voice, and the lists of their bus reductions.  A bank made any
+    // other way has one bus, and bus_of_voice is empty.
+    uint32_t n_buses = 1;
+    std::vector<uint32_t> bus_of_voice;
+    Routes route;
     uint32_t force_path = 0;      // test hook (S2_FORCE_PATH, see RenderArgs)
     int n_sub = 1;                // voice ranges of the pipelined mode; 1 = everything on the bank's stream
     Pipeline pipe;
@@ -395,7 +418,7 @@ s2::RenderArgs base_args(const s2_bank* b, size_t frames, float* d_voice_out, si
     a.release_row = nullptr;
     a.sum_sq = d_sum_sq;
     a.peak = d_peak;
-    a.warp_kinds = b->n_kinds > 1 ? b->d_warp_kinds : nullptr;
+    a.warp_kinds = b->d_warp_kinds;
     return a;
 }
 
@@ -418,10 +441,10 @@ int mix_partials(const s2_bank* b, float* partials, uint32_t n_warps, size_t fra
     return S2_OK;
 }
 
-// Multi-kind banks of up to 32 voices span several warps (one per kind).  Their bus is added from the rows, in voice
-// order from +0.0 as a one-warp bank adds it, after the render: into `a` go the caller's rows, or else a scratch of
-// n_voices rows of `frames` rounded up to 16 bytes in `scratch`.
-bool bus_from_rows(const s2_bank* b) { return b->n_kinds > 1 && b->n_voices <= 32; }
+// Banks of up to 32 voices that span several warps (one per kind, or per bus of a routed bank).  Their bus is added
+// from the rows, in voice order from +0.0 as a one-warp bank adds it, after the render: into `a` go the caller's rows,
+// or else a scratch of n_voices rows of `frames` rounded up to 16 bytes in `scratch`.
+bool bus_from_rows(const s2_bank* b) { return b->n_voices <= 32 && b->n_slots > 32; }
 size_t scratch_row_stride(size_t frames) { return (frames + 3) & ~(size_t)3; }
 
 void rows_for_bus(s2::RenderArgs& a, float* scratch, size_t frames) {
@@ -436,6 +459,60 @@ int mix_rows(const s2_bank* b, const s2::RenderArgs& a, size_t frames, float* bu
     return S2_OK;
 }
 
+// The buses of a routed bank (s2_bank_render_buses).  A render's partial-sum buffer holds the warps' partial rows,
+// then (at s2::bus_scratch_at) the bus scratch rows of the buses added from their voices' rows, then the scratch of
+// the four-frames-per-lane form for each bus that takes it.
+size_t route_wide_floats(size_t frames) { return s2::bus_scratch_floats(512u, (uint32_t)frames); }   // per bus, 0 = none
+size_t route_wide_at(const s2_bank* b, size_t frames) {
+    return s2::bus_scratch_at((uint32_t)b->vpad, (uint32_t)frames) + (size_t)b->route.n_scratch * scratch_row_stride(frames);
+}
+size_t route_floats(const s2_bank* b, size_t frames) {
+    return route_wide_at(b, frames) + b->route.n_big * route_wide_floats(frames);
+}
+
+// The render writes partial rows into `partials`, and without caller rows the bus scratch rows too: the warp table
+// with kWarpBusRows set, which the bank keeps after the plain one.
+void route_args(const s2_bank* b, s2::RenderArgs& a, float* partials) {
+    a.bus_partials = partials;
+    if (!a.voice_out && b->route.n_scratch) a.warp_kinds = b->d_warp_kinds + s2::warp_table_bytes((uint32_t)b->vpad);
+}
+
+// Every bus from one render's partial rows, with the rule of a standalone bank of the bus's voices (mix_partials,
+// mix_rows): one launch per reduction form present, whatever the number of buses.
+int route_mix(const s2_bank* b, const s2::RenderArgs& a, size_t frames, float* d_buses, size_t bus_stride, cudaStream_t st) {
+    const Routes& R = b->route;
+    const bool wide = route_wide_floats(frames) != 0;
+    s2::BusGroup g{};
+    g.frames = (uint32_t)frames;
+    g.buses = d_buses;
+    g.bus_stride = bus_stride;
+    g.rows = a.bus_partials;
+    g.row_stride = frames;
+    g.idx = R.d + R.warps;
+    g.spans = R.spans(R.partial);
+    g.n_spans = R.n_rest + (wide ? 0u : R.n_big);
+    int n = 0;
+    if (g.n_spans) { CUDA_TRY(s2::launch_bus_reduce_grouped(g, st)); n++; }
+    if (wide && R.n_big) {
+        g.spans = R.spans(R.partial) + R.n_rest;
+        g.n_spans = R.n_big;
+        CUDA_TRY(s2::launch_bus_reduce_wide_grouped(g, a.bus_partials + route_wide_at(b, frames), b->d_bus_counters, st));
+        n++;
+    }
+    if (R.n_rows) {
+        const bool scratch = a.voice_out == nullptr;
+        g.rows = scratch ? a.bus_partials + s2::bus_scratch_at((uint32_t)b->vpad, (uint32_t)frames) : a.voice_out;
+        g.row_stride = scratch ? scratch_row_stride(frames) : a.row_stride;
+        g.idx = R.d + (scratch ? R.iota : R.voices);
+        g.spans = R.spans(scratch ? R.rows_scratch : R.rows_voice);
+        g.n_spans = R.n_rows;
+        CUDA_TRY(s2::launch_mix_rows_grouped(g, st));
+        n++;
+    }
+    g_launches.fetch_add(n, std::memory_order_relaxed);
+    return S2_OK;
+}
+
 uint32_t sub_begin(const s2_bank* b, int k) {
     // contiguous slot ranges, multiples of 64 slots so that warps (32 or 64 slots) never straddle two
     const uint64_t groups = (b->n_slots + 63) / 64;
@@ -445,12 +522,16 @@ uint32_t sub_begin(const s2_bank* b, int k) {
 }
 
 int bank_render_pipelined(s2_bank* b, size_t frames, float* d_voice_out, size_t row_stride, float* d_bus_out,
-                          double* d_sum_sq, uint32_t* d_peak) {
+                          double* d_sum_sq, uint32_t* d_peak, float* d_buses, size_t bus_stride) {
     Pipeline& pl = b->pipe;
     const uint32_t n_warps = s2::render_warps((uint32_t)b->n_slots);
     const int p = (int)(pl.step % (uint64_t)kMixBufs);
     s2::RenderArgs a = base_args(b, frames, d_voice_out, row_stride, d_sum_sq, d_peak);
-    if (d_bus_out) {
+    if (d_buses) {
+        int rc = grow(b, pl.d_partials, kMixBufs, pl.partials_cap, route_floats(b, frames));
+        if (rc) return rc;
+        route_args(b, a, pl.d_partials[p]);
+    } else if (d_bus_out) {
         const size_t need = bus_from_rows(b) ? b->n_voices * scratch_row_stride(frames) : partials_floats(n_warps, frames);
         int rc = grow(b, pl.d_partials, kMixBufs, pl.partials_cap, need);
         if (rc) return rc;
@@ -470,17 +551,18 @@ int bank_render_pipelined(s2_bank* b, size_t frames, float* d_voice_out, size_t 
             a.staged_release = pl.d_staging[pl.table_pending];
             a.release_row = release_row;
         }
-        if (d_bus_out && pl.step >= (uint64_t)kMixBufs) CUDA_TRY(cudaStreamWaitEvent(sk, pl.ev_mix[p], 0));   // partials[p] are free again
+        if ((d_bus_out || d_buses) && pl.step >= (uint64_t)kMixBufs) CUDA_TRY(cudaStreamWaitEvent(sk, pl.ev_mix[p], 0));   // partials[p] are free again
         CUDA_TRY(s2::launch_render(a, b->filter_kind, s2::TRACE_NONE, sk));
         g_launches.fetch_add(1, std::memory_order_relaxed);
         if (pl.table_pending >= 0) CUDA_TRY(cudaEventRecord(pl.ev_gather[k][pl.table_pending], sk));   // staging buffer read
         CUDA_TRY(cudaEventRecord(pl.ev_sub[k], sk));
     }
     pl.table_pending = -1;
-    if (d_bus_out) {
+    if (d_bus_out || d_buses) {
         for (int k = 0; k < b->n_sub; k++) CUDA_TRY(cudaStreamWaitEvent(pl.mix, pl.ev_sub[k], 0));
-        int rc = bus_from_rows(b) ? mix_rows(b, a, frames, d_bus_out, pl.mix)
-                                  : mix_partials(b, a.bus_partials, n_warps, frames, d_bus_out, pl.mix);
+        int rc = d_buses ? route_mix(b, a, frames, d_buses, bus_stride, pl.mix)
+                 : bus_from_rows(b) ? mix_rows(b, a, frames, d_bus_out, pl.mix)
+                                    : mix_partials(b, a.bus_partials, n_warps, frames, d_bus_out, pl.mix);
         if (rc) return rc;
         CUDA_TRY(cudaEventRecord(pl.ev_mix[p], pl.mix));
     }
@@ -528,7 +610,7 @@ int ts_block_class(const s2_bank* b, size_t frames, const float* d_voice_out, bo
 }
 
 int bank_render_time_split(s2_bank* b, size_t frames, float* d_voice_out, size_t row_stride, float* d_bus_out,
-                           bool moving) {
+                           bool moving, float* d_buses, size_t bus_stride) {
     TimeSplit& ts = b->split;
     const int p = (int)(ts.step % (uint64_t)kTsBufs);
     const s2::RenderArgs a = base_args(b, frames, d_voice_out, row_stride, nullptr, nullptr);
@@ -555,6 +637,23 @@ int bank_render_time_split(s2_bank* b, size_t frames, float* d_voice_out, size_t
         else
             CUDA_TRY(s2::launch_bus_reduce(d_voice_out, nv, row_stride, (uint32_t)frames, d_bus_out, b->stream));
         g_launches.fetch_add(1, std::memory_order_relaxed);
+    } else if (d_buses) {
+        // per bus, the same rule over the bus's voice rows in voice order
+        const Routes& R = b->route;
+        s2::BusGroup g{};
+        g.frames = (uint32_t)frames;
+        g.buses = d_buses;
+        g.bus_stride = bus_stride;
+        g.rows = d_voice_out;
+        g.row_stride = row_stride;
+        g.idx = R.d + R.voices;
+        g.spans = R.spans(R.ts_narrow);
+        g.n_spans = R.n_ts_narrow;
+        if (g.n_spans) CUDA_TRY(s2::launch_mix_rows_grouped(g, b->stream));
+        g.spans = R.spans(R.ts_wide);
+        g.n_spans = R.n_ts_wide;
+        if (g.n_spans) CUDA_TRY(s2::launch_bus_reduce_grouped(g, b->stream));
+        g_launches.fetch_add((R.n_ts_narrow ? 1 : 0) + (R.n_ts_wide ? 1 : 0), std::memory_order_relaxed);
     }
     ts.step++;
     ts.blocks++;
@@ -563,8 +662,10 @@ int bank_render_time_split(s2_bank* b, size_t frames, float* d_voice_out, size_t
     return S2_OK;
 }
 
+// d_buses (routed banks only): every bus, bus g at d_buses + g * bus_stride, instead of the one bus d_bus_out.
 int bank_render_impl(s2_bank* b, size_t frames, float* d_voice_out, size_t row_stride, float* d_bus_out,
-                     int trace, double* d_sum_sq = nullptr, uint32_t* d_peak = nullptr) {
+                     int trace, double* d_sum_sq = nullptr, uint32_t* d_peak = nullptr, float* d_buses = nullptr,
+                     size_t bus_stride = 0) {
     if (!b) return fail(S2_ERR_INVALID, "null bank");
     if (frames == 0) return S2_OK;
     if (frames > 0x7FFFFFFFull) return fail(S2_ERR_INVALID, "frames %zu too large for one call", frames);
@@ -585,11 +686,11 @@ int bank_render_impl(s2_bank* b, size_t frames, float* d_voice_out, size_t row_s
     CUDA_TRY(cudaSetDevice(b->device));
     if (trace == s2::TRACE_NONE) {
         const int cls = ts_block_class(b, frames, d_voice_out, d_sum_sq != nullptr);
-        if (cls) return bank_render_time_split(b, frames, d_voice_out, row_stride, d_bus_out, cls == 2);
+        if (cls) return bank_render_time_split(b, frames, d_voice_out, row_stride, d_bus_out, cls == 2, d_buses, bus_stride);
     }
     b->split.main_dirty = true;   // the general kernels below move the carried phase on the bank's stream
     if (b->n_sub > 1 && trace == s2::TRACE_NONE)
-        return bank_render_pipelined(b, frames, d_voice_out, row_stride, d_bus_out, d_sum_sq, d_peak);
+        return bank_render_pipelined(b, frames, d_voice_out, row_stride, d_bus_out, d_sum_sq, d_peak, d_buses, bus_stride);
     if (b->n_sub > 1) {   // a trace: it renders the whole bank on the bank's stream
         int rc = settle_edits(b);
         if (rc) return rc;
@@ -597,7 +698,11 @@ int bank_render_impl(s2_bank* b, size_t frames, float* d_voice_out, size_t row_s
 
     const uint32_t n_warps = s2::render_warps((uint32_t)b->n_slots);
     s2::RenderArgs a = base_args(b, frames, d_voice_out, row_stride, d_sum_sq, d_peak);
-    if (d_bus_out && bus_from_rows(b)) {
+    if (d_buses) {
+        int rc = grow(b, &b->d_partials, 1, b->partials_cap, route_floats(b, frames));
+        if (rc) return rc;
+        route_args(b, a, b->d_partials);
+    } else if (d_bus_out && bus_from_rows(b)) {
         int rc = grow(b, &b->d_partials, 1, b->partials_cap, b->n_voices * scratch_row_stride(frames));
         if (rc) return rc;
         rows_for_bus(a, b->d_partials, frames);
@@ -614,9 +719,10 @@ int bank_render_impl(s2_bank* b, size_t frames, float* d_voice_out, size_t row_s
     g_launches.fetch_add(1, std::memory_order_relaxed);
     // the next pipelined render launches on the sub-streams, which do not wait for the bank's stream
     if (b->n_sub > 1) CUDA_TRY(cudaStreamSynchronize(b->stream));
-    if (d_bus_out) {
-        int rc = bus_from_rows(b) ? mix_rows(b, a, frames, d_bus_out, b->stream)
-                                  : mix_partials(b, a.bus_partials, n_warps, frames, d_bus_out, b->stream);
+    if (d_bus_out || d_buses) {
+        int rc = d_buses ? route_mix(b, a, frames, d_buses, bus_stride, b->stream)
+                 : bus_from_rows(b) ? mix_rows(b, a, frames, d_bus_out, b->stream)
+                                    : mix_partials(b, a.bus_partials, n_warps, frames, d_bus_out, b->stream);
         if (rc) return rc;
     }
     b->total_frames += frames;
@@ -680,6 +786,21 @@ void order_kind_group(const s2_voice_desc* voices, std::vector<uint32_t>& ids) {
     ids.swap(out);
 }
 
+// The order in which `full_warps` sorted warps (32 slots each) are laid out: dealt round-robin into 8 bins laid out one
+// after the other, so that every contiguous eighth / quarter / half of the slot range — the voice ranges of
+// s2_bank_set_pipeline — holds the same mix of kinds and envelope lengths, and the ranges' streams advance together.
+std::vector<size_t> deal_warps(size_t full_warps) {
+    std::vector<size_t> order;
+    order.reserve(full_warps);
+    if (full_warps < 16) {
+        for (size_t w = 0; w < full_warps; w++) order.push_back(w);
+        return order;
+    }
+    for (size_t bin = 0; bin < 8; bin++)
+        for (size_t w = bin; w < full_warps; w += 8) order.push_back(w);
+    return order;
+}
+
 // The bank's slots: voice_of_slot, with kPadRow for a padding slot.  Voices are grouped by filter kind (stably, in
 // kind order), each group is ordered by order_kind_group, and every group but the last is padded to whole warps of 32
 // slots, so that each warp runs one filter.  With one kind there is no padding.
@@ -696,26 +817,101 @@ std::vector<uint32_t> layout_slots(const s2_voice_desc* voices, const std::vecto
         order_kind_group(voices, ids);
         slots.insert(slots.end(), ids.begin(), ids.end());
     }
-    // Deal the sorted warps (32 slots each) round-robin into 8 bins laid out one after the other: every contiguous
-    // eighth / quarter / half of the slot range — the voice ranges of s2_bank_set_pipeline — then holds the same
-    // mix of kinds and envelope lengths, so the ranges' streams advance together.
     const size_t full_warps = slots.size() / 32;
-    if (full_warps >= 16) {
-        std::vector<uint32_t> dealt;
-        dealt.reserve(slots.size());
-        for (size_t bin = 0; bin < 8; bin++)
-            for (size_t w = bin; w < full_warps; w += 8)
-                dealt.insert(dealt.end(), slots.begin() + w * 32, slots.begin() + (w + 1) * 32);
-        dealt.insert(dealt.end(), slots.begin() + full_warps * 32, slots.end());
-        slots.swap(dealt);
+    std::vector<uint32_t> dealt;
+    dealt.reserve(slots.size());
+    for (size_t w : deal_warps(full_warps)) dealt.insert(dealt.end(), slots.begin() + w * 32, slots.begin() + (w + 1) * 32);
+    dealt.insert(dealt.end(), slots.begin() + full_warps * 32, slots.end());
+    return dealt;
+}
+
+// A routed bank's slots.  Each bus's voices are laid out by layout_slots as a bank of those voices alone, each bus but
+// the last non-empty one is padded to whole warps, and all the warps are dealt over the voice ranges (deal_warps).
+// warps_of_bus[g] lists bus g's warps in that standalone bank's order, which is the order its partial rows are added
+// in.  Voices of a bus keep their relative order: voice j of the standalone bank is the bus's j-th voice.
+std::vector<uint32_t> layout_routed(const s2_voice_desc* voices, const std::vector<uint32_t>& kinds,
+                                    const std::vector<uint32_t>& bus_of_voice, uint32_t n_buses,
+                                    std::vector<std::vector<uint32_t>>& voices_of_bus,
+                                    std::vector<std::vector<uint32_t>>& warps_of_bus) {
+    voices_of_bus.assign(n_buses, {});
+    for (size_t v = 0; v < kinds.size(); v++) voices_of_bus[bus_of_voice[v]].push_back((uint32_t)v);
+    uint32_t last = 0;
+    for (uint32_t g = 0; g < n_buses; g++)
+        if (!voices_of_bus[g].empty()) last = g;
+    std::vector<uint32_t> cat;                   // the buses' slots one after the other
+    std::vector<uint32_t> owner;                 // bus of each warp of cat
+    std::vector<s2_voice_desc> vg;
+    std::vector<uint32_t> kg;
+    for (uint32_t g = 0; g < n_buses; g++) {
+        const std::vector<uint32_t>& ids = voices_of_bus[g];
+        if (ids.empty()) continue;
+        vg.clear(); kg.clear();
+        for (uint32_t v : ids) { vg.push_back(voices[v]); kg.push_back(kinds[v]); }
+        for (uint32_t s : layout_slots(vg.data(), kg)) cat.push_back(s == s2::kPadRow ? s : ids[s]);
+        if (g != last) while (cat.size() & 31u) cat.push_back(s2::kPadRow);
+        while (owner.size() * 32 < cat.size()) owner.push_back(g);
     }
+    const size_t full_warps = cat.size() / 32;
+    std::vector<size_t> order = deal_warps(full_warps);
+    if (cat.size() & 31u) order.push_back(full_warps);
+    std::vector<uint32_t> slots;
+    slots.reserve(cat.size());
+    warps_of_bus.assign(n_buses, {});
+    std::vector<uint32_t> at(order.size());      // position of each warp of cat in the bank
+    for (size_t i = 0; i < order.size(); i++) {
+        at[order[i]] = (uint32_t)i;
+        const size_t w0 = order[i] * 32;
+        slots.insert(slots.end(), cat.begin() + w0, cat.begin() + std::min(w0 + 32, cat.size()));
+    }
+    for (size_t w = 0; w < order.size(); w++) warps_of_bus[owner[w]].push_back(at[w]);
     return slots;
 }
 
-// s2_bank_create and s2_bank_create_mixed once their arguments are checked: `kinds` holds one valid filter kind per
-// voice.  Nothing is allocated on the device before every voice has passed validation.
+// The device lists of a routed bank's bus reductions (Routes), and in scratch_index the bus-scratch row of every slot.
+std::vector<uint32_t> route_words(Routes& R, const std::vector<std::vector<uint32_t>>& voices_of_bus,
+                                  const std::vector<std::vector<uint32_t>>& warps_of_bus,
+                                  const std::vector<uint32_t>& slot_of_voice, std::vector<uint32_t>& scratch_index) {
+    const uint32_t n_buses = (uint32_t)voices_of_bus.size();
+    std::vector<uint32_t> w, vstart(n_buses), wstart(n_buses), sstart(n_buses);
+    std::vector<bool> from_rows(n_buses);
+    R.voices = w.size();
+    for (uint32_t g = 0; g < n_buses; g++) { vstart[g] = (uint32_t)(w.size() - R.voices); w.insert(w.end(), voices_of_bus[g].begin(), voices_of_bus[g].end()); }
+    R.warps = w.size();
+    for (uint32_t g = 0; g < n_buses; g++) { wstart[g] = (uint32_t)(w.size() - R.warps); w.insert(w.end(), warps_of_bus[g].begin(), warps_of_bus[g].end()); }
+    // buses of up to 32 voices in several warps add their rows (bus_from_rows); their voices get bus-scratch rows
+    for (uint32_t g = 0; g < n_buses; g++) {
+        from_rows[g] = voices_of_bus[g].size() <= 32 && warps_of_bus[g].size() > 1;
+        if (!from_rows[g]) continue;
+        sstart[g] = R.n_scratch;
+        for (uint32_t v : voices_of_bus[g]) scratch_index[slot_of_voice[v]] = R.n_scratch++;
+    }
+    R.iota = w.size();
+    for (uint32_t i = 0; i < R.n_scratch; i++) w.push_back(i);
+    auto span = [&](uint32_t g, uint32_t begin, size_t count) { w.push_back(g); w.push_back(begin); w.push_back((uint32_t)count); };
+    R.rows_voice = w.size();
+    for (uint32_t g = 0; g < n_buses; g++) if (from_rows[g]) { span(g, vstart[g], voices_of_bus[g].size()); R.n_rows++; }
+    R.rows_scratch = w.size();
+    for (uint32_t g = 0; g < n_buses; g++) if (from_rows[g]) span(g, sstart[g], voices_of_bus[g].size());
+    R.partial = w.size();
+    for (int big = 0; big < 2; big++)
+        for (uint32_t g = 0; g < n_buses; g++) {
+            if (from_rows[g] || (warps_of_bus[g].size() >= 512) != (big == 1)) continue;
+            span(g, wstart[g], warps_of_bus[g].size());
+            (big ? R.n_big : R.n_rest)++;
+        }
+    // time-split blocks: the rows of every bus, in voice order (launch_ts_mix_rows up to 32 voices, else the reduction)
+    R.ts_narrow = w.size();
+    for (uint32_t g = 0; g < n_buses; g++) if (voices_of_bus[g].size() <= 32) { span(g, vstart[g], voices_of_bus[g].size()); R.n_ts_narrow++; }
+    R.ts_wide = w.size();
+    for (uint32_t g = 0; g < n_buses; g++) if (voices_of_bus[g].size() > 32) { span(g, vstart[g], voices_of_bus[g].size()); R.n_ts_wide++; }
+    return w;
+}
+
+// s2_bank_create, s2_bank_create_mixed and s2_bank_create_routed once their arguments are checked: `kinds` holds one
+// valid filter kind per voice, and `bus_of_voice` one bus below n_buses per voice (or nothing: one bus).  Nothing is
+// allocated on the device before every voice has passed validation.
 int bank_create(int device, uint32_t sample_rate, std::vector<uint32_t> kinds, const s2_voice_desc* voices,
-                void* stream, s2_bank** out) {
+                void* stream, s2_bank** out, std::vector<uint32_t> bus_of_voice = {}, uint32_t n_buses = 1) {
     const size_t n_voices = kinds.size();
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
@@ -725,7 +921,9 @@ int bank_create(int device, uint32_t sample_rate, std::vector<uint32_t> kinds, c
         int rc = validate_voice(voices[i], i, kinds[i]);
         if (rc) return rc;
     }
-    std::vector<uint32_t> voice_of_slot = layout_slots(voices, kinds);
+    std::vector<std::vector<uint32_t>> voices_of_bus, warps_of_bus;
+    std::vector<uint32_t> voice_of_slot = n_buses > 1
+        ? layout_routed(voices, kinds, bus_of_voice, n_buses, voices_of_bus, warps_of_bus) : layout_slots(voices, kinds);
     if (voice_of_slot.size() > 0x7FFFFFE0ull) return fail(S2_ERR_INVALID, "too many voices");
     CUDA_TRY(cudaSetDevice(device));
 
@@ -749,12 +947,29 @@ int bank_create(int device, uint32_t sample_rate, std::vector<uint32_t> kinds, c
         if (v != s) b->identity = false;
         if (v != s2::kPadRow) b->slot_of_voice[v] = (uint32_t)s;
     }
-    std::vector<uint8_t> warp_kinds((b->n_slots + 31) / 32);
-    for (size_t w = 0; w < warp_kinds.size(); w++) warp_kinds[w] = (uint8_t)kinds[b->voice_of_slot[w * 32]];   // never padding
+    // The warp table: the plain one, and for a routed bank with buses added from their rows the one with
+    // kWarpBusRows, followed by the bus-scratch row of every slot (s2_internal.h).
+    const size_t n_warps = (b->n_slots + 31) / 32, wtb = s2::warp_table_bytes((uint32_t)b->vpad);
+    std::vector<uint32_t> route, scratch_index(n_buses > 1 ? b->n_slots : 0, s2::kPadRow);
+    if (n_buses > 1) route = route_words(b->route, voices_of_bus, warps_of_bus, b->slot_of_voice, scratch_index);
+    std::vector<uint8_t> warp_kinds(b->route.n_scratch ? 2 * wtb + b->n_slots * sizeof(uint32_t) : n_warps);
+    for (size_t w = 0; w < n_warps; w++) {
+        const uint32_t v = b->voice_of_slot[w * 32];   // never padding
+        const size_t bus_voices = n_buses > 1 ? voices_of_bus[bus_of_voice[v]].size() : n_voices;
+        warp_kinds[w] = (uint8_t)(kinds[v] | (bus_voices <= 32 ? s2::kWarpNarrowBus : 0u));
+        if (b->route.n_scratch)
+            warp_kinds[wtb + w] = warp_kinds[w] | (scratch_index[b->slot_of_voice[v]] != s2::kPadRow ? s2::kWarpBusRows : 0u);
+    }
+    if (b->route.n_scratch) memcpy(warp_kinds.data() + 2 * wtb, scratch_index.data(), b->n_slots * sizeof(uint32_t));
     uint32_t seen = 0;
     for (uint32_t k : kinds) seen |= 1u << k;
     b->n_kinds = (uint32_t)__builtin_popcount(seen);
     b->voice_kind.swap(kinds);
+    b->n_buses = n_buses;
+    if (n_buses > 1) b->bus_of_voice.swap(bus_of_voice);
+    // every routed bank renders through the per-warp kernel, which reads each warp's bus width from the table
+    const bool warp_table = b->n_kinds > 1 || n_buses > 1;
+    const size_t counters = std::max<size_t>(1, b->route.n_big) * s2::kBusCounters;
 
     std::vector<float> hp((size_t)s2::P_COUNT * b->vpad, 0.0f), hs((size_t)s2::S_COUNT * b->vpad, 0.0f);
     for (size_t s = 0; s < b->n_slots; s++)
@@ -772,13 +987,16 @@ int bank_create(int device, uint32_t sample_rate, std::vector<uint32_t> kinds, c
     }
     cudaError_t e = cudaMalloc(&b->d_params, hp.size() * sizeof(float));
     if (e == cudaSuccess) e = cudaMalloc(&b->d_state, hs.size() * sizeof(float));
-    if (e == cudaSuccess) e = cudaMalloc(&b->d_bus_counters, s2::kBusCounters * sizeof(unsigned int));
-    if (e == cudaSuccess) e = cudaMemsetAsync(b->d_bus_counters, 0, s2::kBusCounters * sizeof(unsigned int), b->stream);
+    if (e == cudaSuccess) e = cudaMalloc(&b->d_bus_counters, counters * sizeof(unsigned int));
+    if (e == cudaSuccess) e = cudaMemsetAsync(b->d_bus_counters, 0, counters * sizeof(unsigned int), b->stream);
     if (e == cudaSuccess) e = cudaMemcpyAsync(b->d_params, hp.data(), hp.size() * sizeof(float), cudaMemcpyHostToDevice, b->stream);
     if (e == cudaSuccess) e = cudaMemcpyAsync(b->d_state, hs.data(), hs.size() * sizeof(float), cudaMemcpyHostToDevice, b->stream);
-    if (e == cudaSuccess && b->n_kinds > 1) e = cudaMalloc(&b->d_warp_kinds, warp_kinds.size());
-    if (e == cudaSuccess && b->n_kinds > 1)
+    if (e == cudaSuccess && warp_table) e = cudaMalloc(&b->d_warp_kinds, warp_kinds.size());
+    if (e == cudaSuccess && warp_table)
         e = cudaMemcpyAsync(b->d_warp_kinds, warp_kinds.data(), warp_kinds.size(), cudaMemcpyHostToDevice, b->stream);
+    if (e == cudaSuccess && !route.empty()) e = cudaMalloc(&b->route.d, route.size() * sizeof(uint32_t));
+    if (e == cudaSuccess && !route.empty())
+        e = cudaMemcpyAsync(b->route.d, route.data(), route.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, b->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(b->stream);
     if (e != cudaSuccess) {
         int rc = fail(e == cudaErrorMemoryAllocation ? S2_ERR_NOMEM : S2_ERR_CUDA, "bank upload: %s", cudaGetErrorString(e));
@@ -861,6 +1079,28 @@ int s2_bank_create_mixed(int device, uint32_t sample_rate, size_t n_voices, cons
                        stream, out);
 }
 
+int s2_bank_create_routed(int device, uint32_t sample_rate, size_t n_voices, const s2_voice_desc* voices,
+                          const uint32_t* filter_kinds, const uint32_t* bus_of_voice, uint32_t n_buses,
+                          void* stream, s2_bank** out) {
+    if (!out) return fail(S2_ERR_INVALID, "null out");
+    *out = nullptr;
+    if (n_voices == 0 || !voices) return fail(S2_ERR_INVALID, "empty bank");
+    if (!filter_kinds) return fail(S2_ERR_INVALID, "null filter_kinds");
+    if (!bus_of_voice) return fail(S2_ERR_INVALID, "null bus_of_voice");
+    if (n_buses == 0 || n_buses > S2_MAX_BUSES) return fail(S2_ERR_INVALID, "n_buses must be in [1, %u]", S2_MAX_BUSES);
+    if (n_voices > 0x7FFFFFE0ull) return fail(S2_ERR_INVALID, "too many voices");
+    if (sample_rate == 0) return fail(S2_ERR_INVALID, "sample_rate must be > 0");
+    for (size_t i = 0; i < n_voices; i++) {
+        if (filter_kinds[i] > S2_FILTER_FIRST_ORDER_HP)
+            return fail(S2_ERR_INVALID, "voice %zu: filter_kind %u", i, filter_kinds[i]);
+        if (bus_of_voice[i] >= n_buses) return fail(S2_ERR_INVALID, "voice %zu: bus %u of %u", i, bus_of_voice[i], n_buses);
+    }
+    std::vector<uint32_t> kinds(filter_kinds, filter_kinds + n_voices);
+    if (n_buses == 1) return bank_create(device, sample_rate, std::move(kinds), voices, stream, out);   // a mixed bank
+    return bank_create(device, sample_rate, std::move(kinds), voices, stream, out,
+                       std::vector<uint32_t>(bus_of_voice, bus_of_voice + n_voices), n_buses);
+}
+
 void s2_bank_destroy(s2_bank* b) {
     if (!b) return;
     cudaSetDevice(b->device);
@@ -875,6 +1115,7 @@ void s2_bank_destroy(s2_bank* b) {
     cudaFree(b->d_bus_counters);
     cudaFree(b->d_bus);
     cudaFree(b->d_warp_kinds);
+    cudaFree(b->route.d);
     delete b;
 }
 
@@ -883,6 +1124,16 @@ size_t s2_bank_voices(const s2_bank* b) { return b ? b->n_voices : 0; }
 int s2_bank_filter_kinds(const s2_bank* b, uint32_t* out) {
     if (!b || !out) return fail(S2_ERR_INVALID, "null argument");
     std::copy(b->voice_kind.begin(), b->voice_kind.end(), out);
+    return S2_OK;
+}
+
+int s2_bank_buses(const s2_bank* b, uint32_t* n_buses, uint32_t* bus_of_voice) {
+    if (!b) return fail(S2_ERR_INVALID, "null bank");
+    if (n_buses) *n_buses = b->n_buses;
+    if (bus_of_voice) {
+        if (b->bus_of_voice.empty()) std::fill(bus_of_voice, bus_of_voice + b->n_voices, 0u);
+        else std::copy(b->bus_of_voice.begin(), b->bus_of_voice.end(), bus_of_voice);
+    }
     return S2_OK;
 }
 
@@ -1062,6 +1313,22 @@ int s2_bank_render_metered(s2_bank* b, size_t frames, float* d_voice_out, size_t
                             reinterpret_cast<uint32_t*>(d_peak));
 }
 
+int s2_bank_render_buses(s2_bank* b, size_t frames, float* d_voice_out, size_t row_stride, float* d_buses,
+                         size_t bus_stride, double* d_sum_sq, float* d_peak) {
+    if (!b) return fail(S2_ERR_INVALID, "null bank");
+    if (!d_buses) return fail(S2_ERR_INVALID, "null d_buses");
+    if (((uintptr_t)d_buses & 15u) != 0 || (bus_stride & 3u) != 0 || bus_stride < frames)
+        return fail(S2_ERR_INVALID, "d_buses must be 16-byte aligned with bus_stride %% 4 == 0 and >= frames");
+    if (!d_sum_sq != !d_peak) return fail(S2_ERR_INVALID, "null meter (sum_sq and peak are given together)");
+    if (((uintptr_t)d_sum_sq & 7u) != 0 || ((uintptr_t)d_peak & 3u) != 0)
+        return fail(S2_ERR_INVALID, "sum_sq must be 8-byte and peak 4-byte aligned");
+    uint32_t* peak = reinterpret_cast<uint32_t*>(d_peak);
+    if (b->n_buses == 1)   // one bus: the bank's mono bus
+        return bank_render_impl(b, frames, d_voice_out, row_stride, d_buses, s2::TRACE_NONE, d_sum_sq, peak);
+    return bank_render_impl(b, frames, d_voice_out, row_stride, nullptr, s2::TRACE_NONE, d_sum_sq, peak, d_buses,
+                            bus_stride);
+}
+
 int s2_bank_trace_phase(s2_bank* b, size_t frames, float* d_phase_out, size_t row_stride) {
     if (!d_phase_out) return fail(S2_ERR_INVALID, "null phase_out");
     return bank_render_impl(b, frames, d_phase_out, row_stride, nullptr, s2::TRACE_PHASE);
@@ -1168,7 +1435,7 @@ int s2_bank_set_time_split(s2_bank* b, int enable) {
     if (b->n_voices > kTsMaxVoices)
         return fail(S2_ERR_INVALID, "time-split rendering is for narrow banks (<= %zu voices)", kTsMaxVoices);
     if (b->n_sub > 1) return fail(S2_ERR_INVALID, "time-split and pipelined voice ranges are exclusive");
-    { int rc = b->split.create(b->n_voices); if (rc) return rc; }
+    { int rc = b->split.create(b->n_slots); if (rc) return rc; }
     b->split.enabled = true;
     b->split.main_dirty = true;
     b->split.step = 0;

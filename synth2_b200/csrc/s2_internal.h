@@ -70,6 +70,36 @@ struct RenderArgs {
 
 // P_ROW of a padding slot of a mixed-filter bank: no caller voice, never active (s2_capi.cu "slots").
 constexpr uint32_t kPadRow = 0xffffffffu;
+// warp_kinds entry: the filter kind in the low bits, and
+//   kWarpNarrowBus   the warp's bus (the whole bank, unless it is routed) has at most 32 voices, so its partial adds
+//                    in voice order from +0.0 as a one-warp bank's does;
+//   kWarpBusRows     routed banks rendering their buses without caller rows: the warp belongs to a bus of up to 32
+//                    voices and several kinds, whose sum is added from its voices' rows, so its voices write rows to
+//                    the bus scratch.  The row of each slot's voice (kPadRow: none) is a u32 array right after the
+//                    table, at warp_table_bytes(vpad); the bus scratch follows the render's partial rows, at
+//                    bus_partials + bus_scratch_at(vpad, frames), rows (frames + 3) & ~3 floats apart.
+// (RenderArgs carries no field for these: a larger struct changes the code of the single-kind render kernels.)
+constexpr uint32_t kWarpKindMask = 7u;
+constexpr uint32_t kWarpNarrowBus = 8u;
+constexpr uint32_t kWarpBusRows = 16u;
+__host__ __device__ constexpr size_t warp_table_bytes(uint32_t vpad) { return ((size_t)(vpad / 32u) + 3u) & ~(size_t)3u; }
+__host__ __device__ constexpr size_t bus_scratch_at(uint32_t vpad, uint32_t frames) {
+    return ((size_t)(vpad / 32u) * frames + 3u) & ~(size_t)3u;
+}
+
+// One bus of a grouped reduction: its rows are rows + idx[begin + r] * row_stride for r < count, and it is written to
+// buses + bus * bus_stride.
+struct BusSpan { uint32_t bus, begin, count; };
+struct BusGroup {
+    const BusSpan* spans;
+    uint32_t n_spans;
+    const uint32_t* idx;
+    const float* rows;
+    size_t row_stride;
+    float* buses;
+    size_t bus_stride;
+    uint32_t frames;
+};
 
 constexpr int kChunk = 32;          // frames per compute chunk (classification granularity)
 // The render kernel's tile is 32 voices x 64 frames = two chunks: a warp then writes 256 contiguous bytes per output
@@ -102,6 +132,14 @@ cudaError_t launch_bus_reduce(const float* partials, uint32_t n_warps, size_t ro
                               cudaStream_t stream, unsigned int* counters = nullptr, float* scratch = nullptr);
 // floats of scratch the four-frames-per-lane form reads for this shape; 0 where that form does not apply
 size_t bus_scratch_floats(uint32_t n_rows, uint32_t frames);
+// Grouped reductions of routed banks: one launch for every bus of the group, each bus summed exactly as the launcher
+// above sums a standalone bank's rows.  launch_bus_reduce_grouped: the one-frame-per-lane form (a bus of one row is
+// a copy of it, a bus of none is +0.0).  launch_bus_reduce_wide_grouped: the four-frames-per-lane form, for buses
+// that pass its tests; span e uses scratch + e * bus_scratch_floats and counters + e * kBusCounters.
+// launch_mix_rows_grouped: each bus adds its rows sequentially from +0.0, as launch_ts_mix_rows does.
+cudaError_t launch_bus_reduce_grouped(const BusGroup& g, cudaStream_t stream);
+cudaError_t launch_bus_reduce_wide_grouped(const BusGroup& g, float* scratch, unsigned int* counters, cudaStream_t stream);
+cudaError_t launch_mix_rows_grouped(const BusGroup& g, cudaStream_t stream);
 // release_row[slot] = staged[voice_of_slot[slot]]  (bulk note-off table given in voice order)
 cudaError_t launch_gather_u32(const uint32_t* staged, const float* row_index_bits, uint32_t* dst_row,
                               uint32_t n, cudaStream_t stream);

@@ -38,7 +38,7 @@ constexpr int kSegs = 32;                 // time segments per block = lanes per
 // K1: lane = voice slot.  phase recurrence only, 8 frames per trip.
 __global__ void __launch_bounds__(32) ts_phase_kernel(const RenderArgs a, float* __restrict__ seg_phase) {
     const uint32_t slot = blockIdx.x * 32u + threadIdx.x;
-    if (slot >= a.n_voices) return;
+    if (slot >= a.slot_end) return;
     const uint32_t vp = a.vpad;
     const float* __restrict__ P = a.params + slot;
     if (__float_as_uint(P[P_ACTIVE * vp]) == 0u) return;
@@ -159,6 +159,7 @@ __global__ void __launch_bounds__(32) ts_render_kernel(const RenderArgs a, const
     const uint32_t frames = a.frames;
     const uint32_t L = frames / kSegs;
     const uint32_t orow = __float_as_uint(P[P_ROW * vp]);
+    if (orow == kPadRow) return;                             // a padding slot of a routed bank: no voice, no row
     float* __restrict__ gout = a.voice_out + (size_t)orow * a.row_stride;
 
     if (__float_as_uint(P[P_ACTIVE * vp]) == 0u) {
@@ -307,21 +308,21 @@ cudaError_t launch_ts_mix_rows(const float* rows, uint32_t n_rows, size_t row_st
 }
 
 cudaError_t launch_ts_phase(const RenderArgs& a, float* seg_phase, cudaStream_t stream) {
-    if (a.n_voices == 0) return cudaSuccess;
-    ts_phase_kernel<<<(a.n_voices + 31u) / 32u, 32, 0, stream>>>(a, seg_phase);
+    if (a.slot_end == 0) return cudaSuccess;
+    ts_phase_kernel<<<(a.slot_end + 31u) / 32u, 32, 0, stream>>>(a, seg_phase);
     return cudaGetLastError();
 }
 
 cudaError_t launch_ts_render(const RenderArgs& a, uint32_t filter_kind, bool moving, const float* seg_phase,
                              cudaStream_t stream) {
-    if (a.n_voices == 0) return cudaSuccess;
+    if (a.slot_end == 0) return cudaSuccess;
     const size_t smem = (32 * kTsTileStride + 1024) * sizeof(float);
     if (filter_kind == 0) {
-        if (moving) ts_render_kernel<0, true><<<a.n_voices, 32, smem, stream>>>(a, seg_phase);
-        else ts_render_kernel<0, false><<<a.n_voices, 32, smem, stream>>>(a, seg_phase);
+        if (moving) ts_render_kernel<0, true><<<a.slot_end, 32, smem, stream>>>(a, seg_phase);
+        else ts_render_kernel<0, false><<<a.slot_end, 32, smem, stream>>>(a, seg_phase);
     } else {
-        if (moving) ts_render_kernel<1, true><<<a.n_voices, 32, smem, stream>>>(a, seg_phase);
-        else ts_render_kernel<1, false><<<a.n_voices, 32, smem, stream>>>(a, seg_phase);
+        if (moving) ts_render_kernel<1, true><<<a.slot_end, 32, smem, stream>>>(a, seg_phase);
+        else ts_render_kernel<1, false><<<a.slot_end, 32, smem, stream>>>(a, seg_phase);
     }
     return cudaGetLastError();
 }

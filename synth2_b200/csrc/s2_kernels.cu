@@ -101,6 +101,12 @@ __device__ __forceinline__ void fast_tile(int gmode, bool fasthash, FastV& F, co
     }
 }
 
+// The mixed kernel's warp belongs to a bus of at most 32 voices, so its partial adds in voice order from +0.0 (a
+// single-kind bank tests its own width instead; a routed bank's buses have any width).
+__device__ __forceinline__ bool narrow_bus(const RenderArgs& a) {
+    return (a.warp_kinds[a.slot_begin / 32u + blockIdx.x] & kWarpNarrowBus) != 0u;
+}
+
 // 65,536 voices = 13.8 one-warp blocks per SM: without pipelining all of them must be resident at once (a
 // second wave would serialise: measured +20 % time at 144 registers, where only 13 fit).
 template <int FILTER, int TRACE>
@@ -125,7 +131,7 @@ __device__ __forceinline__ void render_body_mixed(const RenderArgs a) {   // by 
 template <int TRACE>
 __global__ void __launch_bounds__(32, S2_MINBLOCKS)
 render_kernel_mixed(const RenderArgs a) {
-    switch (a.warp_kinds[a.slot_begin / 32u + blockIdx.x]) {
+    switch (a.warp_kinds[a.slot_begin / 32u + blockIdx.x] & kWarpKindMask) {
     case FILT_ONE_POLE: render_body_mixed<FILT_ONE_POLE, TRACE>(a); break;
     case FILT_BIQUAD_LP: render_body_mixed<FILT_BIQUAD_LP, TRACE>(a); break;
     case FILT_BIQUAD_HP: render_body_mixed<FILT_BIQUAD_HP, TRACE>(a); break;
@@ -135,6 +141,21 @@ render_kernel_mixed(const RenderArgs a) {
     }
 }
 
+// Row accessors of the bus reductions: row r of a standalone bank's partial rows (or voice rows), and row r of one
+// bus of a routed bank, found through that bus's list of partial rows (its warps) or voice rows.  The summation trees
+// below take either, so a routed bank's bus adds its rows in the order a standalone bank of its voices adds them.
+struct StridedRows {
+    const float* base;
+    size_t stride;
+    __device__ __forceinline__ const float* operator()(uint32_t r) const { return base + (size_t)r * stride; }
+};
+struct ListedRows {
+    const float* base;
+    size_t stride;
+    const uint32_t* idx;
+    __device__ __forceinline__ const float* operator()(uint32_t r) const { return base + (size_t)__ldg(idx + r) * stride; }
+};
+
 // Bus reduction: one kernel, fixed summation order (deterministic).  Block fx owns 32 frames; its 8 warps take the
 // partial rows w, w + 8, w + 16, ... (lane = frame: 128-byte coalesced reads), each with four accumulators over
 // consecutive rows of its sequence, eight loads in flight; the eight warp sums are then added in order.
@@ -142,24 +163,24 @@ render_kernel_mixed(const RenderArgs a) {
 // machine whose every slot is taken by long-running render blocks.  The 4,096 short blocks of the two-stage
 // form it replaces queued for those slots one by one and cost ~30 us of step time for 19 us of work; 128 blocks
 // of 8 warps need one slot each and displace next to nothing (it is latency-bound at ~20 us, off the critical path).
-__global__ void __launch_bounds__(256) bus_reduce_kernel(const float* __restrict__ partials, uint32_t n_rows,
-                                                         size_t row_stride, uint32_t frames, float* __restrict__ bus) {
+template <class Rows>
+__device__ __forceinline__ void bus_reduce_tree(Rows rows, uint32_t n_rows, uint32_t frames, float* __restrict__ bus,
+                                                uint32_t fx) {
     __shared__ float sm[8][33];
     const uint32_t tx = threadIdx.x & 31u, w = threadIdx.x >> 5;
-    const uint32_t t = blockIdx.x * 32u + tx;
+    const uint32_t t = fx * 32u + tx;
     float a0 = 0.0f, a1 = 0.0f, a2 = 0.0f, a3 = 0.0f;
     if (t < frames) {
-        const float* __restrict__ col = partials + t;
         uint32_t r = w;
         for (; r + 56u < n_rows; r += 64u) {                  // rows r, r+8, ..., r+56: eight loads in flight
             float v[8];
 #pragma unroll
-            for (uint32_t k = 0; k < 8u; k++) v[k] = col[(size_t)(r + 8u * k) * row_stride];
+            for (uint32_t k = 0; k < 8u; k++) v[k] = rows(r + 8u * k)[t];
             a0 = __fadd_rn(a0, v[0]); a1 = __fadd_rn(a1, v[1]); a2 = __fadd_rn(a2, v[2]); a3 = __fadd_rn(a3, v[3]);
             a0 = __fadd_rn(a0, v[4]); a1 = __fadd_rn(a1, v[5]); a2 = __fadd_rn(a2, v[6]); a3 = __fadd_rn(a3, v[7]);
         }
         for (uint32_t k = 0; r < n_rows; r += 8u, k++) {     // the rest, same rotation over the accumulators
-            const float v = col[(size_t)r * row_stride];
+            const float v = rows(r)[t];
             if ((k & 3u) == 0u) a0 = __fadd_rn(a0, v);
             else if ((k & 3u) == 1u) a1 = __fadd_rn(a1, v);
             else if ((k & 3u) == 2u) a2 = __fadd_rn(a2, v);
@@ -176,6 +197,11 @@ __global__ void __launch_bounds__(256) bus_reduce_kernel(const float* __restrict
     }
 }
 
+__global__ void __launch_bounds__(256) bus_reduce_kernel(const float* __restrict__ partials, uint32_t n_rows,
+                                                         size_t row_stride, uint32_t frames, float* __restrict__ bus) {
+    bus_reduce_tree(StridedRows{partials, row_stride}, n_rows, frames, bus, blockIdx.x);
+}
+
 // The same reduction for wide banks, four frames per lane: block (fx, rs) owns 128 frames and a quarter of the
 // partial rows; its 8 warps take the rows w, w + 8, ... of that quarter with 16-byte loads (512 contiguous bytes per
 // warp and row, four rows in flight per lane: four times the bytes in flight of the form above, a quarter of its
@@ -184,13 +210,13 @@ __global__ void __launch_bounds__(256) bus_reduce_kernel(const float* __restrict
 // the next step for a third of the time the one-frame-per-lane form needs.
 constexpr uint32_t kRedSplit = 4;
 
-__global__ void __launch_bounds__(256, 8) bus_reduce_wide_kernel(const float* __restrict__ partials, uint32_t n_rows,
-                                                              size_t row_stride, uint32_t frames, float* scratch,
-                                                              unsigned int* counters, float* __restrict__ bus) {
+template <class Rows>
+__device__ __forceinline__ void bus_reduce_wide_tree(Rows rows, uint32_t n_rows, uint32_t frames, float* scratch,
+                                                     unsigned int* counters, float* __restrict__ bus, uint32_t block) {
     __shared__ float4 sm[8][32];
     __shared__ bool last;
     const uint32_t lane = threadIdx.x & 31u, w = threadIdx.x >> 5;
-    const uint32_t fx = blockIdx.x / kRedSplit, rs = blockIdx.x % kRedSplit;
+    const uint32_t fx = block / kRedSplit, rs = block % kRedSplit;
     const uint32_t t = fx * 128u + 4u * lane;
     const uint32_t r1 = (uint32_t)((uint64_t)n_rows * (rs + 1u) / kRedSplit);
     uint32_t r = (uint32_t)((uint64_t)n_rows * rs / kRedSplit) + w;
@@ -198,15 +224,14 @@ __global__ void __launch_bounds__(256, 8) bus_reduce_wide_kernel(const float* __
         return make_float4(__fadd_rn(a.x, v.x), __fadd_rn(a.y, v.y), __fadd_rn(a.z, v.z), __fadd_rn(a.w, v.w));
     };
     float4 a0 = make_float4(0.0f, 0.0f, 0.0f, 0.0f), a1 = a0;
-    const float* __restrict__ col = partials + t;
     for (; r + 24u < r1; r += 32u) {                        // rows r, r + 8, r + 16, r + 24 in flight
         float4 v[4];
 #pragma unroll
-        for (uint32_t k = 0; k < 4u; k++) v[k] = __ldcs(reinterpret_cast<const float4*>(col + (size_t)(r + 8u * k) * row_stride));
+        for (uint32_t k = 0; k < 4u; k++) v[k] = __ldcs(reinterpret_cast<const float4*>(rows(r + 8u * k) + t));
         a0 = add4(a0, v[0]); a1 = add4(a1, v[1]); a0 = add4(a0, v[2]); a1 = add4(a1, v[3]);
     }
     for (uint32_t k = 0; r < r1; r += 8u, k++) {
-        const float4 v = __ldcs(reinterpret_cast<const float4*>(col + (size_t)r * row_stride));
+        const float4 v = __ldcs(reinterpret_cast<const float4*>(rows(r) + t));
         if (k & 1u) a1 = add4(a1, v); else a0 = add4(a0, v);
     }
     sm[w][lane] = add4(a0, a1);
@@ -228,6 +253,55 @@ __global__ void __launch_bounds__(256, 8) bus_reduce_wide_kernel(const float* __
         for (uint32_t k = 1; k < kRedSplit; k++) total = add4(total, __ldcg(reinterpret_cast<const float4*>(scratch + (size_t)k * frames + t)));
         *reinterpret_cast<float4*>(bus + t) = total;
         if (lane == 0) counters[fx] = 0u;                  // ready for the next launch (same stream)
+    }
+}
+
+__global__ void __launch_bounds__(256, 8) bus_reduce_wide_kernel(const float* __restrict__ partials, uint32_t n_rows,
+                                                              size_t row_stride, uint32_t frames, float* scratch,
+                                                              unsigned int* counters, float* __restrict__ bus) {
+    bus_reduce_wide_tree(StridedRows{partials, row_stride}, n_rows, frames, scratch, counters, bus, blockIdx.x);
+}
+
+// Grouped forms for routed banks: blockIdx.x as in the kernels above, blockIdx.y = the span (bus) of the group,
+// striding by gridDim.y past 65,535 spans.  One launch covers every bus of its group, however many.
+__global__ void __launch_bounds__(256) bus_reduce_grouped_kernel(const BusGroup g) {
+    for (uint32_t e = blockIdx.y; e < g.n_spans; e += gridDim.y) {
+        const BusSpan s = g.spans[e];
+        float* __restrict__ bus = g.buses + (size_t)s.bus * g.bus_stride;
+        const ListedRows rows{g.rows, g.row_stride, g.idx + s.begin};
+        if (s.count == 1u) {
+            // a bus of one warp is that warp's partial, as a standalone one-warp bank writes it (a -0.0 stays -0.0)
+            const uint32_t t = blockIdx.x * 32u + (threadIdx.x & 31u);
+            if (threadIdx.x < 32u && t < g.frames) bus[t] = rows(0)[t];
+        } else {
+            bus_reduce_tree(rows, s.count, g.frames, bus, blockIdx.x);
+        }
+        __syncthreads();                                   // the shared sums are free for the next span
+    }
+}
+
+__global__ void __launch_bounds__(256, 8) bus_reduce_wide_grouped_kernel(const BusGroup g, float* scratch,
+                                                                      unsigned int* counters) {
+    for (uint32_t e = blockIdx.y; e < g.n_spans; e += gridDim.y) {
+        const BusSpan s = g.spans[e];
+        bus_reduce_wide_tree(ListedRows{g.rows, g.row_stride, g.idx + s.begin}, s.count, g.frames,
+                             scratch + (size_t)e * kRedSplit * g.frames, counters + (size_t)e * kBusCounters,
+                             g.buses + (size_t)s.bus * g.bus_stride, blockIdx.x);
+        __syncthreads();
+    }
+}
+
+// Buses of up to 32 voices and several kinds (several warps): each adds its voices' rows in voice order from +0.0,
+// the reference's order, as launch_ts_mix_rows does for one bank.  One thread per frame and bus.
+__global__ void __launch_bounds__(256) mix_rows_grouped_kernel(const BusGroup g) {
+    const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= g.frames) return;
+    for (uint32_t e = blockIdx.y; e < g.n_spans; e += gridDim.y) {
+        const BusSpan s = g.spans[e];
+        const ListedRows rows{g.rows, g.row_stride, g.idx + s.begin};
+        float acc = 0.0f;
+        for (uint32_t r = 0; r < s.count; r++) acc = __fadd_rn(acc, rows(r)[t]);
+        g.buses[(size_t)s.bus * g.bus_stride + t] = acc;
     }
 }
 
@@ -325,6 +399,26 @@ cudaError_t launch_render(const RenderArgs& a, uint32_t filter_kind, int trace, 
 size_t bus_scratch_floats(uint32_t n_rows, uint32_t frames) {
     const bool wide = n_rows >= 512u && (frames & 127u) == 0u && frames / 128u <= kBusCounters;
     return wide ? (size_t)kRedSplit * frames : 0;
+}
+
+static dim3 grouped_grid(uint32_t blocks, uint32_t n_spans) { return dim3(blocks, n_spans < 65535u ? n_spans : 65535u); }
+
+cudaError_t launch_bus_reduce_grouped(const BusGroup& g, cudaStream_t stream) {
+    if (g.frames == 0 || g.n_spans == 0) return cudaSuccess;
+    bus_reduce_grouped_kernel<<<grouped_grid((g.frames + 31) / 32, g.n_spans), 256, 0, stream>>>(g);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_bus_reduce_wide_grouped(const BusGroup& g, float* scratch, unsigned int* counters, cudaStream_t stream) {
+    if (g.frames == 0 || g.n_spans == 0) return cudaSuccess;
+    bus_reduce_wide_grouped_kernel<<<grouped_grid(g.frames / 128u * kRedSplit, g.n_spans), 256, 0, stream>>>(g, scratch, counters);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_mix_rows_grouped(const BusGroup& g, cudaStream_t stream) {
+    if (g.frames == 0 || g.n_spans == 0) return cudaSuccess;
+    mix_rows_grouped_kernel<<<grouped_grid((g.frames + 255) / 256, g.n_spans), 256, 0, stream>>>(g);
+    return cudaGetLastError();
 }
 
 cudaError_t launch_bus_reduce(const float* partials, uint32_t n_warps, size_t row_stride, uint32_t frames, float* bus,
